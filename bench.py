@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own serial CPU code
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/<op>.npy
 
 `value` (BASELINE.json configs[1], SURVEY.md 8d "C2"): 1,000,000 x 100,000 uniform rsparsematrix-style
 dgCMatrix, density 1e-3 (~1e8 stored entries, FP64 values, int32 indices), synthetic, generated straight into
@@ -84,7 +85,25 @@ def parse_args():
                     help="keep rowSums/rowMeans on the scatter kernels (no row-ordered copy of the resident mirror)")
     ap.add_argument("--no-band-companion", action="store_true",
                     help="keep A^T v / A v on the L2-gather sweeps (no band-major companions)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<op>.npy (float64, at most 64 MB in all) so that "
+                         "two builds run with the same arguments can be compared output for output")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as out_dir/<name>.npy in float64.  An array longer than its equal share of DUMP_BYTES is
+    replaced by the entries at a fixed, seeded sample of positions (the same positions for the same length)."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = (DUMP_BYTES // max(len(arrays), 1) - 4096) // 8  # 4096: room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a).ravel()
+        if a.size > share:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 def measured_peak():
@@ -222,7 +241,7 @@ def time_cpu(ops, block, reps):
     from oracle import oracle
     from rcppsparse_b200 import synth
 
-    chk = oracle.best(strict=False)  # the line's `kind` says which checker ran
+    chk = oracle.best()  # the line's `kind` says which checker ran
     i, p, x, nrow, ncol = block
     v_c, v_r = synth.dense_vector(1, ncol), synth.dense_vector(2, nrow)
     out = {}
@@ -340,7 +359,7 @@ def in_run_parity(ctx, args):
     c0, c1 = bounds[ctx.rank], bounds[ctx.rank + 1]
     D = DeviceMatrix.synth(spec, c0, c1, device=ctx.local_rank)
     S = shard.ShardedMatrix(shard.GpuLocal(D), bounds, ctx.rank, device=ctx.dev, exchange=args.exchange)
-    chk = oracle.best(strict=False)
+    chk = oracle.best()
     a = (i, p, x, spec.nrow, spec.ncol)
     v_c, v_r = synth.dense_vector(1, spec.ncol), synth.dense_vector(2, spec.nrow)
     d_vc, d_vr = torch.from_numpy(v_c).to(ctx.dev), torch.from_numpy(v_r).to(ctx.dev)
@@ -671,13 +690,16 @@ def run_b200(args, ops):
             if r is not None:
                 r.wait()
 
+    last = {}  # op -> what its call in the latest step returned (a tensor, a Pending, or None for the transpose)
+
     def run_step(marks=None, prev=None):
         """One step.  With overlapped exchanges the results of the PREVIOUS step are waited for after this step's
         first sweep has been launched (its last exchange then runs beside that sweep instead of ending the step
         alone); the caller waits for the last step's results before the closing barrier.  Returns what is pending."""
         pend = []
         for k, op in enumerate(ops):
-            pend.append(run_op(op))
+            last[op] = run_op(op)
+            pend.append(last[op])
             if k == 0:
                 wait_all(prev)
             if marks is not None:
@@ -765,6 +787,15 @@ def run_b200(args, ops):
     sampler.mark_end()
     launches = _lib.lib().sb200_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        outs = {}
+        for op in ops:
+            if op == "transpose":
+                outs.update(zip(("transpose_i", "transpose_p", "transpose_x"), T_keep[0].download_columns()))
+            else:
+                r = last[op]
+                outs[op] = (r.tensor if isinstance(r, shard.Pending) else r).cpu().numpy()
+        dump_outputs(args.dump_outputs, outs)
 
     total_ms = ev[0][0].elapsed_time(tail_ev)  # device time of exactly K steps on the launching stream, last results included
     per_op_ms = {op: float(np.mean([ev[s][k].elapsed_time(ev[s][k + 1]) for s in range(args.steps)]))
@@ -1026,6 +1057,8 @@ def main():
         if o not in ABI_OP:
             raise SystemExit(f"unknown op {o}")
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the CUDA path's results; the reference arm times a column sample")
         run_reference(args, tuple(o for o in ops if o != "transpose") or OPS)
     else:
         run_b200(args, ops)

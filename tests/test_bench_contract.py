@@ -1,8 +1,10 @@
-"""bench.py's JSON contract, checked on CPU through the reference arm (the CUDA arm needs a GPU)."""
+"""bench.py's JSON contract, checked on CPU through the reference arm; the CUDA arm's output dump needs a GPU."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -44,6 +46,29 @@ def test_cuda_arm_refuses_to_run_without_a_gpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=300)
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_steps_results(tmp_path):
+    """--dump-outputs writes what the timed step returned: the four reductions of the seeded workload, in float64,
+    within the parity bar of the oracle's results on the same matrix."""
+    import numpy as np
+
+    from oracle import oracle
+    from rcppsparse_b200 import synth
+
+    lines = run_bench("--steps", "3", "--warmup", "1", "--scale", "0.01", "--no-transpose", "--no-products", "--no-e2e",
+                      "--no-cpu-baseline", "--no-parity", "--dump-outputs", str(tmp_path))
+    assert json.loads(lines[-1])["steps"] == 3
+    spec = synth.config("C2", 0.01)
+    i, p, x = synth.generate_host(spec)
+    args = (i, p, x, spec.nrow, spec.ncol)
+    chk = oracle.best()
+    assert sorted(f.name for f in tmp_path.iterdir()) == ["colMeans.npy", "colSums.npy", "rowMeans.npy", "rowSums.npy"]
+    for op in ("colSums", "rowSums", "colMeans", "rowMeans"):
+        got = np.load(tmp_path / f"{op}.npy")
+        assert got.dtype == np.float64
+        oracle.assert_within(op, got, getattr(chk, op)(*args), *args)
 
 
 def test_value_before_row_copy_arithmetic():

@@ -184,14 +184,16 @@ def test_transpose_chunks_larger_than_the_image(bands, kcols, monkeypatch, check
 @pytest.mark.parametrize("shift", [None, "2", "7", "11"])
 def test_transpose_two_stream_splits_on_every_shape(synth_case, shift, monkeypatch, checker):
     """The two-split transpose of tall matrices (transpose_split.cu) forced on every synthetic shape, with the band
-    width the library would pick and with forced ones (4, 128 and 2048 rows per band where the tables allow it):
-    bit-exact whatever the band width; the second call reuses the plan kept on the handle."""
+    width the library would pick and with forced ones (4, 128 and 2048 rows per band; where the key table holds fewer
+    bands than that gives, the narrowest band it allows): bit-exact whatever the band width; the second call reuses
+    the plan kept on the handle."""
     name, spec, i, p, x = synth_case
     monkeypatch.setenv("SB200_TRANSPOSE_PATH", "split")
     if shift is not None:
-        if (spec.nrow >> int(shift)) >= 3072:
-            pytest.skip("more bands than the key table holds")
-        monkeypatch.setenv("SB200_SPLIT_SHIFT", shift)
+        sh = int(shift)
+        while (spec.nrow >> sh) >= 3072:  # at most 3072 bands (SP_MAX_KEYS)
+            sh += 1
+        monkeypatch.setenv("SB200_SPLIT_SHIFT", str(sh))
     wi, wp, wx = checker.transpose(i, p, x, spec.nrow, spec.ncol)
     with DeviceMatrix.from_host(i, p, x, spec.nrow, spec.ncol) as D:
         launches = []
@@ -604,12 +606,14 @@ def test_row_companion_golden_edges(golden):
 def test_band_companion_products_on_synthetic_shapes(case, band_rows, monkeypatch, checker):
     """Both products from the band-major layouts against the reference's iterator sweeps, for the default band height
     (12288 rows) and for small ones (many bands per matrix: band switches inside a CTA, runs cut by tile
-    boundaries, empty runs, runs longer than a lane group's reach)."""
+    boundaries, empty runs, runs longer than a lane group's reach; where the band-pointer pass takes fewer bands than
+    a height gives, the lowest height it allows)."""
     spec = SYNTH_CASES[case]()
     if band_rows != "default":
-        if spec.nrow // int(band_rows) > 20000:
-            pytest.skip("more bands than the band-pointer pass takes")
-        monkeypatch.setenv("SB200_BMC_ROWS", band_rows)
+        rows = int(band_rows)
+        while spec.nrow // rows > 20000:  # at most 20000 bands; heights are multiples of 16
+            rows += 16
+        monkeypatch.setenv("SB200_BMC_ROWS", str(rows))
     i, p, x = synth.generate_host(spec)
     args = (i, p, x, spec.nrow, spec.ncol)
     v_row = synth.dense_vector(spec.seed + 7, spec.nrow)
@@ -737,8 +741,6 @@ def test_crossprod_against_the_reference(case, checker):
 def test_crossprod_golden_edges(golden, checker):
     g = golden
     args = (g["i"], g["p"], g["x"], g["nrow"], g["ncol"])
-    if g["ncol"] > 1500:
-        pytest.skip("dense result too large for an exhaustive check")
     A = as_matrix(g)
     got = A.crossprod()
     assert got.shape == (g["ncol"], g["ncol"])

@@ -14,7 +14,7 @@ from rcppsparse_b200 import DeviceMatrix, synth  # noqa: E402
 def main():
     n = int(sys.argv[1]) if len(sys.argv) > 1 else 40
     rng = np.random.default_rng(int(sys.argv[2]) if len(sys.argv) > 2 else 7)
-    chk = oracle.best(strict=False)
+    chk = oracle.best()
     done = 0
     for k in range(n):
         nrow = int(10 ** rng.uniform(0, 6.6))
