@@ -12,7 +12,8 @@
 //   wrap, clone, at, operator(), operator[]                reference :387-394, :54-73 (host side, unchanged semantics)
 //   InnerIterator                                          reference :218-233 (host side, unchanged)
 //   Rcpp::traits::Exporter<RcppSparse::Matrix>             reference :398-423
-// Additions: spmv(v) = A v and spmv_t(v) = A^T v (the reference only has the iterator idiom),
+// Additions: spmv(v) = A v and spmv_t(v) = A^T v (the reference only has the iterator idiom), spmm(B) = A B and
+// spmm_t(B) = A^T B for a dense NumericMatrix of k right-hand sides (one sweep instead of k spmv calls),
 // resident() to keep the device mirror between calls (then refresh() after mutating x in place, release() to
 // drop it); SB200_GPUS=n runs the sweeps on n GPUs of this process (sb200_sharded_*).
 //   dense copies (operator()(rows, cols), col, row), InnerIndices, emptyInnerIndices, isAppxSymmetric,
@@ -277,6 +278,11 @@ public:
     return y;
   }
 
+  // Y = A B (B: ncol x k) and Y = A^T B (B: nrow x k) for a dense block of k right-hand sides: one sweep of the matrix
+  // instead of k calls of spmv / spmv_t, and one upload of it on a per-call mirror.  One GPU (like crossprod).
+  Rcpp::NumericMatrix spmm(const Rcpp::NumericMatrix& B) { return block_product(B, false); }
+  Rcpp::NumericMatrix spmm_t(const Rcpp::NumericMatrix& B) { return block_product(B, true); }
+
   // canonical CSC of A^T; the result owns fresh R vectors (no call back into the R interpreter)
   Matrix transpose() {
     const long nnz = x.size();
@@ -436,6 +442,17 @@ public:
   };
 
 private:
+  Rcpp::NumericMatrix block_product(const Rcpp::NumericMatrix& B, bool transposed) {
+    const long rows_b = transposed ? Dim[0] : Dim[1], rows_y = transposed ? Dim[1] : Dim[0];
+    if (B.nrow() != rows_b)
+      throw std::invalid_argument(transposed ? "spmm_t: B must have nrow rows" : "spmm: B must have ncol rows");
+    Rcpp::NumericMatrix Y(rows_y, B.ncol());
+    Lease l(*this, false);
+    const double* b = const_cast<Rcpp::NumericMatrix&>(B).begin();  // only read
+    b200::check(transposed ? sb200_spmm_t(l.m, b, B.ncol(), Y.begin()) : sb200_spmm(l.m, b, B.ncol(), Y.begin()));
+    return Y;
+  }
+
   // position of (row, col) in x / i, or -1: binary search in the column's sorted rows
   int find_in_column(int col, int row) const {
     int lo = p[col], hi = p[col + 1];

@@ -132,6 +132,23 @@ int sb200_vec_div_dev(sb200_matrix* m, double* d, int64_t n, double divisor);
 int sb200_crossprod(sb200_matrix* m, double* out /* ncol*ncol, host */);
 int sb200_crossprod_dev(sb200_matrix* m, double* d_out /* ncol*ncol, device */);
 
+/* Sparse x dense block: Y = A B (sb200_spmm) and Y = A^T B (sb200_spmm_t) for k right-hand sides in one sweep of the
+ * matrix, where k calls of sb200_spmv / sb200_spmv_t would stream it k times (NMF, randomized SVD / PCA, block
+ * Lanczos, subspace iteration, several least-squares right-hand sides).  B and Y are dense and COLUMN-major (R's
+ * NumericMatrix): A B takes B ncol x k and fills Y nrow x k, A^T B takes B nrow x k and fills Y ncol x k.  Column j
+ * of Y is what sb200_spmv / sb200_spmv_t gives for column j of B, within 1e-12 * sum |a b| per entry; NaN and Inf in
+ * B reach exactly the outputs whose stored entries touch them.  k = 0 writes nothing and launches nothing; k = 1 is
+ * sb200_spmv / sb200_spmv_t.  A^T B is bit-stable run to run (no atomics).  A B runs on the row-ordered copy when the
+ * mirror holds one (then also bit-stable; a k-wide call counts once toward building it, like one A v call), else
+ * with FP64 reductions at L2.  Scratch for a row-major copy of B and Y (8 k (nrow + ncol) bytes) comes from the
+ * device; SB200_E_NOMEM when it does not fit.  k < 0, or a NULL B / Y of non-empty shape: SB200_E_INVALID.
+ * Host form: B and Y are host memory; returns when Y is complete.  Device form: device pointers, asynchronous on
+ * the handle's stream. */
+int sb200_spmm(sb200_matrix* m, const double* B /* ncol x k, col-major, host */, int64_t k, double* Y /* nrow x k */);
+int sb200_spmm_t(sb200_matrix* m, const double* B /* nrow x k */, int64_t k, double* Y /* ncol x k */);
+int sb200_spmm_dev(sb200_matrix* m, const double* d_B, int64_t k, double* d_Y);
+int sb200_spmm_t_dev(sb200_matrix* m, const double* d_B, int64_t k, double* d_Y);
+
 /* Which kernel serves the row-indexed sweeps of this matrix: *banded = 1 shared-memory row bands
  * (a band plan is built on first use and cached with the mirror), 0 = plan-free L2 atomics.
  * Decided once per handle from the shape (see DESIGN.md 4.2); SB200_ROW_PLAN=0/1 overrides. */

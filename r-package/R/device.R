@@ -27,6 +27,19 @@ b200_spmv_t <- function(A, v) {
     if (.b200_is_handle(A)) .Call(`_RcppSparse_b200_dm_spmv`, A$ptr, v, TRUE) else .Call(`_RcppSparse_b200_spmv_t`, A, v)
 }
 
+# A B (B: ncol(A) x k) and A^T B (B: nrow(A) x k) for a dense matrix of k right-hand sides, one sweep of A
+b200_spmm <- function(A, B) {
+    B <- as.matrix(B)
+    storage.mode(B) <- "double"
+    if (.b200_is_handle(A)) .Call(`_RcppSparse_b200_dm_spmm`, A$ptr, B, FALSE) else .Call(`_RcppSparse_b200_spmm`, A, B)
+}
+
+b200_spmm_t <- function(A, B) {
+    B <- as.matrix(B)
+    storage.mode(B) <- "double"
+    if (.b200_is_handle(A)) .Call(`_RcppSparse_b200_dm_spmm`, A$ptr, B, TRUE) else .Call(`_RcppSparse_b200_spmm_t`, A, B)
+}
+
 b200_transpose <- function(A) {
     if (.b200_is_handle(A)) .Call(`_RcppSparse_b200_dm_transpose`, A$ptr) else .Call(`_RcppSparse_b200_transpose`, A)
 }

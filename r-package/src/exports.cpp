@@ -2,8 +2,8 @@
 //
 // columnSums keeps the reference's name, signature and result (reference src/example.cpp:26-32); its body is
 // now the class call, which the drop-in header serves from the device.  The b200_* functions are additions:
-// thin wrappers over the class methods (reference inst/include/RcppSparse.h:131-156, 375-385 and the SpMV
-// idiom), and a persistent handle — an external pointer to a heap RcppSparse::Matrix whose device mirror
+// thin wrappers over the class methods (reference inst/include/RcppSparse.h:131-156, 375-385, the SpMV idiom
+// and its k-column form spmm), and a persistent handle — an external pointer to a heap RcppSparse::Matrix whose device mirror
 // therefore survives across .Call()s (one .Call otherwise builds a fresh Matrix, i.e. a fresh upload:
 // reference src/RcppExports.cpp:20).
 #include <RcppSparse.h>
@@ -41,6 +41,12 @@ Rcpp::S4 b200_transpose(RcppSparse::Matrix& A) { return A.transpose().wrap(); }
 //[[Rcpp::export]]
 Rcpp::NumericMatrix b200_crossprod(RcppSparse::Matrix& A) { return A.crossprod(); }
 
+//[[Rcpp::export]]
+Rcpp::NumericMatrix b200_spmm(RcppSparse::Matrix& A, const Rcpp::NumericMatrix& B) { return A.spmm(B); }
+
+//[[Rcpp::export]]
+Rcpp::NumericMatrix b200_spmm_t(RcppSparse::Matrix& A, const Rcpp::NumericMatrix& B) { return A.spmm_t(B); }
+
 // ---- persistent device-resident handle ---------------------------------------------------------------------
 // The external pointer owns a heap Matrix; the Matrix holds Rcpp handles to the dgCMatrix slots (so R keeps them
 // alive) and, after its first sweep, the device mirror.  The finalizer deletes the Matrix, which releases the
@@ -69,6 +75,12 @@ Rcpp::NumericVector b200_dm_sweep(SEXP handle, int op) {
 Rcpp::NumericVector b200_dm_spmv(SEXP handle, const Rcpp::NumericVector& v, bool transposed) {
     MatrixPtr A(handle);
     return transposed ? A->spmv_t(v) : A->spmv(v);
+}
+
+//[[Rcpp::export]]
+Rcpp::NumericMatrix b200_dm_spmm(SEXP handle, const Rcpp::NumericMatrix& B, bool transposed) {
+    MatrixPtr A(handle);
+    return transposed ? A->spmm_t(B) : A->spmm(B);
 }
 
 //[[Rcpp::export]]

@@ -24,7 +24,7 @@ SYMBOLS = [
     "sb200_vec_div_dev", "sb200_launch_count", "sb200_algorithmic_bytes", "sb200_synth_create",
     "sb200_synth_vector_dev", "sb200_matrix_download_columns", "sb200_matrix_row_path", "sb200_matrix_row_companion",
     "sb200_crossprod", "sb200_crossprod_dev", "sb200_matrix_band_companion", "sb200_matrix_layouts", "sb200_matrix_layout_bytes", "sb200_trim",
-    "sb200_col_sums_in_rows", "sb200_gather_block",
+    "sb200_col_sums_in_rows", "sb200_gather_block", "sb200_spmm", "sb200_spmm_t", "sb200_spmm_dev", "sb200_spmm_t_dev",
     "sb200_sharded_create", "sb200_sharded_destroy", "sb200_sharded_info", "sb200_sharded_block", "sb200_sharded_col_sums",
     "sb200_sharded_row_sums", "sb200_sharded_col_means", "sb200_sharded_row_means", "sb200_sharded_spmv", "sb200_sharded_spmv_t", "sb200_sharded_transpose",
     "sb200_exchange_create", "sb200_exchange_connect", "sb200_exchange_destroy", "sb200_exchange_window",
@@ -94,6 +94,10 @@ def lib() -> C.CDLL:
         "sb200_trim": ([C.c_int], C.c_int),
         "sb200_col_sums_in_rows": ([vp, vp, i64, C.c_int, vp], C.c_int),
         "sb200_gather_block": ([vp, vp, i64, vp, i64, vp], C.c_int),
+        "sb200_spmm": ([vp, vp, i64, vp], C.c_int),
+        "sb200_spmm_t": ([vp, vp, i64, vp], C.c_int),
+        "sb200_spmm_dev": ([vp, vp, i64, vp], C.c_int),
+        "sb200_spmm_t_dev": ([vp, vp, i64, vp], C.c_int),
         "sb200_sharded_create": ([vp, vp, vp, i32, i32, i64, C.c_int, vp, u32, pp], C.c_int),
         "sb200_sharded_destroy": ([vp], C.c_int),
         "sb200_sharded_info": ([vp, C.POINTER(C.c_int), vp], C.c_int),

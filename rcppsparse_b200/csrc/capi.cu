@@ -627,6 +627,49 @@ int sb200_transpose(sb200_matrix* m, int32_t* p_out, int32_t* i_out, double* x_o
   return SB200_OK;
 }
 
+// ---- sparse x dense block (spmm.cu) -------------------------------------------------------------------------
+// Arguments of the four spmm entry points.  k = 0 is an empty result: it reads nothing (not even a lazily kept `i`)
+// and launches nothing.
+static int spmm_args(const sb200_matrix* m, bool transposed, const void* B, int64_t k, const void* Y) {
+  if (k < 0) return fail(SB200_E_INVALID, "spmm: k must not be negative");
+  const int64_t b_rows = transposed ? m->nrow : m->ncol, y_rows = transposed ? m->ncol : m->nrow;
+  if (k > 0 && ((b_rows > 0 && !B) || (y_rows > 0 && !Y))) return fail(SB200_E_INVALID, "spmm: NULL operand or result");
+  return SB200_OK;
+}
+
+static int spmm_to_host(sb200_matrix* m, bool transposed, const double* B, int64_t k, double* Y) {
+  const int64_t b_rows = transposed ? m->nrow : m->ncol, y_rows = transposed ? m->ncol : m->nrow;
+  if (k == 1) return run_to_host(m, transposed ? SWEEP_SPMV_T : SWEEP_SPMV, B, b_rows, 0.0, Y, y_rows);
+  if ((b_rows > 0 && k > INT64_MAX / 8 / b_rows) || (y_rows > 0 && k > INT64_MAX / 8 / y_rows))
+    return fail(SB200_E_NOMEM, "spmm: the dense operand or result does not fit in device memory");
+  const size_t b_bytes = sizeof(double) * static_cast<size_t>(b_rows * k), y_bytes = sizeof(double) * static_cast<size_t>(y_rows * k);
+  double *d_B = nullptr, *d_Y = nullptr;
+  int rc = pool_alloc(reinterpret_cast<void**>(&d_B), b_bytes > 0 ? b_bytes : 16, m->stream);
+  if (rc == SB200_OK) rc = pool_alloc(reinterpret_cast<void**>(&d_Y), y_bytes > 0 ? y_bytes : 16, m->stream);
+  // R's matrices are pageable: large ones go through the pinned-chunk workers, which use their own streams
+  if (rc == SB200_OK && b_bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(B)) {
+    rc = cudaStreamSynchronize(m->stream) == cudaSuccess ? SB200_OK : fail(SB200_E_CUDA, "spmm: stream sync failed");
+    if (rc == SB200_OK) rc = staged_h2d(m->device, d_B, B, b_bytes);
+  } else if (rc == SB200_OK && b_bytes > 0) {
+    const cudaError_t e = cudaMemcpyAsync(d_B, B, b_bytes, cudaMemcpyHostToDevice, m->stream);
+    if (e != cudaSuccess) rc = cuda_fail(e, "spmm: operand upload", __FILE__, __LINE__);
+  }
+  if (rc == SB200_OK) rc = launch_spmm(m, transposed, d_B, k, d_Y);
+  if (rc == SB200_OK && y_bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(Y)) {
+    rc = cudaStreamSynchronize(m->stream) == cudaSuccess ? SB200_OK : fail(SB200_E_CUDA, "spmm: stream sync failed");
+    if (rc == SB200_OK) rc = staged_d2h(m->device, Y, d_Y, y_bytes);
+  } else if (rc == SB200_OK && y_bytes > 0) {
+    const cudaError_t e = cudaMemcpyAsync(Y, d_Y, y_bytes, cudaMemcpyDeviceToHost, m->stream);
+    if (e != cudaSuccess) rc = cuda_fail(e, "spmm: result download", __FILE__, __LINE__);
+  }
+  const cudaError_t es = cudaStreamSynchronize(m->stream);
+  if (rc == SB200_OK && es != cudaSuccess) rc = cuda_fail(es, "spmm: stream sync", __FILE__, __LINE__);
+  if (rc == SB200_E_NOMEM) cudaGetLastError();
+  pool_free(d_B, m->stream);
+  pool_free(d_Y, m->stream);
+  return rc;
+}
+
 // ---- crossprod (dense A^T A) -------------------------------------------------------------------------------
 // Runs on the row-ordered copy: the cached one of a mirror that owns its arrays (built now if need be), a
 // temporary one otherwise (adopted arrays: the caller may have changed the values since any earlier copy).
@@ -683,6 +726,35 @@ int sb200_crossprod(sb200_matrix* m, double* out) {
   }
   pool_free(d_res, m->stream);
   return rc;
+}
+
+int sb200_spmm(sb200_matrix* m, const double* B, int64_t k, double* Y) {
+  ENTER_COLS(m);
+  SB_TRY(spmm_args(m, false, B, k, Y));
+  if (k == 0) return SB200_OK;
+  SB_TRY(ensure_rows(m));
+  return spmm_to_host(m, false, B, k, Y);
+}
+int sb200_spmm_t(sb200_matrix* m, const double* B, int64_t k, double* Y) {
+  ENTER_COLS(m);
+  SB_TRY(spmm_args(m, true, B, k, Y));
+  if (k == 0) return SB200_OK;
+  SB_TRY(ensure_rows(m));
+  return spmm_to_host(m, true, B, k, Y);
+}
+int sb200_spmm_dev(sb200_matrix* m, const double* d_B, int64_t k, double* d_Y) {
+  ENTER_COLS(m);
+  SB_TRY(spmm_args(m, false, d_B, k, d_Y));
+  if (k == 0) return SB200_OK;
+  SB_TRY(ensure_rows(m));
+  return launch_spmm(m, false, d_B, k, d_Y);
+}
+int sb200_spmm_t_dev(sb200_matrix* m, const double* d_B, int64_t k, double* d_Y) {
+  ENTER_COLS(m);
+  SB_TRY(spmm_args(m, true, d_B, k, d_Y));
+  if (k == 0) return SB200_OK;
+  SB_TRY(ensure_rows(m));
+  return launch_spmm(m, true, d_B, k, d_Y);
 }
 
 int sb200_matrix_row_path(sb200_matrix* m, int* banded) {

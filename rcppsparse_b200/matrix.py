@@ -219,6 +219,25 @@ class DeviceMatrix:
         check(_lib.lib().sb200_spmv_t(self._h, _ptr(v), _ptr(y)))
         return y
 
+    # ---- sparse x dense block: k right-hand sides in one sweep (sparse_b200.h sb200_spmm) ---------------------------
+    def _spmm(self, fn, B, rows: int, out_rows: int, what: str):
+        B = np.asarray(B)
+        if B.ndim != 2 or B.shape[0] != rows:
+            raise ValueError(f"{what}: B must be a 2-D array with {rows} rows")
+        B = np.asfortranarray(B, np.float64)
+        k = int(B.shape[1])
+        Y = np.empty((out_rows, k), np.float64, order="F")
+        check(fn(self._h, _ptr(B), k, _ptr(Y)))
+        return Y
+
+    def spmm(self, B):
+        """A B for a dense (ncol, k) block, as a Fortran-ordered (nrow, k) array: k products A v in one sweep."""
+        return self._spmm(_lib.lib().sb200_spmm, B, self.ncol, self.nrow, "A B")
+
+    def spmm_t(self, B):
+        """A^T B for a dense (nrow, k) block, as a Fortran-ordered (ncol, k) array: k products A^T v in one sweep."""
+        return self._spmm(_lib.lib().sb200_spmm_t, B, self.nrow, self.ncol, "A^T B")
+
     # ---- range cursors and dense extraction as batched device ops (SURVEY.md 8f N4) --------------------------------
     def col_sums_in_rows(self, rows, negate: bool = False):
         """Per column, the sum over the entries whose row is (negate: is not) in ``rows`` — every column's
@@ -258,6 +277,15 @@ class DeviceMatrix:
 
     def spmv_t_dev(self, d_v, d_y) -> None:
         check(_lib.lib().sb200_spmv_t_dev(self._h, _ptr(d_v), _ptr(d_y)))
+
+    def spmm_dev(self, d_B, k: int, d_Y) -> None:
+        """d_Y (nrow x k) = A d_B (ncol x k), both column-major device buffers (e.g. torch tensors whose transpose is
+        contiguous)."""
+        check(_lib.lib().sb200_spmm_dev(self._h, _ptr(d_B), int(k), _ptr(d_Y)))
+
+    def spmm_t_dev(self, d_B, k: int, d_Y) -> None:
+        """d_Y (ncol x k) = A^T d_B (nrow x k), both column-major device buffers."""
+        check(_lib.lib().sb200_spmm_t_dev(self._h, _ptr(d_B), int(k), _ptr(d_Y)))
 
     def vec_div_dev(self, d, n: int, divisor: float) -> None:
         check(_lib.lib().sb200_vec_div_dev(self._h, _ptr(d), n, divisor))
@@ -552,6 +580,13 @@ class Matrix:
 
     def spmv_t(self, v):
         return self._call(True, lambda m: m.spmv_t(v))
+
+    # ---- A B and A^T B for a dense block of k right-hand sides: additions, one device -------------------------------------
+    def spmm(self, B):
+        return self._call(False, lambda m: m.spmm(B))
+
+    def spmm_t(self, B):
+        return self._call(False, lambda m: m.spmm_t(B))
 
     # ---- RcppSparse.h:375-385 ---------------------------------------------------------------------------------------------
     def transpose(self) -> "Matrix":
