@@ -279,7 +279,7 @@ public:
   }
 
   // Y = A B (B: ncol x k) and Y = A^T B (B: nrow x k) for a dense block of k right-hand sides: one sweep of the matrix
-  // instead of k calls of spmv / spmv_t, and one upload of it on a per-call mirror.  One GPU (like crossprod).
+  // instead of k calls of spmv / spmv_t, and one upload of it on a per-call mirror.  SB200_GPUS > 1: on that many GPUs.
   Rcpp::NumericMatrix spmm(const Rcpp::NumericMatrix& B) { return block_product(B, false); }
   Rcpp::NumericMatrix spmm_t(const Rcpp::NumericMatrix& B) { return block_product(B, true); }
 
@@ -447,9 +447,12 @@ private:
     if (B.nrow() != rows_b)
       throw std::invalid_argument(transposed ? "spmm_t: B must have nrow rows" : "spmm: B must have ncol rows");
     Rcpp::NumericMatrix Y(rows_y, B.ncol());
-    Lease l(*this, false);
+    Lease l(*this, true);
     const double* b = const_cast<Rcpp::NumericMatrix&>(B).begin();  // only read
-    b200::check(transposed ? sb200_spmm_t(l.m, b, B.ncol(), Y.begin()) : sb200_spmm(l.m, b, B.ncol(), Y.begin()));
+    if (l.s)
+      b200::check(transposed ? sb200_sharded_spmm_t(l.s, b, B.ncol(), Y.begin()) : sb200_sharded_spmm(l.s, b, B.ncol(), Y.begin()));
+    else
+      b200::check(transposed ? sb200_spmm_t(l.m, b, B.ncol(), Y.begin()) : sb200_spmm(l.m, b, B.ncol(), Y.begin()));
     return Y;
   }
 
@@ -471,7 +474,8 @@ private:
   std::shared_ptr<b200::Mirror> mirror_;
 
   // The device handle(s) for one call: uploaded from the slots as they are now, dropped again at the end of the call
-  // unless the Matrix is resident.  multi = the op has a several-GPU form (the sweeps and the transpose; not crossprod).
+  // unless the Matrix is resident.  multi = the op has a several-GPU form (the sweeps, the block products and the
+  // transpose; not crossprod).
   struct Lease {
     b200::Mirror& mm;
     sb200_matrix* m = nullptr;

@@ -254,6 +254,19 @@ int sb200_sharded_col_means(sb200_sharded* s, double* out /* ncol */);
 int sb200_sharded_row_means(sb200_sharded* s, double* out /* nrow */);
 int sb200_sharded_spmv(sb200_sharded* s, const double* v /* ncol */, double* y /* nrow */);
 int sb200_sharded_spmv_t(sb200_sharded* s, const double* v /* nrow */, double* y /* ncol */);
+/* Y = A B and Y = A^T B for k right-hand sides (sb200_spmm / sb200_spmm_t) on every device of the handle.  Same contract
+ * as the one-GPU host form: B and Y are column-major host buffers, the call returns when Y is complete, column j of Y is
+ * what sb200_sharded_spmv / sb200_sharded_spmv_t gives for column j of B within 1e-12 * sum |a b| per entry, NaN and Inf
+ * in B reach exactly the outputs they touch, k = 0 writes and launches nothing, k < 0 or a NULL B / Y of non-empty
+ * shape is SB200_E_INVALID, scratch that does not fit is SB200_E_NOMEM (the handle stays usable).
+ * A^T B: every device gets all of B, runs the one-GPU block product on its block and copies its rows of Y home; bit-
+ * stable run to run, and at n_gpus = 1 bit-identical to sb200_spmm_t.  A B: device w gets its block's rows of B and
+ * leaves a full-height partial A_w B_w (8 nrow k bytes of device memory per block, kept between calls); device q sums
+ * rows [q nrow / n_gpus, (q+1) nrow / n_gpus) of all partials over peer memory in block order and copies them home.
+ * Bit-stable run to run when every block serves A B from its row-ordered copy; a k-wide call counts once per block
+ * toward building that copy, like one A v call.  Devices are ordered by CUDA events only, so blocks may share a device. */
+int sb200_sharded_spmm(sb200_sharded* s, const double* B /* ncol x k, col-major, host */, int64_t k, double* Y /* nrow x k */);
+int sb200_sharded_spmm_t(sb200_sharded* s, const double* B /* nrow x k */, int64_t k, double* Y /* ncol x k */);
 /* Matrix::transpose() (RcppSparse.h:375-385) of the whole matrix into host arrays: local transposes on every device, row
  * pieces exchanged over peer memory in block (= column) order, every device copies its rows home (SURVEY.md 8e).
  * Bit-exact like the one-GPU transpose.  Blocking. */

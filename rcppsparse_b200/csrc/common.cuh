@@ -169,10 +169,15 @@ int64_t split_plan_bytes(const SplitPlan* sp);
 bool host_is_pageable(const void* p);
 int staged_h2d(int device, void* d_dst, const void* h_src, size_t bytes);
 int staged_d2h(int device, void* h_dst, const void* d_src, size_t bytes);
+// strided: `runs` runs of `width` bytes, dpitch / hpitch bytes apart on the device / the host
+int staged_h2d_2d(int device, void* d_dst, size_t dpitch, const void* h_src, size_t hpitch, size_t width, size_t runs);
+int staged_d2h_2d(int device, void* h_dst, size_t hpitch, const void* d_src, size_t dpitch, size_t width, size_t runs);
 constexpr size_t STAGED_COPY_MIN_BYTES = 32u << 20;  // below this the driver's own staging is as good
 int launch_crossprod(const sb200_matrix* T, int32_t ncol_a, double* d_res, cudaStream_t st);  // crossprod.cu
 // spmm.cu: d_Y = A d_B (transposed = false) or A^T d_B, k right-hand sides, both column-major; k = 1 is launch_sweep
 int launch_spmm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, double* d_Y);
+// the same up to the final transpose: d_Yrm is ROW-major (y_rows x k); a block without entries or columns gives zeros
+int launch_spmm_rm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, double* d_Yrm);
 int build_row_companion(sb200_matrix* m);  // capi.cu; non-fatal: leaves rows_state = -1 when it cannot be built
 void drop_row_companion(sb200_matrix* m);
 int row_companion_after();                 // SB200_ROW_COMPANION_AFTER (default 8, 0 = never build on its own)

@@ -99,53 +99,74 @@ cudaError_t ensure_pool(Pool& g_pool, int device) {
   return cudaSuccess;
 }
 
-void run_h2d(int device, Worker& w, int k, int n, unsigned char* dst, const unsigned char* src, size_t bytes, cudaError_t* err) {
+// The copy is `runs` runs of `width` bytes, `dpitch` apart on the device and `hpitch` apart on the host (one run: a
+// contiguous range).  Chunks never straddle two runs; chunk c of the whole list goes to worker c mod n.
+struct Span {
+  unsigned char* dev;
+  unsigned char* host;
+  size_t dpitch, hpitch, width;
+  size_t runs;
+  size_t per_run() const { return (width + chunk_bytes() - 1) / chunk_bytes(); }
+  size_t chunks() const { return runs * per_run(); }
+  // device address, host address and length of chunk c
+  void at(size_t c, unsigned char** d, unsigned char** h, size_t* len) const {
+    const size_t r = c / per_run(), off = (c % per_run()) * chunk_bytes();
+    *d = dev + r * dpitch + off;
+    *h = host + r * hpitch + off;
+    *len = width - off < chunk_bytes() ? width - off : chunk_bytes();
+  }
+};
+
+void run_h2d(int device, Worker& w, int k, int n, const Span sp, cudaError_t* err) {
   cudaError_t e = cudaSetDevice(device);
-  const size_t CHUNK = chunk_bytes();
-  const size_t chunks = (bytes + CHUNK - 1) / CHUNK;
+  const size_t chunks = sp.chunks();
   int it = 0;
   for (size_t c = k; c < chunks && e == cudaSuccess; c += n, ++it) {
     const int b = it & 1;
-    const size_t off = c * CHUNK, len = bytes - off < CHUNK ? bytes - off : CHUNK;
+    unsigned char *d, *h;
+    size_t len;
+    sp.at(c, &d, &h, &len);
     if (it >= 2) e = cudaEventSynchronize(w.ev[b]);  // the DMA that last read this buffer is done
     if (e != cudaSuccess) break;
-    memcpy(w.buf[b], src + off, len);
-    e = cudaMemcpyAsync(dst + off, w.buf[b], len, cudaMemcpyHostToDevice, w.stream);
+    memcpy(w.buf[b], h, len);
+    e = cudaMemcpyAsync(d, w.buf[b], len, cudaMemcpyHostToDevice, w.stream);
     if (e == cudaSuccess) e = cudaEventRecord(w.ev[b], w.stream);
   }
   const cudaError_t es = cudaStreamSynchronize(w.stream);
   *err = e != cudaSuccess ? e : es;
 }
 
-void run_d2h(int device, Worker& w, int k, int n, unsigned char* dst, const unsigned char* src, size_t bytes, cudaError_t* err) {
+void run_d2h(int device, Worker& w, int k, int n, const Span sp, cudaError_t* err) {
   cudaError_t e = cudaSetDevice(device);
-  const size_t CHUNK = chunk_bytes();
-  const size_t chunks = (bytes + CHUNK - 1) / CHUNK;
+  const size_t chunks = sp.chunks();
   // software pipeline: the DMA of my next chunk runs while I memcpy the previous one out of pinned memory
-  size_t prev_off = 0, prev_len = 0;
+  unsigned char* prev_h = nullptr;
+  size_t prev_len = 0;
   int prev_b = -1, it = 0;
   for (size_t c = k; c < chunks && e == cudaSuccess; c += n, ++it) {
     const int b = it & 1;
-    const size_t off = c * CHUNK, len = bytes - off < CHUNK ? bytes - off : CHUNK;
-    e = cudaMemcpyAsync(w.buf[b], src + off, len, cudaMemcpyDeviceToHost, w.stream);
+    unsigned char *d, *h;
+    size_t len;
+    sp.at(c, &d, &h, &len);
+    e = cudaMemcpyAsync(w.buf[b], d, len, cudaMemcpyDeviceToHost, w.stream);
     if (e == cudaSuccess) e = cudaEventRecord(w.ev[b], w.stream);
     if (prev_b >= 0 && e == cudaSuccess) {
       e = cudaEventSynchronize(w.ev[prev_b]);
-      if (e == cudaSuccess) memcpy(dst + prev_off, w.buf[prev_b], prev_len);
+      if (e == cudaSuccess) memcpy(prev_h, w.buf[prev_b], prev_len);
     }
     prev_b = b;
-    prev_off = off;
+    prev_h = h;
     prev_len = len;
   }
   if (prev_b >= 0 && e == cudaSuccess) {
     e = cudaEventSynchronize(w.ev[prev_b]);
-    if (e == cudaSuccess) memcpy(dst + prev_off, w.buf[prev_b], prev_len);
+    if (e == cudaSuccess) memcpy(prev_h, w.buf[prev_b], prev_len);
   }
   *err = e;
 }
 
-int staged(int device, void* a, const void* b, size_t bytes, bool up) {
-  if (bytes == 0) return SB200_OK;
+int staged(int device, const Span& sp, bool up) {
+  if (sp.width == 0 || sp.runs == 0) return SB200_OK;
   if (device < 0 || device >= MAX_DEVICES) return fail(SB200_E_INVALID, "staged copy: device index out of range");
   Pool& g_pool = g_pools[device];
   std::lock_guard<std::mutex> lock(g_pool.mu);
@@ -157,17 +178,16 @@ int staged(int device, void* a, const void* b, size_t bytes, bool up) {
   threads.reserve(n);
   for (int k = 0; k < n; ++k) {
     errs[k] = cudaSuccess;
-    if (up)
-      threads.emplace_back(run_h2d, device, std::ref(g_pool.w[k]), k, n, static_cast<unsigned char*>(a),
-                           static_cast<const unsigned char*>(b), bytes, &errs[k]);
-    else
-      threads.emplace_back(run_d2h, device, std::ref(g_pool.w[k]), k, n, static_cast<unsigned char*>(a),
-                           static_cast<const unsigned char*>(b), bytes, &errs[k]);
+    threads.emplace_back(up ? run_h2d : run_d2h, device, std::ref(g_pool.w[k]), k, n, sp, &errs[k]);
   }
   for (auto& t : threads) t.join();
   for (int k = 0; k < n; ++k)
     if (errs[k] != cudaSuccess) return cuda_fail(errs[k], up ? "staged host-to-device copy" : "staged device-to-host copy", __FILE__, __LINE__);
   return SB200_OK;
+}
+
+Span span(void* d, const void* h, size_t dpitch, size_t hpitch, size_t width, size_t runs) {
+  return Span{static_cast<unsigned char*>(d), static_cast<unsigned char*>(const_cast<void*>(h)), dpitch, hpitch, width, runs};
 }
 
 }  // namespace
@@ -185,7 +205,17 @@ bool host_is_pageable(const void* p) {
 
 // Blocking.  The device range must not be in use by work that has not completed (callers synchronise the stream
 // that allocated / produced it first); on return the data has arrived.
-int staged_h2d(int device, void* d_dst, const void* h_src, size_t bytes) { return staged(device, d_dst, h_src, bytes, true); }
-int staged_d2h(int device, void* h_dst, const void* d_src, size_t bytes) { return staged(device, h_dst, d_src, bytes, false); }
+int staged_h2d(int device, void* d_dst, const void* h_src, size_t bytes) { return staged(device, span(d_dst, h_src, 0, 0, bytes, 1), true); }
+int staged_d2h(int device, void* h_dst, const void* d_src, size_t bytes) {
+  return staged(device, span(const_cast<void*>(d_src), h_dst, 0, 0, bytes, 1), false);
+}
+// Strided forms: `runs` runs of `width` bytes, `dpitch` bytes apart on the device and `hpitch` apart on the host (a
+// column-major slice of a host matrix: runs = its columns).
+int staged_h2d_2d(int device, void* d_dst, size_t dpitch, const void* h_src, size_t hpitch, size_t width, size_t runs) {
+  return staged(device, span(d_dst, h_src, dpitch, hpitch, width, runs), true);
+}
+int staged_d2h_2d(int device, void* h_dst, size_t hpitch, const void* d_src, size_t dpitch, size_t width, size_t runs) {
+  return staged(device, span(const_cast<void*>(d_src), h_dst, dpitch, hpitch, width, runs), false);
+}
 
 }  // namespace sb200

@@ -13,6 +13,16 @@
 //                                                      on every device at once; the mean's division by the GLOBAL
 //                                                      ncol rides in that kernel (RcppSparse.h:154).
 // All launches come from the calling thread, device after device, nothing blocks until the final synchronisation.
+//
+// The k-wide products (sb200_sharded_spmm / _t) follow the same split:
+//   A^T B   every device gets the whole B, runs the one-GPU block product on its block, and its rows of Y (a strided
+//           piece of the caller's column-major Y) go straight home;
+//   A B     device w gets its rows of B (a strided slice), leaves its full-height partial A_w B_w ROW-major in a buffer
+//           of plain cudaMalloc memory (pool memory is not peer-readable), and device q sums rows
+//           [q nrow / W, (q+1) nrow / W) of all partials over peer memory, in rank order, turning the sum column-major
+//           in the same pass (sharded_sum_transpose_kernel); then every device copies its rows home.
+//           Ordering across devices is CUDA events only (no in-kernel barrier), so blocks that share a device are fine.
+// Host copies run from one thread per device (a copy from pageable memory blocks the thread that issues it).
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -39,6 +49,11 @@ struct sb200_sharded {
   std::vector<sb200_matrix*> blocks;
   std::vector<sb200_exchange*> windows;
   int64_t partial_off, result_off;  // byte offsets of the row partial / the row result inside every window
+  // k-wide A B: per block a row-major nrow x k partial (cudaMalloc: peers read it), grown on demand, kept between calls
+  std::vector<double*> mm_partial;
+  std::vector<size_t> mm_partial_bytes;
+  std::vector<cudaEvent_t> ev_partial;  // per block: its partial is complete
+  std::vector<cudaEvent_t> ev_reduced;  // per block: its reduce has read every partial
 };
 
 namespace sb200 {
@@ -67,6 +82,18 @@ struct WallTrace {  // SB200_TRACE=1: host wall clock of the phases of an entry 
 void destroy_sharded(sb200_sharded* s) {
   if (!s) return;
   WallTrace tr("sharded destroy");
+  for (cudaEvent_t e : s->ev_reduced)  // no reader still has a partial in flight (every call also ends synchronised)
+    if (e) cudaEventSynchronize(e);
+  for (size_t k = 0; k < s->mm_partial.size(); ++k) {
+    DeviceGuard g(s->devices[k]);
+    if (s->mm_partial[k]) cudaFree(s->mm_partial[k]);
+  }
+  for (size_t k = 0; k < s->ev_partial.size(); ++k) {
+    DeviceGuard g(s->devices[k]);
+    if (s->ev_partial[k]) cudaEventDestroy(s->ev_partial[k]);
+    if (s->ev_reduced[k]) cudaEventDestroy(s->ev_reduced[k]);
+  }
+  cudaGetLastError();
   for (sb200_matrix* m : s->blocks)
     if (m) sb200_matrix_destroy(m);
   tr.phase("blocks");
@@ -184,6 +211,283 @@ __global__ void shard_row_dst_kernel(const TpPtrs tp, int world, int32_t nrow, c
 
 __global__ void __launch_bounds__(256) push_rows_local_kernel(const PushRowsSrc a, int world, const PtrDest d) {
   push_rows_body(a, world, d);
+}
+
+// ---- k-wide products: the rank-ordered reduce of the row-major partials ------------------------------------------------
+struct PartialPtrs {
+  const double* p[PUSH_MAX_RANKS];  // the blocks' row-major nrow x k partials (peer-readable)
+};
+
+constexpr int SUMT_THREADS = 256;
+constexpr int SUMT_TILE = 1024;                       // outputs per tile
+constexpr int SUMT_U = SUMT_TILE / SUMT_THREADS;      // outputs per thread: their loads are in flight together
+constexpr int SUMT_SMEM = 2016;                       // max of tr * (w | 1): the folded last slab, tr = 32, w = 63
+
+// Tile geometry: tc = min(k, 32) columns, tr = the largest multiple of 32 rows with tr * tc <= SUMT_TILE.  For small k a
+// tile is many rows of few columns, so every lane has an output whatever k is.  Above 32 the columns go in slabs of 32
+// and the last slab takes the k mod 32 left over (33 .. 63 columns): no slab is so narrow that its peer loads, one
+// run of w values per row at a row stride of 8k bytes, stop being coalesced.
+void sumt_geometry(int64_t k, int* tr, int* tc) {
+  *tc = static_cast<int>(k < 32 ? k : 32);
+  *tr = (SUMT_TILE / *tc) / 32 * 32;
+}
+
+// out (nq x k, column-major) = rows [r0, r0 + nq) of P_0 + P_1 + ... + P_{world-1} (row-major nrow x k), added in rank
+// order with __dadd_rn like xg_reduce_kernel: the same bits on every device and every run.  A tile's rows are runs of
+// w contiguous values in every partial (one contiguous run of rows * k values when w = k): loaded in order, summed in
+// registers, staged in shared memory at an odd pitch, and stored column by column with consecutive lanes on
+// consecutive rows.
+__global__ void __launch_bounds__(SUMT_THREADS) sharded_sum_transpose_kernel(const __grid_constant__ PartialPtrs P, int world, int64_t k, int64_t r0,
+                                                                           int64_t nq, int tr, int tc, double* __restrict__ out) {
+  __shared__ double tile[SUMT_SMEM];
+  const int64_t row_tiles = (nq + tr - 1) / tr;
+  const int64_t slabs = k / tc;  // >= 1; the last one also takes the k mod tc columns left over
+  for (int64_t t = blockIdx.x; t < row_tiles * slabs; t += gridDim.x) {
+    const int64_t rt = (t / slabs) * tr;  // first row of the tile, relative to r0
+    const int64_t c0 = (t % slabs) * tc;  // first column
+    const int w = static_cast<int>(t % slabs == slabs - 1 ? k - c0 : tc);
+    const int rows = static_cast<int>(nq - rt < tr ? nq - rt : tr);
+    const int pitch = w | 1;  // odd: the column-wise reads below hit 32 different banks
+    const int n = rows * w;
+    const int64_t base = (r0 + rt) * k + c0;
+    for (int e0 = threadIdx.x; e0 < n; e0 += SUMT_THREADS * SUMT_U) {
+      int64_t off[SUMT_U];
+      double acc[SUMT_U];
+#pragma unroll
+      for (int u = 0; u < SUMT_U; ++u) {
+        const int e = e0 + u * SUMT_THREADS;
+        off[u] = e < n ? base + static_cast<int64_t>(e / w) * k + e % w : 0;
+        acc[u] = e < n ? P.p[0][off[u]] : 0.0;
+      }
+      for (int q = 1; q < world; ++q) {
+        const double* __restrict__ pq = P.p[q];
+        double v[SUMT_U];
+#pragma unroll
+        for (int u = 0; u < SUMT_U; ++u) v[u] = e0 + u * SUMT_THREADS < n ? pq[off[u]] : 0.0;
+#pragma unroll
+        for (int u = 0; u < SUMT_U; ++u) acc[u] = __dadd_rn(acc[u], v[u]);
+      }
+#pragma unroll
+      for (int u = 0; u < SUMT_U; ++u) {
+        const int e = e0 + u * SUMT_THREADS;
+        if (e < n) tile[(e / w) * pitch + e % w] = acc[u];
+      }
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < n; e += SUMT_THREADS) {
+      const int c = e / rows, r = e % rows;
+      out[(c0 + c) * nq + rt + r] = tile[r * pitch + c];
+    }
+    __syncthreads();
+  }
+}
+
+int launch_sum_transpose(cudaStream_t st, int sm_count, const PartialPtrs& P, int world, int64_t k, int64_t r0, int64_t nq,
+                         double* out) {
+  if (nq == 0 || k == 0) return SB200_OK;
+  int tr = 0, tc = 0;
+  sumt_geometry(k, &tr, &tc);
+  const int64_t tiles = ((nq + tr - 1) / tr) * (k / tc);
+  const int64_t grid = std::min<int64_t>(tiles, static_cast<int64_t>(sm_count) * 8);
+  sharded_sum_transpose_kernel<<<static_cast<unsigned>(grid), SUMT_THREADS, 0, st>>>(P, world, k, r0, nq, tr, tc, out);
+  count_launch();
+  SB_CUDA(cudaGetLastError());
+  return SB200_OK;
+}
+
+// Strided copy between a column-major host matrix and a device buffer: `runs` columns of `width` bytes, hpitch / dpitch
+// bytes apart.  Blocking: returns when the data has arrived.  Large pageable ones go through the pinned-chunk workers,
+// the rest is one cudaMemcpy2DAsync on the block's stream.
+int copy_columns(const sb200_matrix* m, bool up, double* host, size_t hpitch, double* dev, size_t dpitch, size_t width, int64_t runs) {
+  if (width == 0 || runs == 0) return SB200_OK;
+  SB_CUDA(cudaStreamSynchronize(m->stream));  // the device buffer was allocated in the stream's order
+  if (width * static_cast<size_t>(runs) >= STAGED_COPY_MIN_BYTES && host_is_pageable(host))
+    return up ? staged_h2d_2d(m->device, dev, dpitch, host, hpitch, width, static_cast<size_t>(runs))
+              : staged_d2h_2d(m->device, host, hpitch, dev, dpitch, width, static_cast<size_t>(runs));
+  if (up)
+    SB_CUDA(cudaMemcpy2DAsync(dev, dpitch, host, hpitch, width, static_cast<size_t>(runs), cudaMemcpyHostToDevice, m->stream));
+  else
+    SB_CUDA(cudaMemcpy2DAsync(host, hpitch, dev, dpitch, width, static_cast<size_t>(runs), cudaMemcpyDeviceToHost, m->stream));
+  SB_CUDA(cudaStreamSynchronize(m->stream));
+  return SB200_OK;
+}
+
+// fn(w) on one host thread per block; the first failure, with its message, is returned
+template <typename F>
+int on_every_block(sb200_sharded* s, const char* what, F fn) {
+  std::vector<int> rcs(s->world, SB200_OK);
+  std::vector<std::string> errs(s->world);
+  std::vector<std::thread> workers;
+  for (int w = 0; w < s->world; ++w)
+    workers.emplace_back([&, w] {
+      if (cudaSetDevice(s->blocks[w]->device) != cudaSuccess) {
+        rcs[w] = SB200_E_CUDA;
+        errs[w] = "cudaSetDevice failed";
+        return;
+      }
+      rcs[w] = fn(w);
+      if (rcs[w] != SB200_OK) errs[w] = sb200_last_error();
+    });
+  for (auto& t : workers) t.join();
+  for (int w = 0; w < s->world; ++w)
+    if (rcs[w] != SB200_OK) return fail(rcs[w], std::string(what) + ", column block " + std::to_string(w) + ": " + errs[w]);
+  return SB200_OK;
+}
+
+int ensure_spmm_state(sb200_sharded* s) {
+  if (!s->ev_partial.empty()) return SB200_OK;
+  s->mm_partial.assign(s->world, nullptr);
+  s->mm_partial_bytes.assign(s->world, 0);
+  s->ev_partial.assign(s->world, nullptr);
+  s->ev_reduced.assign(s->world, nullptr);
+  for (int w = 0; w < s->world; ++w) {
+    DeviceGuard g(s->devices[w]);
+    SB_CUDA(cudaEventCreateWithFlags(&s->ev_partial[w], cudaEventDisableTiming));
+    SB_CUDA(cudaEventCreateWithFlags(&s->ev_reduced[w], cudaEventDisableTiming));
+  }
+  return SB200_OK;
+}
+
+// block w's partial holds at least `bytes`; the current device is block w's
+int ensure_partial(sb200_sharded* s, int w, size_t bytes) {
+  if (s->mm_partial_bytes[w] >= bytes) return SB200_OK;
+  for (cudaEvent_t e : s->ev_reduced) SB_CUDA(cudaEventSynchronize(e));  // no reader still has the old one in flight
+  if (s->mm_partial[w]) cudaFree(s->mm_partial[w]);
+  s->mm_partial[w] = nullptr;
+  s->mm_partial_bytes[w] = 0;
+  if (cudaMalloc(reinterpret_cast<void**>(&s->mm_partial[w]), bytes) != cudaSuccess) {
+    cudaGetLastError();
+    s->mm_partial[w] = nullptr;
+    return fail(SB200_E_NOMEM, "sharded spmm: the row-major partial (8 nrow k bytes) does not fit on device " +
+                                   std::to_string(s->devices[w]));
+  }
+  s->mm_partial_bytes[w] = bytes;
+  return SB200_OK;
+}
+
+int sharded_spmm_args(const sb200_sharded* s, bool transposed, const double* B, int64_t k, const double* Y) {
+  if (k < 0) return fail(SB200_E_INVALID, "spmm: k must not be negative");
+  const int64_t b_rows = transposed ? s->nrow : s->ncol, y_rows = transposed ? s->ncol : s->nrow;
+  if (k > 0 && ((b_rows > 0 && !B) || (y_rows > 0 && !Y))) return fail(SB200_E_INVALID, "spmm: NULL operand or result");
+  return SB200_OK;
+}
+
+// Y = A B (transposed = false) or A^T B, host buffers, column-major.  Four phases: operands up (a thread per block,
+// blocking), launches (this thread, device after device, ordered by events), results home (a thread per block), and a
+// synchronisation of every stream whatever happened before.
+int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_t k, double* Y) {
+  const int W = s->world;
+  const int64_t nrow = s->nrow, ncol = s->ncol;
+  const int64_t b_rows = transposed ? nrow : ncol, y_rows = transposed ? ncol : nrow;
+  if (k == 0 || y_rows == 0) return SB200_OK;
+  if ((b_rows > 0 && k > INT64_MAX / 8 / b_rows) || k > INT64_MAX / 8 / y_rows)
+    return fail(SB200_E_NOMEM, "spmm: the dense operand or result does not fit in device memory");
+  WallTrace tr(transposed ? "sharded spmm_t" : "sharded spmm");
+  DeviceGuard restore(s->blocks[0]->device);
+  SB_TRY(ensure_spmm_state(s));
+  // rows of the operand block w reads and of the result piece it brings home
+  auto b_lo = [&](int w) { return transposed ? int64_t{0} : s->bounds[w]; };
+  auto b_n = [&](int w) { return transposed ? nrow : s->bounds[w + 1] - s->bounds[w]; };
+  auto y_lo = [&](int w) { return transposed ? s->bounds[w] : nrow * w / W; };
+  auto y_n = [&](int w) { return transposed ? s->bounds[w + 1] - s->bounds[w] : nrow * (w + 1) / W - nrow * w / W; };
+  std::vector<double*> dB(W, nullptr), dY(W, nullptr);
+  int rc = SB200_OK;
+  for (int w = 0; w < W && rc == SB200_OK; ++w) {
+    sb200_matrix* m = s->blocks[w];
+    DeviceGuard g(m->device);
+    const double partial = transposed ? 0.0 : 8.0 * static_cast<double>(k) * static_cast<double>(nrow);
+    const double need = 8.0 * static_cast<double>(k) * static_cast<double>(b_n(w) + y_n(w)) +
+                        std::max(0.0, partial - static_cast<double>(s->mm_partial_bytes[w]));
+    if (need > static_cast<double>(device_free_bytes())) {
+      rc = fail(SB200_E_NOMEM, "sharded spmm: the operand, result and partial of block " + std::to_string(w) +
+                                   " do not fit on device " + std::to_string(m->device));
+      break;
+    }
+    rc = pool_alloc(reinterpret_cast<void**>(&dB[w]), std::max<size_t>(16, sizeof(double) * static_cast<size_t>(b_n(w) * k)), m->stream);
+    if (rc == SB200_OK)
+      rc = pool_alloc(reinterpret_cast<void**>(&dY[w]), std::max<size_t>(16, sizeof(double) * static_cast<size_t>(y_n(w) * k)), m->stream);
+    if (rc == SB200_OK && !transposed) rc = ensure_partial(s, w, sizeof(double) * static_cast<size_t>(nrow * k));
+  }
+  tr.phase("scratch");
+  // 1. operands up: block w's rows of B, a strided slice (A B) or all of it (A^T B)
+  if (rc == SB200_OK)
+    rc = on_every_block(s, "sharded spmm: operand upload", [&](int w) {
+      return copy_columns(s->blocks[w], true, const_cast<double*>(B) + b_lo(w), sizeof(double) * static_cast<size_t>(b_rows), dB[w],
+                          sizeof(double) * static_cast<size_t>(b_n(w)), sizeof(double) * static_cast<size_t>(b_n(w)), k);
+    });
+  tr.phase("operands up");
+  // 2. the device part, from every operand resident to every result piece complete (SB200_TRACE: CUDA-event time per device)
+  std::vector<cudaEvent_t> t0(W, nullptr), t1(W, nullptr);
+  const bool timed = tr.on;
+  for (int w = 0; w < W && timed && rc == SB200_OK; ++w) {
+    DeviceGuard g(s->blocks[w]->device);
+    if (cudaEventCreate(&t0[w]) != cudaSuccess || cudaEventCreate(&t1[w]) != cudaSuccess ||
+        cudaEventRecord(t0[w], s->blocks[w]->stream) != cudaSuccess)
+      rc = fail(SB200_E_CUDA, "sharded spmm: timing events");
+  }
+  if (rc == SB200_OK && transposed) {
+    for (int w = 0; w < W && rc == SB200_OK; ++w) {
+      DeviceGuard g(s->blocks[w]->device);
+      rc = launch_spmm(s->blocks[w], true, dB[w], k, dY[w]);
+    }
+  } else if (rc == SB200_OK) {
+    PartialPtrs P{};
+    for (int w = 0; w < W && rc == SB200_OK; ++w) {
+      sb200_matrix* m = s->blocks[w];
+      DeviceGuard g(m->device);
+      P.p[w] = s->mm_partial[w];
+      rc = launch_spmm_rm(m, false, dB[w], k, s->mm_partial[w]);
+      if (rc == SB200_OK && cudaEventRecord(s->ev_partial[w], m->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaEventRecord");
+    }
+    for (int q = 0; q < W && rc == SB200_OK; ++q) {
+      sb200_matrix* m = s->blocks[q];
+      DeviceGuard g(m->device);
+      for (int w = 0; w < W && rc == SB200_OK; ++w)
+        if (cudaStreamWaitEvent(m->stream, s->ev_partial[w], 0) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaStreamWaitEvent");
+      if (rc == SB200_OK) rc = launch_sum_transpose(m->stream, m->sm_count, P, W, k, y_lo(q), y_n(q), dY[q]);
+      if (rc == SB200_OK && cudaEventRecord(s->ev_reduced[q], m->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaEventRecord");
+    }
+  }
+  for (int w = 0; w < W && timed && rc == SB200_OK; ++w) {
+    DeviceGuard g(s->blocks[w]->device);
+    if (cudaEventRecord(t1[w], s->blocks[w]->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "sharded spmm: timing events");
+  }
+  tr.phase("launched");
+  // 3. results home: block w's piece of Y, `y_n(w)` rows of every column
+  if (rc == SB200_OK)
+    rc = on_every_block(s, "sharded spmm: result download", [&](int w) {
+      return copy_columns(s->blocks[w], false, Y + y_lo(w), sizeof(double) * static_cast<size_t>(y_rows), dY[w],
+                          sizeof(double) * static_cast<size_t>(y_n(w)), sizeof(double) * static_cast<size_t>(y_n(w)), k);
+    });
+  tr.phase("results home");
+  // 4. every stream is waited for (no partial is rewritten or freed while a reader may still run), scratch released
+  for (int w = 0; w < W; ++w) {
+    sb200_matrix* m = s->blocks[w];
+    DeviceGuard g(m->device);
+    const cudaError_t e = cudaStreamSynchronize(m->stream);
+    if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded spmm", __FILE__, __LINE__);
+    pool_free(dB[w], m->stream);
+    pool_free(dY[w], m->stream);
+  }
+  if (timed && rc == SB200_OK) {
+    std::string per;
+    float worst = 0.0f;
+    for (int w = 0; w < W; ++w) {
+      DeviceGuard g(s->blocks[w]->device);
+      float ms = 0.0f;
+      cudaEventElapsedTime(&ms, t0[w], t1[w]);
+      worst = std::max(worst, ms);
+      per += (w ? " " : "") + std::to_string(ms);
+    }
+    fprintf(stderr, "[sb200 trace] %s: device part %.4f ms (max over devices; per device: %s)\n", tr.title, worst, per.c_str());
+  }
+  for (int w = 0; w < W; ++w) {
+    DeviceGuard g(s->blocks[w]->device);
+    if (t0[w]) cudaEventDestroy(t0[w]);
+    if (t1[w]) cudaEventDestroy(t1[w]);
+  }
+  if (rc == SB200_E_NOMEM) cudaGetLastError();  // a refused allocation leaves the streams usable
+  return rc;
 }
 
 }  // namespace
@@ -358,6 +662,16 @@ int sb200_sharded_spmv(sb200_sharded* s, const double* v, double* y) {
   SB_TRY(check_sharded(s));
   if (s->ncol > 0 && !v) return fail(SB200_E_INVALID, "operand vector is NULL");
   return run_rows(s, SWEEP_SPMV, v, 0.0, y);
+}
+int sb200_sharded_spmm(sb200_sharded* s, const double* B, int64_t k, double* Y) {
+  SB_TRY(check_sharded(s));
+  SB_TRY(sharded_spmm_args(s, false, B, k, Y));
+  return run_block_product(s, false, B, k, Y);
+}
+int sb200_sharded_spmm_t(sb200_sharded* s, const double* B, int64_t k, double* Y) {
+  SB_TRY(check_sharded(s));
+  SB_TRY(sharded_spmm_args(s, true, B, k, Y));
+  return run_block_product(s, true, B, k, Y);
 }
 
 

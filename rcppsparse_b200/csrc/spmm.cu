@@ -26,6 +26,9 @@
 //     A B = (A^T)^T B, so gather-only and deterministic there too.
 //
 // Sizes are 64-bit inside the kernels: nrow * k may pass 2^31.
+//
+// launch_spmm_rm stops before the final transpose and leaves Y row-major: the sharded A B (sharded.cu) sums the
+// blocks' row-major partials across devices and turns the sum column-major in the same pass.
 #include <cuda_runtime.h>
 #include <limits.h>
 #include <stdint.h>
@@ -310,17 +313,19 @@ static bool bytes_of(int64_t rows, int64_t k, size_t* out) {
   return true;
 }
 
-int launch_spmm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, double* d_Y) {
+// d_Yrm (y_rows x k, ROW-major) = A d_B or A^T d_B (d_B column-major): everything launch_spmm does before its final
+// transpose.  The sharded A B (sharded.cu) sums these row-major partials across devices and transposes while it sums.
+int launch_spmm_rm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, double* d_Yrm) {
   const int64_t b_rows = transposed ? m->nrow : m->ncol;
   const int64_t y_rows = transposed ? m->ncol : m->nrow;
   if (k == 0 || y_rows == 0) return SB200_OK;
-  if (k == 1) return launch_sweep(m, transposed ? SWEEP_SPMV_T : SWEEP_SPMV, d_B, 0.0, d_Y);
+  if (k == 1) return launch_sweep(m, transposed ? SWEEP_SPMV_T : SWEEP_SPMV, d_B, 0.0, d_Yrm);  // n x 1: both layouts
   cudaStream_t st = m->stream;
   size_t b_bytes = 0, y_bytes = 0;
   if (!bytes_of(b_rows, k, &b_bytes) || !bytes_of(y_rows, k, &y_bytes))
     return fail(SB200_E_NOMEM, "spmm: the dense operand or result does not fit in device memory");
   if (m->nnz == 0 || b_rows == 0) {  // no stored entry: the zero matrix, as k calls of spmv give
-    SB_CUDA(cudaMemsetAsync(d_Y, 0, y_bytes, st));
+    SB_CUDA(cudaMemsetAsync(d_Yrm, 0, y_bytes, st));
     return SB200_OK;
   }
   // A B on a resident mirror: same ski-rental rule as A v (launch_sweep) — a k-wide call counts once
@@ -330,23 +335,37 @@ int launch_spmm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, 
   }
   const bool on_rows = !transposed && m->rows_state == 1;
   if (on_rows) m->rows->stream = st;
-  double *b_rm = nullptr, *y_rm = nullptr;
+  double* b_rm = nullptr;
   int rc = pool_alloc(reinterpret_cast<void**>(&b_rm), b_bytes, st);
-  if (rc == SB200_OK) rc = pool_alloc(reinterpret_cast<void**>(&y_rm), y_bytes, st);
   if (rc == SB200_OK) rc = launch_transpose(st, d_B, k, b_rows, b_rm);  // column-major b_rows x k -> row-major
   if (rc == SB200_OK) {
     if (transposed)
-      rc = gather_rm(m, b_rm, k, y_rm, st);
+      rc = gather_rm(m, b_rm, k, d_Yrm, st);
     else if (on_rows)
-      rc = gather_rm(m->rows, b_rm, k, y_rm, st);  // A B = (A^T)^T B on the row-ordered copy
+      rc = gather_rm(m->rows, b_rm, k, d_Yrm, st);  // A B = (A^T)^T B on the row-ordered copy
     else {
-      const cudaError_t e = cudaMemsetAsync(y_rm, 0, y_bytes, st);
-      rc = e == cudaSuccess ? launch_by_width<ScatterSel>(m, params_of(m, b_rm, k, y_rm), st)
+      const cudaError_t e = cudaMemsetAsync(d_Yrm, 0, y_bytes, st);
+      rc = e == cudaSuccess ? launch_by_width<ScatterSel>(m, params_of(m, b_rm, k, d_Yrm), st)
                             : cuda_fail(e, "cudaMemsetAsync", __FILE__, __LINE__);
     }
   }
-  if (rc == SB200_OK) rc = launch_transpose(st, y_rm, y_rows, k, d_Y);  // row-major y_rows x k -> column-major
   pool_free(b_rm, st);
+  if (rc == SB200_E_NOMEM) cudaGetLastError();  // a refused allocation leaves the stream usable
+  return rc;
+}
+
+int launch_spmm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, double* d_Y) {
+  const int64_t b_rows = transposed ? m->nrow : m->ncol;
+  const int64_t y_rows = transposed ? m->ncol : m->nrow;
+  // k <= 1 or no stored entry: the row-major result is the column-major one (n x 1, or all zeros)
+  if (k <= 1 || y_rows == 0 || m->nnz == 0 || b_rows == 0) return launch_spmm_rm(m, transposed, d_B, k, d_Y);
+  cudaStream_t st = m->stream;
+  size_t y_bytes = 0;
+  if (!bytes_of(y_rows, k, &y_bytes)) return fail(SB200_E_NOMEM, "spmm: the dense operand or result does not fit in device memory");
+  double* y_rm = nullptr;
+  int rc = pool_alloc(reinterpret_cast<void**>(&y_rm), y_bytes, st);
+  if (rc == SB200_OK) rc = launch_spmm_rm(m, transposed, d_B, k, y_rm);
+  if (rc == SB200_OK) rc = launch_transpose(st, y_rm, y_rows, k, d_Y);  // row-major y_rows x k -> column-major
   pool_free(y_rm, st);
   if (rc == SB200_E_NOMEM) cudaGetLastError();  // a refused allocation leaves the stream usable
   return rc;

@@ -383,6 +383,18 @@ class ShardedHostMatrix:
             raise ValueError("A^T v: v must have nrow entries")
         return self._vec(_lib.lib().sb200_sharded_spmv_t, self.ncol, _ptr(v))
 
+    # the same argument checks and column-major handling as the one-GPU block products
+    _spmm = DeviceMatrix._spmm
+
+    def spmm(self, B):
+        """A B for a dense (ncol, k) block on every GPU of the handle, as a Fortran-ordered (nrow, k) array
+        (sparse_b200.h sb200_sharded_spmm)."""
+        return self._spmm(_lib.lib().sb200_sharded_spmm, B, self.ncol, self.nrow, "A B")
+
+    def spmm_t(self, B):
+        """A^T B for a dense (nrow, k) block on every GPU of the handle, as a Fortran-ordered (ncol, k) array."""
+        return self._spmm(_lib.lib().sb200_sharded_spmm_t, B, self.nrow, self.ncol, "A^T B")
+
     def transpose_host(self):
         """CSC(A^T) of the whole matrix: local transposes on every GPU, row pieces exchanged over peer memory, every
         GPU copies its rows home (sparse_b200.h sb200_sharded_transpose; reference RcppSparse.h:375-385)."""
@@ -581,12 +593,12 @@ class Matrix:
     def spmv_t(self, v):
         return self._call(True, lambda m: m.spmv_t(v))
 
-    # ---- A B and A^T B for a dense block of k right-hand sides: additions, one device -------------------------------------
+    # ---- A B and A^T B for a dense block of k right-hand sides: additions ---------------------------------------------------
     def spmm(self, B):
-        return self._call(False, lambda m: m.spmm(B))
+        return self._call(True, lambda m: m.spmm(B))
 
     def spmm_t(self, B):
-        return self._call(False, lambda m: m.spmm_t(B))
+        return self._call(True, lambda m: m.spmm_t(B))
 
     # ---- RcppSparse.h:375-385 ---------------------------------------------------------------------------------------------
     def transpose(self) -> "Matrix":
