@@ -7,7 +7,7 @@
 //   constructors (4 vectors / S4 / default)                reference :33-42
 //   rows cols nrow ncol n_nonzero nonzeros innerIndexPtr outerIndexPtr InnerNNZs   :44-51, :357-359
 //   colSums rowSums colMeans rowMeans                      reference :131-156  -> sb200_col_sums ... sb200_row_means
-//   crossprod                                              reference :158-194  -> sb200_crossprod
+//   crossprod                                              reference :158-194  -> sb200_crossprod / sb200_sharded_crossprod
 //   transpose (and the vignette's t)                       reference :375-385  -> sb200_transpose / sb200_sharded_transpose
 //   wrap, clone, at, operator(), operator[]                reference :387-394, :54-73 (host side, unchanged semantics)
 //   InnerIterator                                          reference :218-233 (host side, unchanged)
@@ -15,7 +15,7 @@
 // Additions: spmv(v) = A v and spmv_t(v) = A^T v (the reference only has the iterator idiom), spmm(B) = A B and
 // spmm_t(B) = A^T B for a dense NumericMatrix of k right-hand sides (one sweep instead of k spmv calls),
 // resident() to keep the device mirror between calls (then refresh() after mutating x in place, release() to
-// drop it); SB200_GPUS=n runs the sweeps on n GPUs of this process (sb200_sharded_*).
+// drop it); SB200_GPUS=n runs the device ops on n GPUs of this process (sb200_sharded_*).
 //   dense copies (operator()(rows, cols), col, row), InnerIndices, emptyInnerIndices, isAppxSymmetric,
 //   InnerIteratorInRange / NotInRange, InnerRowIterator       reference :75-128, :196-216, :238-373 (host side; the
 //   row iterator and the symmetry test do what their interfaces promise — the reference's own walk is broken)
@@ -254,11 +254,12 @@ public:
     return means;
   }
 
-  // dense A^T A (reference :158-194): ncol x ncol, exactly symmetric -> sb200_crossprod
+  // dense A^T A (reference :158-194): ncol x ncol, exactly symmetric -> sb200_crossprod; on several GPUs
+  // sb200_sharded_crossprod, which adds in the reference's row order (its result bit for bit)
   Rcpp::NumericMatrix crossprod() {
     Rcpp::NumericMatrix res(Dim[1], Dim[1]);
-    Lease l(*this, false);
-    b200::check(sb200_crossprod(l.m, res.begin()));
+    Lease l(*this, true);
+    b200::check(l.s ? sb200_sharded_crossprod(l.s, res.begin()) : sb200_crossprod(l.m, res.begin()));
     return res;
   }
 
@@ -474,8 +475,8 @@ private:
   std::shared_ptr<b200::Mirror> mirror_;
 
   // The device handle(s) for one call: uploaded from the slots as they are now, dropped again at the end of the call
-  // unless the Matrix is resident.  multi = the op has a several-GPU form (the sweeps, the block products and the
-  // transpose; not crossprod).
+  // unless the Matrix is resident.  multi = the op has a several-GPU form (the sweeps, the block products, the
+  // transpose and crossprod).
   struct Lease {
     b200::Mirror& mm;
     sb200_matrix* m = nullptr;

@@ -271,6 +271,16 @@ int sb200_sharded_spmm_t(sb200_sharded* s, const double* B /* nrow x k */, int64
  * pieces exchanged over peer memory in block (= column) order, every device copies its rows home (SURVEY.md 8e).
  * Bit-exact like the one-GPU transpose.  Blocking. */
 int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out /* nrow + 1 */, int32_t* i_out /* nnz */, double* x_out /* nnz */);
+/* Matrix::crossprod() (RcppSparse.h:158-194) on every device of the handle: dense A^T A into the column-major host buffer
+ * `out`.  Every entry res(a, b) is the sum over rows r of x_ra * x_rb, from +0.0, added in ascending row order with no
+ * contraction and no atomics: the reference's result bit for bit (NaN payloads aside; NaN positions match), exactly
+ * symmetric, and the same bits run to run, for any n_gpus and any placement.  Device w computes the result columns of its
+ * block, a contiguous range of `out` (8 ncol ncol_w bytes of device memory, plus a 12 nnz byte row-ordered copy of the
+ * whole matrix built per call over peer memory), and copies it home over its own link.  ncol = 0 writes nothing; nnz = 0
+ * or nrow = 0 gives zeros.  A NULL `out` with ncol > 0 is SB200_E_INVALID; device memory that does not fit is
+ * SB200_E_NOMEM before anything is written (the handle stays usable).  Devices are ordered by CUDA events and host
+ * synchronisation only, so blocks may share a device.  Blocking. */
+int sb200_sharded_crossprod(sb200_sharded* s, double* out /* ncol*ncol, column-major, host */);
 
 /* Scratch, results and cached layouts come from the device's stream-ordered memory pool, which keeps freed blocks
  * for reuse (a multi-GB cudaMalloc/cudaFree pair costs as much as a sweep).  sb200_trim synchronises the device and

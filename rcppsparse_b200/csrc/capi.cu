@@ -209,6 +209,18 @@ int build_row_companion(sb200_matrix* m) {
   return SB200_OK;
 }
 
+const sb200_matrix* crossprod_row_copy(sb200_matrix* m) {
+  if (m->owns_arrays && m->rows_state != 1) {
+    const int keep = m->rows_state;
+    m->rows_state = 0;
+    build_row_companion(m);
+    if (m->rows_state != 1) m->rows_state = keep;
+  }
+  if (m->rows_state != 1) return nullptr;
+  m->rows->stream = m->stream;
+  return m->rows;
+}
+
 int finish_matrix(sb200_matrix* m, unsigned flags) {
   SB_TRY(enqueue_finish(m, flags));
   SB_CUDA(cudaStreamSynchronize(m->stream));
@@ -679,16 +691,7 @@ static int crossprod_into(sb200_matrix* m, double* d_res) {
       SB_CUDA(cudaMemsetAsync(d_res, 0, sizeof(double) * static_cast<size_t>(m->ncol) * static_cast<size_t>(m->ncol), m->stream));
     return SB200_OK;
   }
-  if (m->owns_arrays && m->rows_state != 1) {
-    const int keep = m->rows_state;
-    m->rows_state = 0;
-    build_row_companion(m);
-    if (m->rows_state != 1) m->rows_state = keep;
-  }
-  if (m->rows_state == 1) {
-    m->rows->stream = m->stream;
-    return launch_crossprod(m->rows, m->ncol, d_res, m->stream);
-  }
+  if (const sb200_matrix* rows = crossprod_row_copy(m)) return launch_crossprod(rows, m->ncol, d_res, m->stream);
   sb200_matrix* t = nullptr;
   SB_TRY(alloc_matrix(m->device, m->ncol, m->nrow, m->nnz, &t));
   cudaStreamSynchronize(t->stream);

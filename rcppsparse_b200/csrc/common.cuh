@@ -174,6 +174,11 @@ int staged_h2d_2d(int device, void* d_dst, size_t dpitch, const void* h_src, siz
 int staged_d2h_2d(int device, void* h_dst, size_t hpitch, const void* d_src, size_t dpitch, size_t width, size_t runs);
 constexpr size_t STAGED_COPY_MIN_BYTES = 32u << 20;  // below this the driver's own staging is as good
 int launch_crossprod(const sb200_matrix* T, int32_t ncol_a, double* d_res, cudaStream_t st);  // crossprod.cu
+// crossprod.cu: slab (ncol x blk->ncol, column-major) = A^T A_blk in ascending row order, on blk's stream; rp / rc / rv are
+// the row-ordered copy of the WHOLE matrix (global column ids) on blk's device
+int launch_crossprod_slab(const sb200_matrix* blk, const int32_t* rp, const int32_t* rc, const double* rv, int64_t ncol, double* slab);
+// capi.cu: the row-ordered copy crossprod runs on, built now if the mirror owns its arrays and has room (null if not)
+const sb200_matrix* crossprod_row_copy(sb200_matrix* m);
 // spmm.cu: d_Y = A d_B (transposed = false) or A^T d_B, k right-hand sides, both column-major; k = 1 is launch_sweep
 int launch_spmm(sb200_matrix* m, bool transposed, const double* d_B, int64_t k, double* d_Y);
 // the same up to the final transpose: d_Yrm is ROW-major (y_rows x k); a block without entries or columns gives zeros

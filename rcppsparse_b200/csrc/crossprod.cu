@@ -8,7 +8,9 @@
 // column pair.  Only the upper triangle is accumulated; a tiled mirror pass then copies it below the diagonal,
 // so the result is exactly symmetric like the reference's (which assigns res(col2, col1) = res(col1, col2)).
 // The order of the additions inside one entry is not the reference's ascending-row order: results agree within
-// the 1e-12 * sum|terms| bar, not bitwise.
+// the 1e-12 * sum|terms| bar, not bitwise.  The sharded form (crossprod_slab_kernel below) keeps that order instead.
+#include <algorithm>
+
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -71,7 +73,111 @@ __global__ void __launch_bounds__(256) mirror_upper_kernel(double* __restrict__ 
   }
 }
 
+// ---- the ordered column sweep of the sharded crossprod (sharded.cu, sb200_sharded_crossprod) ------------------------
+// slab(a, b) = sum over the rows r of column b, in ascending r, of x_ra * x_rb, from +0.0 with __dmul_rn / __dadd_rn:
+// the reference's order of additions (RcppSparse.h:178-188), so res(a, b) and res(b, a) come out bitwise equal.
+// A warp owns (local column b, output rows [a0, a0 + SLAB_SPAN)) with that span's accumulators in shared memory.  It
+// takes column b's entries 32 rows at a time: every lane binary-searches its row of the whole-matrix row-ordered copy
+// for the piece inside the span and prefetches up to SLAB_PREFETCH of its entries; then the rows are applied one after
+// another, lanes on distinct slots, a __syncwarp between rows.  The span is stored once, coalesced: no memset.
+constexpr int SLAB_THREADS = 256;
+constexpr int SLAB_WARPS = SLAB_THREADS / 32;
+constexpr int SLAB_SPAN = 512;      // accumulators per warp (32 KB per CTA)
+constexpr int SLAB_PREFETCH = 2;    // entries of a row's piece that travel in registers; longer pieces are read in the apply
+
+__device__ __forceinline__ int32_t lower_bound_i32(const int32_t* __restrict__ a, int32_t lo, int32_t hi, int32_t key) {
+  while (lo < hi) {
+    const int32_t mid = lo + ((hi - lo) >> 1);
+    if (__ldg(a + mid) < key)
+      lo = mid + 1;
+    else
+      hi = mid;
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(SLAB_THREADS) crossprod_slab_kernel(const int32_t* __restrict__ bp, const int32_t* __restrict__ bi,
+                                                                     const double* __restrict__ bx, int64_t ncol_w,
+                                                                     const int32_t* __restrict__ rp, const int32_t* __restrict__ rc,
+                                                                     const double* __restrict__ rv, int64_t ncol,
+                                                                     double* __restrict__ slab) {
+  __shared__ double s_acc[SLAB_WARPS][SLAB_SPAN];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  double* acc = s_acc[warp];
+  const int64_t spans = (ncol + SLAB_SPAN - 1) / SLAB_SPAN;
+  const int64_t warps_total = static_cast<int64_t>(gridDim.x) * SLAB_WARPS;
+  for (int64_t task = static_cast<int64_t>(blockIdx.x) * SLAB_WARPS + warp; task < ncol_w * spans; task += warps_total) {
+    const int64_t b = task / spans;
+    const int64_t a0 = (task % spans) * SLAB_SPAN;
+    const int32_t lo_key = static_cast<int32_t>(a0);
+    const int32_t width = static_cast<int32_t>(ncol - a0 < SLAB_SPAN ? ncol - a0 : SLAB_SPAN);
+    const int32_t hi_key = lo_key + width;
+    for (int t = lane; t < SLAB_SPAN; t += 32) acc[t] = 0.0;
+    __syncwarp();
+    const int32_t e0 = __ldg(bp + b), e1 = __ldg(bp + b + 1);
+    for (int32_t base = e0; base < e1; base += 32) {
+      int32_t lo = 0, hi = 0;
+      double xb = 0.0;
+      int32_t pc[SLAB_PREFETCH];
+      double pv[SLAB_PREFETCH];
+#pragma unroll
+      for (int u = 0; u < SLAB_PREFETCH; ++u) {
+        pc[u] = 0;
+        pv[u] = 0.0;
+      }
+      if (base + lane < e1) {
+        const int32_t r = __ldg(bi + base + lane);
+        xb = __ldg(bx + base + lane);
+        const int32_t s0 = __ldg(rp + r), s1 = __ldg(rp + r + 1);
+        lo = lower_bound_i32(rc, s0, s1, lo_key);
+        hi = lower_bound_i32(rc, lo, lo + min(s1 - lo, width), hi_key);  // at most `width` distinct columns fall inside
+#pragma unroll
+        for (int u = 0; u < SLAB_PREFETCH; ++u)
+          if (lo + u < hi) {
+            pc[u] = __ldg(rc + lo + u) - lo_key;
+            pv[u] = __ldg(rv + lo + u);
+          }
+      }
+      const int rows = min(32, e1 - base);
+      for (int j = 0; j < rows; ++j) {  // ascending r: the rows of a column are sorted
+        const int32_t lj = __shfl_sync(0xffffffffu, lo, j);
+        const int32_t n = __shfl_sync(0xffffffffu, hi, j) - lj;
+        const double xj = __shfl_sync(0xffffffffu, xb, j);
+        if (n == 0) continue;  // uniform: the piece of row j misses the span
+        if (n <= SLAB_PREFETCH) {
+#pragma unroll
+          for (int u = 0; u < SLAB_PREFETCH; ++u) {
+            const int32_t c = __shfl_sync(0xffffffffu, pc[u], j);
+            const double v = __shfl_sync(0xffffffffu, pv[u], j);
+            if (lane == u && u < n) acc[c] = __dadd_rn(acc[c], __dmul_rn(v, xj));
+          }
+        } else {
+          for (int32_t t = lj + lane; t < lj + n; t += 32) {
+            const int32_t c = __ldg(rc + t) - lo_key;
+            acc[c] = __dadd_rn(acc[c], __dmul_rn(__ldg(rv + t), xj));
+          }
+        }
+        __syncwarp();  // the next row may add to the same slots
+      }
+    }
+    double* out = slab + b * ncol + a0;
+    for (int t = lane; t < width; t += 32) out[t] = acc[t];
+    __syncwarp();
+  }
+}
+
 }  // namespace
+
+int launch_crossprod_slab(const sb200_matrix* blk, const int32_t* rp, const int32_t* rc, const double* rv, int64_t ncol, double* slab) {
+  if (blk->ncol == 0 || ncol == 0) return SB200_OK;
+  const int64_t tasks = static_cast<int64_t>(blk->ncol) * ((ncol + SLAB_SPAN - 1) / SLAB_SPAN);
+  const int64_t blocks = std::min<int64_t>((tasks + SLAB_WARPS - 1) / SLAB_WARPS, static_cast<int64_t>(blk->sm_count) * 8);
+  crossprod_slab_kernel<<<static_cast<unsigned>(blocks), SLAB_THREADS, 0, blk->stream>>>(blk->d_p, blk->d_i, blk->d_x, blk->ncol, rp, rc,
+                                                                                          rv, ncol, slab);
+  count_launch();
+  SB_CUDA(cudaGetLastError());
+  return SB200_OK;
+}
 
 // T = the row-ordered copy of the mirror (its "columns" are the rows of A, its i the column ids of A)
 int launch_crossprod(const sb200_matrix* T, int32_t ncol_a, double* d_res, cudaStream_t st) {

@@ -213,6 +213,116 @@ __global__ void __launch_bounds__(256) push_rows_local_kernel(const PushRowsSrc 
   push_rows_body(a, world, d);
 }
 
+// Whole rows from the blocks' row-ordered copies, shared by the sharded transpose (rows dealt to owners) and the sharded
+// crossprod (every row to every device).  T[k] is block k's row-ordered copy on its device (local column ids), or null
+// for a block without entries.  count(): row counts over the blocks, scanned into the whole matrix's row pointer P on
+// device 0 and copied to the host.  offsets(rb): where every block's piece of every row starts in the arrays of the
+// row's owner (rows [rb[q], rb[q+1]) belong to owner q, relative to the owner's first row), on the block's device.
+// push(rb, d): every block pushes its pieces into the owners' arrays d over peer memory, asynchronously on its stream;
+// block order is column order inside a row, so the rows come out as the one-GPU transpose has them.
+struct RowExchange {
+  sb200_sharded* s;
+  std::vector<const sb200_matrix*> T;
+  TpPtrs tp{};
+  int32_t* tpc = nullptr;  // device 0: copies of every block's row pointer
+  uint32_t* cnt = nullptr;
+  int32_t* P = nullptr;
+  void* ws = nullptr;
+  int64_t* dst = nullptr;
+  std::vector<int64_t*> dstk;  // device k: its slice of dst
+  RowExchange(sb200_sharded* sh, std::vector<const sb200_matrix*> t) : s(sh), T(std::move(t)), dstk(sh->world, nullptr) {}
+  ~RowExchange() {  // released on every way out, once nothing reads it any more
+    for (int k = s->world - 1; k >= 0; --k) {
+      DeviceGuard g(s->blocks[k]->device);
+      cudaStreamSynchronize(s->blocks[k]->stream);
+      if (k > 0) pool_free(dstk[k], s->blocks[k]->stream);
+    }
+    cudaStream_t st0 = s->blocks[0]->stream;
+    DeviceGuard g(s->blocks[0]->device);
+    pool_free(tpc, st0);
+    pool_free(cnt, st0);
+    pool_free(P, st0);
+    pool_free(ws, st0);
+    pool_free(dst, st0);
+    cudaGetLastError();
+  }
+  unsigned grid() const { return static_cast<unsigned>(std::min<int64_t>((static_cast<int64_t>(s->nrow) + 255) / 256, 4096)); }
+
+  int count(int32_t* p_host) {
+    const int W = s->world;
+    const int32_t nrow = s->nrow;
+    sb200_matrix* m0 = s->blocks[0];
+    cudaStream_t st0 = m0->stream;
+    DeviceGuard g(m0->device);
+    // the library's arrays are pool memory, which peers cannot address: bring the (small) row pointers to device 0
+    const size_t pb = sizeof(int32_t) * (static_cast<size_t>(nrow) + 1);
+    SB_TRY(pool_alloc(reinterpret_cast<void**>(&tpc), pb * W, st0));
+    for (int k = 0; k < PUSH_MAX_RANKS; ++k) tp.p[k] = k < W ? tpc + static_cast<size_t>(k) * (nrow + 1) : nullptr;
+    for (int k = 0; k < W; ++k) {
+      int32_t* to = tpc + static_cast<size_t>(k) * (nrow + 1);
+      if (T[k])
+        SB_CUDA(cudaMemcpyPeerAsync(to, m0->device, T[k]->d_p, s->blocks[k]->device, pb, st0));
+      else
+        SB_CUDA(cudaMemsetAsync(to, 0, pb, st0));
+    }
+    const size_t ws_bytes = scan_workspace_bytes(nrow);
+    SB_TRY(pool_alloc(reinterpret_cast<void**>(&cnt), sizeof(uint32_t) * static_cast<size_t>(nrow), st0));
+    SB_TRY(pool_alloc(reinterpret_cast<void**>(&P), sizeof(int32_t) * (static_cast<size_t>(nrow) + 1), st0));
+    SB_TRY(pool_alloc(&ws, ws_bytes, st0));
+    shard_row_counts_kernel<<<grid(), 256, 0, st0>>>(tp, W, nrow, cnt);
+    count_launch();
+    SB_CUDA(cudaGetLastError());
+    SB_TRY(exclusive_scan_u32(st0, cnt, P, nrow, nullptr, ws, ws_bytes));
+    SB_CUDA(cudaMemcpyAsync(p_host, P, sizeof(int32_t) * (static_cast<size_t>(nrow) + 1), cudaMemcpyDeviceToHost, st0));
+    SB_CUDA(cudaStreamSynchronize(st0));
+    if (p_host[nrow] != s->nnz) return fail(SB200_E_CUDA, "sharded rows: the blocks' row counts do not add up to nnz");
+    return SB200_OK;
+  }
+
+  int offsets(const RowBounds& rb) {
+    const int W = s->world;
+    const int32_t nrow = s->nrow;
+    sb200_matrix* m0 = s->blocks[0];
+    {
+      DeviceGuard g(m0->device);
+      SB_TRY(pool_alloc(reinterpret_cast<void**>(&dst), sizeof(int64_t) * static_cast<size_t>(W) * nrow, m0->stream));
+      shard_row_dst_kernel<<<grid(), 256, 0, m0->stream>>>(tp, W, nrow, P, rb, dst);
+      count_launch();
+      SB_CUDA(cudaGetLastError());
+      SB_CUDA(cudaStreamSynchronize(m0->stream));
+    }
+    dstk[0] = dst;
+    for (int k = 1; k < W; ++k) {
+      DeviceGuard gk(s->blocks[k]->device);
+      SB_TRY(pool_alloc(reinterpret_cast<void**>(&dstk[k]), sizeof(int64_t) * static_cast<size_t>(nrow), s->blocks[k]->stream));
+      SB_CUDA(cudaMemcpyPeerAsync(dstk[k], s->blocks[k]->device, dst + static_cast<int64_t>(k) * nrow, m0->device,
+                                  sizeof(int64_t) * static_cast<size_t>(nrow), s->blocks[k]->stream));
+    }
+    return SB200_OK;
+  }
+
+  int push(const RowBounds& rb, const PtrDest& pd) {
+    for (int k = 0; k < s->world; ++k) {
+      if (!T[k]) continue;
+      DeviceGuard gk(s->blocks[k]->device);
+      PushRowsSrc a;
+      a.p_loc = T[k]->d_p;
+      a.cols = T[k]->d_i;
+      a.vals = T[k]->d_x;
+      a.dst_off = dstk[k];
+      a.nrow = s->nrow;
+      a.col_offset = static_cast<int32_t>(s->bounds[k]);
+      for (int q = 0; q <= PUSH_MAX_RANKS; ++q) a.rb[q] = rb.rb[q];
+      int64_t blocks = ((static_cast<int64_t>(s->nrow) + 31) / 32 + 7) / 8;
+      if (blocks > 592) blocks = 592;
+      push_rows_local_kernel<<<static_cast<unsigned>(blocks), 256, 0, s->blocks[k]->stream>>>(a, s->world, pd);
+      count_launch();
+      SB_CUDA(cudaGetLastError());
+    }
+    return SB200_OK;
+  }
+};
+
 // ---- k-wide products: the rank-ordered reduce of the row-major partials ------------------------------------------------
 struct PartialPtrs {
   const double* p[PUSH_MAX_RANKS];  // the blocks' row-major nrow x k partials (peer-readable)
@@ -711,16 +821,10 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
       });
     for (auto& w : workers) w.join();
   }
-  struct Scratch {  // everything below is released on every way out
+  struct Scratch {  // the local transposes and the owners' arrays are released on every way out
     std::vector<sb200_matrix*>& T;
     sb200_sharded* s;
-    uint32_t* cnt = nullptr;
-    int32_t* P = nullptr;
-    void* ws = nullptr;
-    int64_t* dst = nullptr;
-    int32_t* tpc = nullptr;          // device 0: copies of every block's row pointer
-    std::vector<int64_t*> dstk;      // device k: its slice of dst
-    std::vector<int32_t*> oc;        // the owners' arrays: plain cudaMalloc, visible to the peers (pool memory is not)
+    std::vector<int32_t*> oc;  // the owners' arrays: plain cudaMalloc, visible to the peers (pool memory is not)
     std::vector<double*> ov;
     ~Scratch() {
       for (int k = 0; k < s->world; ++k) {
@@ -728,14 +832,6 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
         cudaStreamSynchronize(s->blocks[k]->stream);
         if (k < static_cast<int>(oc.size()) && oc[k]) cudaFree(oc[k]);
         if (k < static_cast<int>(ov.size()) && ov[k]) cudaFree(ov[k]);
-        if (k > 0 && k < static_cast<int>(dstk.size())) pool_free(dstk[k], s->blocks[k]->stream);
-        if (k == 0) {
-          pool_free(tpc, s->blocks[0]->stream);
-          pool_free(cnt, s->blocks[0]->stream);
-          pool_free(P, s->blocks[0]->stream);
-          pool_free(ws, s->blocks[0]->stream);
-          pool_free(dst, s->blocks[0]->stream);
-        }
         if (T[k]) sb200_matrix_destroy(T[k]);
       }
       cudaGetLastError();
@@ -744,61 +840,28 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
   lap("local transposes");
   for (int k = 0; k < W; ++k)
     if (rcs[k] != SB200_OK) return fail(rcs[k], "sharded transpose, column block " + std::to_string(k) + ": " + errs[k]);
-  // 2. row counts over the blocks -> p_out (device 0)
-  sb200_matrix* m0 = s->blocks[0];
-  cudaStream_t st0 = m0->stream;
-  TpPtrs tp;
-  const size_t ws_bytes = scan_workspace_bytes(nrow);
+  // 2. row counts over the blocks -> p_out
+  RowExchange rx(s, std::vector<const sb200_matrix*>(T.begin(), T.end()));
+  SB_TRY(rx.count(p_out));
+  lap("row counts, scan, p_out");
+  // 3. rows dealt to the devices: nnz-balanced contiguous ranges
+  RowBounds rb;
+  rb.rb[0] = 0;
+  for (int q = 1; q < W; ++q) {
+    const int64_t target = (s->nnz * q) / W;
+    int32_t lo = rb.rb[q - 1], hi = nrow;
+    while (lo < hi) {
+      const int32_t mid = lo + ((hi - lo) >> 1);
+      if (p_out[mid] < target)
+        lo = mid + 1;
+      else
+        hi = mid;
+    }
+    rb.rb[q] = lo;
+  }
+  for (int q = W; q <= PUSH_MAX_RANKS; ++q) rb.rb[q] = nrow;
+  SB_TRY(rx.offsets(rb));
   {
-    DeviceGuard g(m0->device);
-    // the library's arrays are pool memory, which peers cannot address: bring the (small) row pointers to device 0
-    const size_t pb = sizeof(int32_t) * (static_cast<size_t>(nrow) + 1);
-    SB_TRY(pool_alloc(reinterpret_cast<void**>(&sc.tpc), pb * W, st0));
-    for (int k = 0; k < PUSH_MAX_RANKS; ++k) tp.p[k] = k < W ? sc.tpc + static_cast<size_t>(k) * (nrow + 1) : nullptr;
-    for (int k = 0; k < W; ++k)
-      SB_CUDA(cudaMemcpyPeerAsync(sc.tpc + static_cast<size_t>(k) * (nrow + 1), m0->device, T[k]->d_p, s->blocks[k]->device, pb, st0));
-    SB_TRY(pool_alloc(reinterpret_cast<void**>(&sc.cnt), sizeof(uint32_t) * static_cast<size_t>(nrow), st0));
-    SB_TRY(pool_alloc(reinterpret_cast<void**>(&sc.P), sizeof(int32_t) * (static_cast<size_t>(nrow) + 1), st0));
-    SB_TRY(pool_alloc(&sc.ws, ws_bytes, st0));
-    SB_TRY(pool_alloc(reinterpret_cast<void**>(&sc.dst), sizeof(int64_t) * static_cast<size_t>(W) * nrow, st0));
-    const unsigned grid = static_cast<unsigned>(std::min<int64_t>((static_cast<int64_t>(nrow) + 255) / 256, 4096));
-    shard_row_counts_kernel<<<grid, 256, 0, st0>>>(tp, W, nrow, sc.cnt);
-    count_launch();
-    SB_CUDA(cudaGetLastError());
-    SB_TRY(exclusive_scan_u32(st0, sc.cnt, sc.P, nrow, nullptr, sc.ws, ws_bytes));
-    SB_CUDA(cudaMemcpyAsync(p_out, sc.P, sizeof(int32_t) * (static_cast<size_t>(nrow) + 1), cudaMemcpyDeviceToHost, st0));
-    SB_CUDA(cudaStreamSynchronize(st0));
-    lap("row counts, scan, p_out");
-    if (p_out[nrow] != s->nnz) return fail(SB200_E_CUDA, "sharded transpose: the blocks' row counts do not add up to nnz");
-    // 3. rows dealt to the devices: nnz-balanced contiguous ranges
-    RowBounds rb;
-    rb.rb[0] = 0;
-    for (int q = 1; q < W; ++q) {
-      const int64_t target = (s->nnz * q) / W;
-      int32_t lo = rb.rb[q - 1], hi = nrow;
-      while (lo < hi) {
-        const int32_t mid = lo + ((hi - lo) >> 1);
-        if (p_out[mid] < target)
-          lo = mid + 1;
-        else
-          hi = mid;
-      }
-      rb.rb[q] = lo;
-    }
-    for (int q = W; q <= PUSH_MAX_RANKS; ++q) rb.rb[q] = nrow;
-    shard_row_dst_kernel<<<grid, 256, 0, st0>>>(tp, W, nrow, sc.P, rb, sc.dst);
-    count_launch();
-    SB_CUDA(cudaGetLastError());
-    SB_CUDA(cudaStreamSynchronize(st0));
-    // every device gets its slice of dst
-    sc.dstk.assign(W, nullptr);
-    sc.dstk[0] = sc.dst;
-    for (int k = 1; k < W; ++k) {
-      DeviceGuard gk(s->blocks[k]->device);
-      SB_TRY(pool_alloc(reinterpret_cast<void**>(&sc.dstk[k]), sizeof(int64_t) * static_cast<size_t>(nrow), s->blocks[k]->stream));
-      SB_CUDA(cudaMemcpyPeerAsync(sc.dstk[k], s->blocks[k]->device, sc.dst + static_cast<int64_t>(k) * nrow, m0->device,
-                                  sizeof(int64_t) * static_cast<size_t>(nrow), s->blocks[k]->stream));
-    }
     // 4. the owners' arrays
     sc.oc.assign(W, nullptr);
     sc.ov.assign(W, nullptr);
@@ -814,22 +877,7 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
       pd.c[q] = q < W ? sc.oc[q] : nullptr;
       pd.v[q] = q < W ? sc.ov[q] : nullptr;
     }
-    for (int k = 0; k < W; ++k) {
-      DeviceGuard gk(s->blocks[k]->device);
-      PushRowsSrc a;
-      a.p_loc = T[k]->d_p;
-      a.cols = T[k]->d_i;
-      a.vals = T[k]->d_x;
-      a.dst_off = sc.dstk[k];
-      a.nrow = nrow;
-      a.col_offset = static_cast<int32_t>(s->bounds[k]);
-      for (int q = 0; q <= PUSH_MAX_RANKS; ++q) a.rb[q] = rb.rb[q];
-      int64_t blocks = ((static_cast<int64_t>(nrow) + 31) / 32 + 7) / 8;
-      if (blocks > 592) blocks = 592;
-      push_rows_local_kernel<<<static_cast<unsigned>(blocks), 256, 0, s->blocks[k]->stream>>>(a, W, pd);
-      count_launch();
-      SB_CUDA(cudaGetLastError());
-    }
+    SB_TRY(rx.push(rb, pd));
     for (int k = 0; k < W; ++k) {
       DeviceGuard gk(s->blocks[k]->device);
       SB_CUDA(cudaStreamSynchronize(s->blocks[k]->stream));
@@ -863,6 +911,178 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
     lap("copies to the host");
     for (int q = 0; q < W; ++q)
       if (drc[q] != SB200_OK) return fail(drc[q], "sharded transpose: copying rows of device " + std::to_string(q) + " to the host failed");
+  }
+  return SB200_OK;
+}
+
+// Matrix::crossprod() (RcppSparse.h:158-194): block w computes the full-height slab A^T A_w, result columns
+// [bounds[w], bounds[w+1]), which is one contiguous range of the column-major `out`.  Its columns need every whole row that
+// has an entry in them, so every block first gets the row-ordered copy of the whole matrix: the blocks' own row-ordered
+// copies, their pieces of every row pushed over peer memory into every block's copy (plain cudaMalloc: peers write it).
+// The ordered sweep (crossprod.cu, crossprod_slab_kernel) adds every entry in ascending row order, so the result is the
+// reference's bit for bit, exactly symmetric, and the same for every split and placement.  Slabs go home from one
+// thread per block.
+int sb200_sharded_crossprod(sb200_sharded* s, double* out) {
+  SB_TRY(check_sharded(s));
+  const int W = s->world;
+  const int64_t nrow = s->nrow, ncol = s->ncol, nnz = s->nnz;
+  if (ncol == 0) return SB200_OK;
+  if (!out) return fail(SB200_E_INVALID, "output buffer is NULL");
+  if (nnz == 0 || nrow == 0) {  // no products at all: the zero matrix
+    for (int64_t c = 0; c < ncol; ++c) memset(out + c * ncol, 0, sizeof(double) * static_cast<size_t>(ncol));
+    return SB200_OK;
+  }
+  WallTrace tr("sharded crossprod");
+  DeviceGuard restore(s->blocks[0]->device);
+  auto ncol_w = [&](int w) { return s->bounds[w + 1] - s->bounds[w]; };
+  // 0. every device must hold the slabs and whole-matrix copies of the blocks it carries
+  {
+    std::vector<int> seen;
+    for (int w = 0; w < W; ++w) {
+      const int dev = s->blocks[w]->device;
+      if (std::find(seen.begin(), seen.end(), dev) != seen.end()) continue;
+      seen.push_back(dev);
+      double need = 0.0;
+      for (int v = 0; v < W; ++v)
+        if (s->blocks[v]->device == dev && ncol_w(v) > 0)
+          need += 8.0 * static_cast<double>(ncol) * static_cast<double>(ncol_w(v)) + 12.0 * static_cast<double>(nnz) +
+                  4.0 * static_cast<double>(nrow + 1) + 4096.0;
+      DeviceGuard g(dev);
+      if (need > static_cast<double>(device_free_bytes()))
+        return fail(SB200_E_NOMEM, "sharded crossprod: the result slabs (8 ncol ncol_w bytes) and row-ordered copies of the blocks on device " +
+                                       std::to_string(dev) + " do not fit");
+    }
+  }
+  struct Scratch {  // released on every way out, after every stream is done with it
+    sb200_sharded* s;
+    std::vector<sb200_matrix*> tmp;  // temporary row-ordered copies (blocks that keep none)
+    std::vector<int32_t*> rp, rc;    // every block's copy of the whole matrix's rows
+    std::vector<double*> rv, slab;
+    ~Scratch() {
+      for (int w = 0; w < s->world; ++w) {
+        sb200_matrix* m = s->blocks[w];
+        DeviceGuard g(m->device);
+        cudaStreamSynchronize(m->stream);
+        if (rc[w]) cudaFree(rc[w]);
+        if (rv[w]) cudaFree(rv[w]);
+        pool_free(rp[w], m->stream);
+        pool_free(slab[w], m->stream);
+        if (tmp[w]) sb200_matrix_destroy(tmp[w]);
+      }
+      cudaGetLastError();
+    }
+  } sc{s, std::vector<sb200_matrix*>(W, nullptr), std::vector<int32_t*>(W, nullptr), std::vector<int32_t*>(W, nullptr),
+       std::vector<double*>(W, nullptr), std::vector<double*>(W, nullptr)};
+  // 1. the blocks' row-ordered copies: the one a block keeps (built now where it fits, as sb200_crossprod does), else
+  //    a temporary transpose
+  std::vector<const sb200_matrix*> T(W, nullptr);
+  SB_TRY(on_every_block(s, "sharded crossprod: row-ordered copy", [&](int w) {
+    sb200_matrix* m = s->blocks[w];
+    if (m->nnz == 0) return SB200_OK;
+    if ((T[w] = crossprod_row_copy(m))) return SB200_OK;
+    SB_TRY(sb200_transpose_dev(m, &sc.tmp[w]));
+    T[w] = sc.tmp[w];
+    return SB200_OK;
+  }));
+  tr.phase("row-ordered copies");
+  // 2. the whole matrix's row pointer, and where every block's piece of every row starts in it
+  RowExchange rx(s, T);
+  std::vector<int32_t> P(static_cast<size_t>(nrow) + 1);
+  SB_TRY(rx.count(P.data()));
+  RowBounds all;  // one owner of every row: each block's copy holds them all
+  all.rb[0] = 0;
+  for (int q = 1; q <= PUSH_MAX_RANKS; ++q) all.rb[q] = static_cast<int32_t>(nrow);
+  SB_TRY(rx.offsets(all));
+  // 3. every block's copy and slab
+  int rc = SB200_OK;
+  for (int w = 0; w < W && rc == SB200_OK; ++w) {
+    if (ncol_w(w) == 0) continue;
+    sb200_matrix* m = s->blocks[w];
+    DeviceGuard g(m->device);
+    if (cudaMalloc(reinterpret_cast<void**>(&sc.rc[w]), padded_bytes(sizeof(int32_t) * static_cast<size_t>(nnz))) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&sc.rv[w]), padded_bytes(sizeof(double) * static_cast<size_t>(nnz))) != cudaSuccess) {
+      cudaGetLastError();
+      rc = fail(SB200_E_NOMEM, "sharded crossprod: the row-ordered copy does not fit on device " + std::to_string(m->device));
+      break;
+    }
+    rc = pool_alloc(reinterpret_cast<void**>(&sc.rp[w]), sizeof(int32_t) * static_cast<size_t>(nrow + 1), m->stream);
+    if (rc == SB200_OK)
+      rc = pool_alloc(reinterpret_cast<void**>(&sc.slab[w]), sizeof(double) * static_cast<size_t>(ncol) * static_cast<size_t>(ncol_w(w)),
+                      m->stream);
+    if (rc != SB200_OK) {
+      cudaGetLastError();
+      rc = fail(SB200_E_NOMEM, "sharded crossprod: the result slab of block " + std::to_string(w) + " does not fit on device " +
+                                   std::to_string(m->device));
+    }
+  }
+  if (rc != SB200_OK) return rc;
+  tr.phase("scratch");
+  // 4. the device part: the gather, then the ordered sweep (SB200_TRACE: CUDA-event time per device)
+  std::vector<cudaEvent_t> t0(W, nullptr), t1(W, nullptr);
+  struct Events {
+    sb200_sharded* s;
+    std::vector<cudaEvent_t>& a;
+    std::vector<cudaEvent_t>& b;
+    ~Events() {
+      for (int w = 0; w < s->world; ++w) {
+        DeviceGuard g(s->blocks[w]->device);
+        if (a[w]) cudaEventDestroy(a[w]);
+        if (b[w]) cudaEventDestroy(b[w]);
+      }
+    }
+  } ev{s, t0, t1};
+  for (int w = 0; w < W && tr.on; ++w) {
+    DeviceGuard g(s->blocks[w]->device);
+    SB_CUDA(cudaEventCreate(&t0[w]));
+    SB_CUDA(cudaEventCreate(&t1[w]));
+    SB_CUDA(cudaEventRecord(t0[w], s->blocks[w]->stream));
+  }
+  for (int w = 0; w < W; ++w) {
+    if (ncol_w(w) == 0) continue;
+    sb200_matrix* m0 = s->blocks[0];
+    DeviceGuard g(s->blocks[w]->device);
+    SB_CUDA(cudaMemcpyPeerAsync(sc.rp[w], s->blocks[w]->device, rx.P, m0->device, sizeof(int32_t) * static_cast<size_t>(nrow + 1),
+                                s->blocks[w]->stream));
+    PtrDest pd{};
+    pd.c[0] = sc.rc[w];
+    pd.v[0] = sc.rv[w];
+    SB_TRY(rx.push(all, pd));
+  }
+  for (int w = 0; w < W; ++w) {  // every piece has landed in every copy
+    DeviceGuard g(s->blocks[w]->device);
+    SB_CUDA(cudaStreamSynchronize(s->blocks[w]->stream));
+  }
+  tr.phase("rows gathered");
+  for (int w = 0; w < W; ++w) {
+    DeviceGuard g(s->blocks[w]->device);
+    SB_TRY(launch_crossprod_slab(s->blocks[w], sc.rp[w], sc.rc[w], sc.rv[w], ncol, sc.slab[w]));
+    if (tr.on) SB_CUDA(cudaEventRecord(t1[w], s->blocks[w]->stream));
+  }
+  tr.phase("launched");
+  // 5. every slab home over its block's own link
+  SB_TRY(on_every_block(s, "sharded crossprod: result download", [&](int w) {
+    sb200_matrix* m = s->blocks[w];
+    const size_t bytes = sizeof(double) * static_cast<size_t>(ncol) * static_cast<size_t>(ncol_w(w));
+    if (bytes == 0) return SB200_OK;
+    double* host = out + s->bounds[w] * ncol;
+    SB_CUDA(cudaStreamSynchronize(m->stream));
+    if (bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(host)) return staged_d2h(m->device, host, sc.slab[w], bytes);
+    SB_CUDA(cudaMemcpyAsync(host, sc.slab[w], bytes, cudaMemcpyDeviceToHost, m->stream));
+    SB_CUDA(cudaStreamSynchronize(m->stream));
+    return SB200_OK;
+  }));
+  tr.phase("results home");
+  if (tr.on) {
+    std::string per;
+    float worst = 0.0f;
+    for (int w = 0; w < W; ++w) {
+      DeviceGuard g(s->blocks[w]->device);
+      float ms = 0.0f;
+      cudaEventElapsedTime(&ms, t0[w], t1[w]);
+      worst = std::max(worst, ms);
+      per += (w ? " " : "") + std::to_string(ms);
+    }
+    fprintf(stderr, "[sb200 trace] %s: device part %.4f ms (max over devices; per device: %s)\n", tr.title, worst, per.c_str());
   }
   return SB200_OK;
 }

@@ -404,6 +404,13 @@ class ShardedHostMatrix:
         check(_lib.lib().sb200_sharded_transpose(self._h, _ptr(p), _ptr(i), _ptr(x)))
         return i, p, x
 
+    def crossprod(self):
+        """Dense A^T A, (ncol, ncol), on every GPU of the handle: the reference's result bit for bit, exactly symmetric
+        (sparse_b200.h sb200_sharded_crossprod; reference RcppSparse.h:158-194)."""
+        out = np.empty((self.ncol, self.ncol), np.float64)
+        check(_lib.lib().sb200_sharded_crossprod(self._h, _ptr(out)))
+        return out
+
 
 class Matrix:
     """Python mirror of ``RcppSparse::Matrix`` (reference RcppSparse.h:25-395), hot-path members.
@@ -415,7 +422,7 @@ class Matrix:
     ``.Call`` pays anyway (src/RcppExports.cpp:20).  ``resident=True`` (or ``resident()``) keeps the mirror, and
     the layouts the library caches on it, between calls; it is tied to THIS object (SURVEY.md H4: never cached
     by host address), rebuilt when a member is re-pointed, and after an in-place edit of ``x`` it needs
-    ``refresh()`` (of ``i``/``p``: ``release()``).  ``gpus > 1`` (default: SB200_GPUS) runs the sweeps on that many
+    ``refresh()`` (of ``i``/``p``: ``release()``).  ``gpus > 1`` (default: SB200_GPUS) runs every op on that many
     GPUs of this process (sb200_sharded_*).
     """
 
@@ -584,7 +591,7 @@ class Matrix:
         return self._call(True, lambda m: m.row_means())
 
     def crossprod(self):
-        return self._call(False, lambda m: m.crossprod())
+        return self._call(True, lambda m: m.crossprod())
 
     # ---- A v and A^T v: additions (the reference has only the iterator idiom, SURVEY.md D1) -----------------------------
     def spmv(self, v):
