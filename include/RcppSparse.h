@@ -14,7 +14,8 @@
 //   Rcpp::traits::Exporter<RcppSparse::Matrix>             reference :398-423
 // Additions: spmv(v) = A v and spmv_t(v) = A^T v (the reference only has the iterator idiom), spmm(B) = A B and
 // spmm_t(B) = A^T B for a dense NumericMatrix of k right-hand sides (one sweep instead of k spmv calls),
-// resident() to keep the device mirror between calls (then refresh() after mutating x in place, release() to
+// colVars() / rowVars() = the sample variance of every column / row (sparseMatrixStats::colVars / rowVars: implicit
+// zeros included, over n - 1; NaN where R's var gives NA, n < 2), resident() to keep the device mirror between calls (then refresh() after mutating x in place, release() to
 // drop it); SB200_GPUS=n runs the device ops on n GPUs of this process (sb200_sharded_*).
 //   dense copies (operator()(rows, cols), col, row), InnerIndices, emptyInnerIndices, isAppxSymmetric,
 //   InnerIteratorInRange / NotInRange, InnerRowIterator       reference :75-128, :196-216, :238-373 (host side; the
@@ -252,6 +253,21 @@ public:
     Lease l(*this, true);
     b200::check(l.s ? sb200_sharded_row_means(l.s, means.begin()) : sb200_row_means(l.m, means.begin()));
     return means;
+  }
+
+  // sample variances, two passes around colMeans / rowMeans -> sb200_col_vars / sb200_row_vars (sb200_sharded_* on
+  // several GPUs)
+  Rcpp::NumericVector colVars() {
+    Rcpp::NumericVector vars(Dim[1]);
+    Lease l(*this, true);
+    b200::check(l.s ? sb200_sharded_col_vars(l.s, vars.begin()) : sb200_col_vars(l.m, vars.begin()));
+    return vars;
+  }
+  Rcpp::NumericVector rowVars() {
+    Rcpp::NumericVector vars(Dim[0]);
+    Lease l(*this, true);
+    b200::check(l.s ? sb200_sharded_row_vars(l.s, vars.begin()) : sb200_row_vars(l.m, vars.begin()));
+    return vars;
   }
 
   // dense A^T A (reference :158-194): ncol x ncol, exactly symmetric -> sb200_crossprod; on several GPUs

@@ -106,6 +106,22 @@ int sb200_spmv(sb200_matrix* m, const double* v /* ncol */, double* y /* nrow */
 int sb200_spmv_t(sb200_matrix* m, const double* v /* nrow */, double* y /* ncol */);
 int sb200_transpose(sb200_matrix* m, int32_t* p_out, int32_t* i_out, double* x_out);
 
+/* Column and row variances (sparseMatrixStats::colVars / rowVars; the reference has none): out[c] is the sample variance
+ * of the nrow values of column c — its stored entries and its nrow - nnz_c implicit zeros — over nrow - 1, as R's
+ * var(A[, c]); out[r] the same over the ncol values of row r, over ncol - 1.  Two passes: the mean m is exactly what
+ * sb200_col_means / sb200_row_means return (same sweep, same division), then S = sum over the stored entries of
+ * (x - m)^2, and the result is (S + (n - cnt) m^2) / (n - 1) with cnt the stored entries (explicit zeros count).  No
+ * one-pass formula: within 1e-12 * exact + 2 * spacing(m)^2 of the exact variance of the double inputs, also on nearly
+ * constant data (mean 1e9, variance 1).  colVars is bit-stable run to run; rowVars is where rowSums is (on the
+ * row-ordered copy; the plan-free and banded paths add with FP64 atomics), and like rowSums it runs on that copy when
+ * the mirror has one, else on the path sb200_matrix_row_path reports; one call counts once toward building the copy.
+ * NaN or +-Inf among the entries of a column / row make that output NaN and no other.  An empty column / row gives +0.0.
+ * A dimension below 2 gives NaN for every output (R gives NA there); an output dimension of 0 writes nothing.  Scratch
+ * (8 bytes per output, 16 for rowVars) comes from the device: SB200_E_NOMEM when it does not fit.  A NULL output of
+ * non-empty shape: SB200_E_INVALID. */
+int sb200_col_vars(sb200_matrix* m, double* out /* ncol */);
+int sb200_row_vars(sb200_matrix* m, double* out /* nrow */);
+
 /* ---- the sweeps, device-buffer form (asynchronous on the handle's stream) ------------------
  * Operands and results are device pointers on the handle's device.  Used by the sharding
  * layer (results feed NCCL collectives without touching the host) and by bench.py.
@@ -115,6 +131,9 @@ int sb200_col_sums_dev(sb200_matrix* m, double divisor, double* d_out /* ncol */
 int sb200_row_sums_dev(sb200_matrix* m, double divisor, double* d_out /* nrow */);
 int sb200_spmv_dev(sb200_matrix* m, const double* d_v /* ncol */, double* d_y /* nrow */);
 int sb200_spmv_t_dev(sb200_matrix* m, const double* d_v /* nrow */, double* d_y /* ncol */);
+/* sb200_col_vars / sb200_row_vars into a device buffer, asynchronous on the handle's stream (tools/vars_bench.py). */
+int sb200_col_vars_dev(sb200_matrix* m, double* d_out /* ncol */);
+int sb200_row_vars_dev(sb200_matrix* m, double* d_out /* nrow */);
 /* Result stays in HBM as a new handle that owns its arrays (Dim swapped). */
 int sb200_transpose_dev(sb200_matrix* m, sb200_matrix** out);
 /* The same transpose (RcppSparse.h:375-385) written into a result that sb200_transpose_dev produced earlier for a matrix
@@ -281,6 +300,15 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out /* nrow + 1 */, int
  * SB200_E_NOMEM before anything is written (the handle stays usable).  Devices are ordered by CUDA events and host
  * synchronisation only, so blocks may share a device.  Blocking. */
 int sb200_sharded_crossprod(sb200_sharded* s, double* out /* ncol*ncol, column-major, host */);
+/* sb200_col_vars / sb200_row_vars on every device of the handle, same contract and bar.  colVars: every block runs the
+ * one-GPU two-pass sweep on its columns and its slice goes straight home; bit-stable, and bit-identical to
+ * sb200_col_vars at n_gpus = 1.  rowVars: the global row means as sb200_sharded_row_means computes them, then every
+ * block's sums of squares and entry counts over its own columns (16 nrow bytes of device memory per block, kept
+ * between calls; SB200_E_NOMEM when they do not fit), added in block order over peer memory, device q finishing rows
+ * [q nrow / n_gpus, (q+1) nrow / n_gpus) and copying them home.  Bit-stable where every block serves its row sums
+ * from its row-ordered copy.  That reduce is ordered by CUDA events only, so blocks may share a device.  Blocking. */
+int sb200_sharded_col_vars(sb200_sharded* s, double* out /* ncol */);
+int sb200_sharded_row_vars(sb200_sharded* s, double* out /* nrow */);
 
 /* Scratch, results and cached layouts come from the device's stream-ordered memory pool, which keeps freed blocks
  * for reuse (a multi-GB cudaMalloc/cudaFree pair costs as much as a sweep).  sb200_trim synchronises the device and
@@ -292,7 +320,8 @@ int sb200_trim(int device);
 int64_t sb200_launch_count(void);
 /* Name and per-launch algorithmic bytes (SURVEY.md 8d figures) of the dominant kernel of an op:
  * op = "col_sums" | "row_sums" | "col_means" | "row_means" | "spmv" | "spmv_t" | "transpose" |
- * "row_sums_companion" | "row_means_companion" (what the row sums read once the row-ordered copy exists). */
+ * "row_sums_companion" | "row_means_companion" (what the row sums read once the row-ordered copy exists) |
+ * "col_vars" | "row_vars" (compulsory: every array once, as for the sums; the two passes read x twice). */
 int sb200_algorithmic_bytes(const sb200_matrix* m, const char* op, int64_t* bytes);
 
 /* ---- synthetic matrices generated straight into HBM (tests and benchmarks) -----------------

@@ -16,6 +16,9 @@ b200_colSums  <- function(A) .b200_sweep(A, 0L, function(M) .Call(`_RcppSparse_b
 b200_rowSums  <- function(A) .b200_sweep(A, 1L, function(M) .Call(`_RcppSparse_b200_rowSums`, M))
 b200_colMeans <- function(A) .b200_sweep(A, 2L, function(M) .Call(`_RcppSparse_b200_colMeans`, M))
 b200_rowMeans <- function(A) .b200_sweep(A, 3L, function(M) .Call(`_RcppSparse_b200_rowMeans`, M))
+# sample variances of the columns / rows (implicit zeros included, over n - 1, as var(A[, j]); NaN where var gives NA)
+b200_colVars  <- function(A) .b200_sweep(A, 4L, function(M) .Call(`_RcppSparse_b200_colVars`, M))
+b200_rowVars  <- function(A) .b200_sweep(A, 5L, function(M) .Call(`_RcppSparse_b200_rowVars`, M))
 
 b200_spmv <- function(A, v) {
     v <- as.double(v)

@@ -3,7 +3,7 @@
 // columnSums keeps the reference's name, signature and result (reference src/example.cpp:26-32); its body is
 // now the class call, which the drop-in header serves from the device.  The b200_* functions are additions:
 // thin wrappers over the class methods (reference inst/include/RcppSparse.h:131-156, 375-385, the SpMV idiom
-// and its k-column form spmm), and a persistent handle — an external pointer to a heap RcppSparse::Matrix whose device mirror
+// and its k-column form spmm, and the column / row variances), and a persistent handle — an external pointer to a heap RcppSparse::Matrix whose device mirror
 // therefore survives across .Call()s (one .Call otherwise builds a fresh Matrix, i.e. a fresh upload:
 // reference src/RcppExports.cpp:20).
 #include <RcppSparse.h>
@@ -28,6 +28,12 @@ Rcpp::NumericVector b200_colMeans(RcppSparse::Matrix& A) { return A.colMeans(); 
 
 //[[Rcpp::export]]
 Rcpp::NumericVector b200_rowMeans(RcppSparse::Matrix& A) { return A.rowMeans(); }
+
+//[[Rcpp::export]]
+Rcpp::NumericVector b200_colVars(RcppSparse::Matrix& A) { return A.colVars(); }
+
+//[[Rcpp::export]]
+Rcpp::NumericVector b200_rowVars(RcppSparse::Matrix& A) { return A.rowVars(); }
 
 //[[Rcpp::export]]
 Rcpp::NumericVector b200_spmv(RcppSparse::Matrix& A, const Rcpp::NumericVector& v) { return A.spmv(v); }
@@ -67,6 +73,8 @@ Rcpp::NumericVector b200_dm_sweep(SEXP handle, int op) {
         case 1: return A->rowSums();
         case 2: return A->colMeans();
         case 3: return A->rowMeans();
+        case 4: return A->colVars();
+        case 5: return A->rowVars();
         default: throw std::invalid_argument("b200_dm_sweep: unknown op");
     }
 }

@@ -25,9 +25,10 @@ SYMBOLS = [
     "sb200_synth_vector_dev", "sb200_matrix_download_columns", "sb200_matrix_row_path", "sb200_matrix_row_companion",
     "sb200_crossprod", "sb200_crossprod_dev", "sb200_matrix_band_companion", "sb200_matrix_layouts", "sb200_matrix_layout_bytes", "sb200_trim",
     "sb200_col_sums_in_rows", "sb200_gather_block", "sb200_spmm", "sb200_spmm_t", "sb200_spmm_dev", "sb200_spmm_t_dev",
+    "sb200_col_vars", "sb200_row_vars", "sb200_col_vars_dev", "sb200_row_vars_dev",
     "sb200_sharded_create", "sb200_sharded_destroy", "sb200_sharded_info", "sb200_sharded_block", "sb200_sharded_col_sums",
     "sb200_sharded_row_sums", "sb200_sharded_col_means", "sb200_sharded_row_means", "sb200_sharded_spmv", "sb200_sharded_spmv_t", "sb200_sharded_transpose",
-    "sb200_sharded_spmm", "sb200_sharded_spmm_t", "sb200_sharded_crossprod",
+    "sb200_sharded_spmm", "sb200_sharded_spmm_t", "sb200_sharded_crossprod", "sb200_sharded_col_vars", "sb200_sharded_row_vars",
     "sb200_exchange_create", "sb200_exchange_connect", "sb200_exchange_destroy", "sb200_exchange_window",
     "sb200_exchange_gather", "sb200_exchange_reduce", "sb200_exchange_push_rows", "sb200_exchange_barrier", "sb200_exchange_status",
 ]
@@ -99,6 +100,10 @@ def lib() -> C.CDLL:
         "sb200_spmm_t": ([vp, vp, i64, vp], C.c_int),
         "sb200_spmm_dev": ([vp, vp, i64, vp], C.c_int),
         "sb200_spmm_t_dev": ([vp, vp, i64, vp], C.c_int),
+        "sb200_col_vars": ([vp, vp], C.c_int),
+        "sb200_row_vars": ([vp, vp], C.c_int),
+        "sb200_col_vars_dev": ([vp, vp], C.c_int),
+        "sb200_row_vars_dev": ([vp, vp], C.c_int),
         "sb200_sharded_create": ([vp, vp, vp, i32, i32, i64, C.c_int, vp, u32, pp], C.c_int),
         "sb200_sharded_destroy": ([vp], C.c_int),
         "sb200_sharded_info": ([vp, C.POINTER(C.c_int), vp], C.c_int),
@@ -113,6 +118,8 @@ def lib() -> C.CDLL:
         "sb200_sharded_spmm": ([vp, vp, i64, vp], C.c_int),
         "sb200_sharded_spmm_t": ([vp, vp, i64, vp], C.c_int),
         "sb200_sharded_crossprod": ([vp, vp], C.c_int),
+        "sb200_sharded_col_vars": ([vp, vp], C.c_int),
+        "sb200_sharded_row_vars": ([vp, vp], C.c_int),
         "sb200_crossprod": ([vp, vp], C.c_int),
         "sb200_crossprod_dev": ([vp, vp], C.c_int),
         "sb200_exchange_create": ([C.c_int, i64, pp, vp], C.c_int),

@@ -18,7 +18,7 @@ OBJ = os.path.join(PKG, "build")
 LIB = os.path.join(PKG, "libsparse_b200.so")
 MICROBENCH = os.path.join(PKG, "microbench")
 
-LIB_SOURCES = ["capi.cu", "blockcache.cu", "sweep.cu", "scan.cu", "validate.cu", "bands.cu", "transpose.cu", "transpose_split.cu", "bmc.cu", "synth.cu", "exchange.cu", "sharded.cu", "extract.cu", "crossprod.cu", "spmm.cu", "hostcopy.cu"]
+LIB_SOURCES = ["capi.cu", "blockcache.cu", "sweep.cu", "scan.cu", "validate.cu", "bands.cu", "transpose.cu", "transpose_split.cu", "bmc.cu", "synth.cu", "exchange.cu", "sharded.cu", "extract.cu", "crossprod.cu", "spmm.cu", "hostcopy.cu", "vars.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xptxas", "-v",
               "--expt-relaxed-constexpr"] + ARCH

@@ -295,15 +295,18 @@ struct ScatterArgs {
   int lock_every;
   unsigned int* lock_counters;  // [S], zeroed before the launch
   int cluster;                  // CTAs per thread-block cluster (adjacent bands), 1 = no clusters
+  const double* mean;           // rowVars' second pass: [nrow] row means (band_var_kernel), else null
+  int mean_rows;                // rows of mean staged per band (the widest band), 0 without
 };
 
 constexpr int SC_CAPW = 512;       // flattened entries a warp stages per round
 constexpr int SC_PRIVATE_ROWS = 256;  // bands this narrow get one accumulator copy PER WARP (32 KB)
 
-static size_t scatter_smem_bytes(int max_rows, bool spmv) {
+static size_t scatter_smem_bytes(int max_rows, bool spmv, int mean_rows = 0) {
   size_t rows = static_cast<size_t>(max_rows > 0 ? max_rows : 1);
   if (rows < static_cast<size_t>(BAND_WARPS) * SC_PRIVATE_ROWS) rows = static_cast<size_t>(BAND_WARPS) * SC_PRIVATE_ROWS;
-  return sizeof(double) * rows + BAND_WARPS * SC_CAPW * sizeof(int32_t) + (spmv ? BAND_WARPS * SC_CAPW : 0) + 16;
+  return sizeof(double) * (rows + static_cast<size_t>(mean_rows)) + BAND_WARPS * SC_CAPW * sizeof(int32_t) +
+         (spmv ? BAND_WARPS * SC_CAPW : 0) + 16;
 }
 
 // CTA (band b, column split h).  A warp takes 32 consecutive columns of the chunk, one run descriptor
@@ -311,15 +314,20 @@ static size_t scatter_smem_bytes(int max_rows, bool spmv) {
 // warp's flat list in shared memory (entry index per slot; ~1 store per entry), then the lanes walk
 // the list 32 slots at a time, so consecutive lanes read consecutive entries of a run (coalesced),
 // U loads in flight before the first shared-memory FP64 add.
-template <bool SPMV>
-__global__ void __launch_bounds__(BAND_THREADS) band_scatter_kernel(const ScatterArgs a) {
+// VAR (rowVars' second pass): the band's slice of the row means sits in shared memory after the accumulators, and an
+// entry adds (x - mean[row])^2 instead of x.
+// (tid = threadIdx.x, read in the kernel itself: there the compiler knows its range from the launch bounds)
+template <bool SPMV, bool VAR>
+__device__ __forceinline__ void band_scatter_body(const ScatterArgs& a, const int tid) {
   extern __shared__ __align__(16) unsigned char ssm[];
   const BandView& bv = a.bv;
   const int MR = a.max_rows;
   double* acc = reinterpret_cast<double*>(ssm);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  int32_t* flat = reinterpret_cast<int32_t*>(acc + MR) + warp * SC_CAPW;
-  uint8_t* flatl = reinterpret_cast<uint8_t*>(reinterpret_cast<int32_t*>(acc + MR) + BAND_WARPS * SC_CAPW) + warp * SC_CAPW;
+  double* means = acc + MR;  // VAR only
+  const int lane = tid & 31, warp = tid >> 5;
+  double* const acc_end = acc + MR + (VAR ? a.mean_rows : 0);
+  int32_t* flat = reinterpret_cast<int32_t*>(acc_end) + warp * SC_CAPW;
+  uint8_t* flatl = reinterpret_cast<uint8_t*>(reinterpret_cast<int32_t*>(acc_end) + BAND_WARPS * SC_CAPW) + warp * SC_CAPW;
   constexpr int U = BAND_UNROLL;
   const int units = bv.nb * bv.S;
   for (int u = blockIdx.x; u < units; u += gridDim.x) {
@@ -336,6 +344,8 @@ __global__ void __launch_bounds__(BAND_THREADS) band_scatter_kernel(const Scatte
     const unsigned lt_mask = (1u << lane) - 1u;
     __syncthreads();
     for (int r = tid; r < (priv ? R * BAND_WARPS : R); r += BAND_THREADS) acc[r] = 0.0;
+    if constexpr (VAR)
+      for (int r = tid; r < R; r += BAND_THREADS) means[r] = __ldg(a.mean + row0 + r);
     __syncthreads();
     // software-pipelined descriptors: the next chunk's are fetched (and its runs prefetched to L2)
     // while the current chunk is walked
@@ -431,6 +441,15 @@ __global__ void __launch_bounds__(BAND_THREADS) band_scatter_kernel(const Scatte
               xx[t] = __dmul_rn(xx[t], w);
             }
           }
+          if constexpr (VAR) {
+#pragma unroll
+            for (int t = 0; t < U; ++t) {
+              if (rr[t] >= 0) {
+                const double d = __dsub_rn(xx[t], means[rr[t]]);
+                xx[t] = __dmul_rn(d, d);
+              }
+            }
+          }
           if (priv) {
 #pragma unroll
             for (int t = 0; t < U; ++t) {
@@ -477,6 +496,13 @@ __global__ void __launch_bounds__(BAND_THREADS) band_scatter_kernel(const Scatte
     }
   }
 }
+
+template <bool SPMV>
+__global__ void __launch_bounds__(BAND_THREADS) band_scatter_kernel(const ScatterArgs a) {
+  band_scatter_body<SPMV, false>(a, threadIdx.x);
+}
+
+__global__ void __launch_bounds__(BAND_THREADS) band_var_kernel(const ScatterArgs a) { band_scatter_body<false, true>(a, threadIdx.x); }
 
 // ================================================================================================
 // transpose: banded stable scatter
@@ -949,17 +975,20 @@ int ensure_scatter_plan(sb200_matrix* m) {
   return build_band_plan(m, SCATTER_ROWS_CAP, bands, S, &m->plan_scatter);
 }
 
-int launch_band_scatter(sb200_matrix* m, const double* d_v, double* d_out) {
+// d_mean set: rowVars' second pass (band_var_kernel), d_v is null then
+static int launch_band_scatter_impl(sb200_matrix* m, const double* d_v, const double* d_mean, double* d_out) {
   SB_TRY(ensure_scatter_plan(m));
   const BandPlan* bp = m->plan_scatter;
   ScatterArgs a;
   a.bv = make_view(m, bp);
   a.v = d_v;
   a.out = d_out;
+  a.mean = d_mean;
+  a.mean_rows = d_mean ? (bp->max_rows > 0 ? bp->max_rows : 1) : 0;
   if (bp->S > 1) SB_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * static_cast<size_t>(m->nrow), m->stream));
   a.max_rows = (bp->max_rows > 0 ? bp->max_rows : 1);
   if (a.max_rows < BAND_WARPS * SC_PRIVATE_ROWS) a.max_rows = BAND_WARPS * SC_PRIVATE_ROWS;  // room for the per-warp copies
-  const size_t smem = scatter_smem_bytes(a.max_rows, d_v != nullptr);
+  const size_t smem = scatter_smem_bytes(a.max_rows, d_v != nullptr, a.mean_rows);
   int ctas = static_cast<int>((200 * 1024) / (smem + 2048));
   if (ctas > 2) ctas = 2;
   if (ctas < 1) ctas = 1;
@@ -975,15 +1004,14 @@ int launch_band_scatter(sb200_matrix* m, const double* d_v, double* d_out) {
   a.lock_every = lock_every;
   a.lock_counters = reinterpret_cast<unsigned int*>(static_cast<unsigned char*>(m->d_ws) + 16 + 4 * 1024 + 8 * 1024);
   if (lock_every > 0 && static_cast<size_t>(bp->S) * 4 > m->ws_bytes - (16 + 4 * 1024 + 8 * 1024)) a.lock_every = 0;
-  auto kern = d_v ? reinterpret_cast<const void*>(&band_scatter_kernel<true>)
-                  : reinterpret_cast<const void*>(&band_scatter_kernel<false>);
-  SB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  void (*const kern)(ScatterArgs) = d_mean ? band_var_kernel : d_v ? band_scatter_kernel<true> : band_scatter_kernel<false>;
+  SB_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(kern), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   if (a.lock_every > 0) {
     // a soft barrier between CTAs is only safe if they are all resident: ask the driver to guarantee it
     SB_CUDA(cudaMemsetAsync(a.lock_counters, 0, sizeof(unsigned int) * bp->S, m->stream));
     a.cluster = 1;
     void* params[] = {&a};
-    cudaError_t e = cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(BAND_THREADS), params, smem, m->stream);
+    cudaError_t e = cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(kern), dim3(grid), dim3(BAND_THREADS), params, smem, m->stream);
     if (e == cudaErrorCooperativeLaunchTooLarge || e == cudaErrorNotSupported || e == cudaErrorLaunchOutOfResources) {
       cudaGetLastError();
       a.lock_every = 0;  // fall back to free-running CTAs
@@ -1015,8 +1043,7 @@ int launch_band_scatter(sb200_matrix* m, const double* d_v, double* d_out) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = d_v ? cudaLaunchKernelEx(&cfg, band_scatter_kernel<true>, a)
-                        : cudaLaunchKernelEx(&cfg, band_scatter_kernel<false>, a);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, a);
     if (e == cudaSuccess) {
       count_launch();
       return SB200_OK;
@@ -1024,12 +1051,17 @@ int launch_band_scatter(sb200_matrix* m, const double* d_v, double* d_out) {
     cudaGetLastError();  // cluster launch not possible with this footprint: free-running CTAs
     a.cluster = 1;
   }
-  if (d_v)
-    band_scatter_kernel<true><<<grid, BAND_THREADS, smem, m->stream>>>(a);
-  else
-    band_scatter_kernel<false><<<grid, BAND_THREADS, smem, m->stream>>>(a);
+  kern<<<grid, BAND_THREADS, smem, m->stream>>>(a);
   count_launch();
   SB_CUDA(cudaGetLastError());
+  return SB200_OK;
+}
+
+int launch_band_scatter(sb200_matrix* m, const double* d_v, double* d_out) { return launch_band_scatter_impl(m, d_v, nullptr, d_out); }
+
+int launch_band_var(sb200_matrix* m, const double* d_mean, double* d_S, const int32_t** d_rowptr) {
+  SB_TRY(launch_band_scatter_impl(m, nullptr, d_mean, d_S));
+  *d_rowptr = m->plan_scatter->d_rowptr;  // kept with the plan: the row counts are its differences
   return SB200_OK;
 }
 

@@ -505,6 +505,16 @@ int sb200_spmv_t_dev(sb200_matrix* m, const double* d_v, double* d_y) {
   if ((m->nrow > 0 && !d_v) || (m->ncol > 0 && !d_y)) return fail(SB200_E_INVALID, "NULL operand");
   return launch_sweep(m, SWEEP_SPMV_T, d_v, 0.0, d_y);
 }
+int sb200_col_vars_dev(sb200_matrix* m, double* d_out) {
+  ENTER_COLS(m);
+  if (m->ncol > 0 && !d_out) return fail(SB200_E_INVALID, "d_out is NULL");
+  return launch_col_vars(m, d_out);
+}
+int sb200_row_vars_dev(sb200_matrix* m, double* d_out) {
+  ENTER(m);
+  if (m->nrow > 0 && !d_out) return fail(SB200_E_INVALID, "d_out is NULL");
+  return launch_row_vars(m, d_out);
+}
 int sb200_vec_div_dev(sb200_matrix* m, double* d, int64_t n, double divisor) {
   ENTER_COLS(m);
   return launch_vec_div(m->stream, d, n, divisor);
@@ -586,6 +596,14 @@ int sb200_row_means(sb200_matrix* m, double* out) {
     return SB200_OK;
   }
   return run_to_host(m, SWEEP_ROWSUM, nullptr, 0, static_cast<double>(m->ncol), out, m->nrow);
+}
+int sb200_col_vars(sb200_matrix* m, double* out) {
+  ENTER_COLS(m);
+  return run_to_host(m, SWEEP_COLVAR, nullptr, 0, 0.0, out, m->ncol);
+}
+int sb200_row_vars(sb200_matrix* m, double* out) {
+  ENTER(m);
+  return run_to_host(m, SWEEP_ROWVAR, nullptr, 0, 0.0, out, m->nrow);
 }
 int sb200_spmv(sb200_matrix* m, const double* v, double* y) {
   ENTER(m);
@@ -848,9 +866,9 @@ int sb200_algorithmic_bytes(const sb200_matrix* m, const char* op, int64_t* byte
   const int64_t N = m->nnz, n = m->ncol, r = m->nrow;
   const std::string s(op);
   // SURVEY.md section 8(d): compulsory traffic only — every array once, the output once
-  if (s == "col_sums" || s == "col_means")
+  if (s == "col_sums" || s == "col_means" || s == "col_vars")  // colVars: the two passes read x twice (16N + ...)
     *bytes = 8 * N + 4 * (n + 1) + 8 * n;
-  else if (s == "row_sums" || s == "row_means")
+  else if (s == "row_sums" || s == "row_means" || s == "row_vars")
     *bytes = 12 * N + 8 * r;
   else if (s == "row_sums_companion" || s == "row_means_companion")  // row-ordered x once, row pointer, output
     *bytes = 8 * N + 4 * (r + 1) + 8 * r;

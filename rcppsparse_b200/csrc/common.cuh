@@ -130,10 +130,24 @@ struct DeviceGuard {
 };
 
 // sweep.cu
-enum SweepMode { SWEEP_COLSUM = 0, SWEEP_SPMV_T = 1, SWEEP_ROWSUM = 2, SWEEP_SPMV = 3 };
+// COLVAR / ROWVAR: colVars / rowVars through launch_sweep (vars.cu); COLVAR is also the kernel mode of their second pass
+enum SweepMode { SWEEP_COLSUM = 0, SWEEP_SPMV_T = 1, SWEEP_ROWSUM = 2, SWEEP_SPMV = 3, SWEEP_COLVAR = 4, SWEEP_ROWVAR = 5 };
 int build_sweep_plan(sb200_matrix* m);
 int launch_sweep(sb200_matrix* m, SweepMode mode, const double* d_v, double divisor, double* d_out);
 int launch_vec_div(cudaStream_t s, double* d, int64_t n, double divisor);
+int launch_col_var_sweep(sb200_matrix* m, const double* d_mean, double n, double* d_out);  // n = 0: raw sums of squares
+
+// vars.cu: two-pass variances.  The variance of n values (n >= 2) of which cnt are stored entries whose squared
+// deviations from the mean mu sum to S and n - cnt are zeros, over n - 1 (R's var()).
+__device__ __forceinline__ double var_from_sums(double S, double cnt, double mu, double n) {
+  return __ddiv_rn(__dadd_rn(S, __dmul_rn(__dsub_rn(n, cnt), __dmul_rn(mu, mu))), __dsub_rn(n, 1.0));
+}
+int launch_col_vars(sb200_matrix* m, double* d_out);  // ncol outputs, NaN when nrow < 2
+int launch_row_vars(sb200_matrix* m, double* d_out);  // nrow outputs, NaN when ncol < 2
+// Second pass of rowVars without the formula, for the sharded reduce: d_S[r] = sum over row r's stored entries of
+// (x - d_mean[r])^2, d_cnt[r] = their number (as a double), on the path rowSums takes on this mirror.
+int launch_row_var_sums(sb200_matrix* m, const double* d_mean, double* d_S, double* d_cnt);
+int launch_fill_nan(cudaStream_t s, double* d, int64_t n);
 
 // validate.cu
 int validate_structure(sb200_matrix* m, bool rows = true);  // p always; i (range, ascending inside a column) when rows
@@ -153,6 +167,8 @@ int decide_row_path(sb200_matrix* m);
 int decide_gather_path(sb200_matrix* m);
 int launch_band_gather(sb200_matrix* m, const double* d_v, double* d_out);
 int launch_band_scatter(sb200_matrix* m, const double* d_v, double* d_out);  // d_v null = rowSums
+// rowVars' second pass on the row bands: d_S[r] = sum of (x - d_mean[r])^2 over row r; *d_rowptr = the plan's row pointer
+int launch_band_var(sb200_matrix* m, const double* d_mean, double* d_S, const int32_t** d_rowptr);
 int launch_band_ptr(sb200_matrix* m, const int32_t* d_rb, int nb, int32_t* d_bpt);
 // bmc.cu
 int build_band_companion(sb200_matrix* m);  // non-fatal: leaves bmc_state = -1 when it cannot be built

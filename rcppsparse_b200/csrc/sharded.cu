@@ -23,6 +23,9 @@
 //           in the same pass (sharded_sum_transpose_kernel); then every device copies its rows home.
 //           Ordering across devices is CUDA events only (no in-kernel barrier), so blocks that share a device are fine.
 // Host copies run from one thread per device (a copy from pageable memory blocks the thread that issues it).
+// The variances (sb200_sharded_col_vars / _row_vars): colVars is column-indexed like colMeans; rowVars takes the global row
+// means as rowMeans does, then reduces every block's sums of squared deviations and entry counts in rank order over peer
+// memory (sharded_row_var_kernel, ordered by events like the A B reduce) and applies the formula on every device.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -30,6 +33,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <limits>
 #include <chrono>
 #include <new>
 #include <string>
@@ -128,10 +132,10 @@ int run_columns(sb200_sharded* s, SweepMode mode, const double* v_host, double d
   return rc;
 }
 
-// row-indexed op: partials in the windows, rank-ordered P2P reduction on every device, result read from device 0
-int run_rows(sb200_sharded* s, SweepMode mode, const double* v_host, double divisor, double* out) {
-  if (s->nrow > 0 && !out) return fail(SB200_E_INVALID, "output buffer is NULL");
-  DeviceGuard restore(s->blocks[0]->device);  // the exchange entry points switch devices; put the caller's back on return
+// row-indexed op up to its result: partials in the windows, rank-ordered P2P reduction on every device.  The result
+// (divided by divisor when it is not 0) is at byte offset *off of every window, in each block's stream order.
+int rows_into_windows(sb200_sharded* s, SweepMode mode, const double* v_host, double divisor, int64_t* off) {
+  *off = s->world > 1 ? s->result_off : s->partial_off;
   int rc = SB200_OK;
   for (int k = 0; k < s->world && rc == SB200_OK; ++k) {
     sb200_matrix* m = s->blocks[k];
@@ -153,9 +157,17 @@ int run_rows(sb200_sharded* s, SweepMode mode, const double* v_host, double divi
                           divisor);
     }
   }
+  return rc;
+}
+
+// row-indexed op: rows_into_windows, result read from device 0
+int run_rows(sb200_sharded* s, SweepMode mode, const double* v_host, double divisor, double* out) {
+  if (s->nrow > 0 && !out) return fail(SB200_E_INVALID, "output buffer is NULL");
+  DeviceGuard restore(s->blocks[0]->device);  // the exchange entry points switch devices; put the caller's back on return
+  int64_t off = 0;
+  int rc = rows_into_windows(s, mode, v_host, divisor, &off);
   if (rc == SB200_OK && s->nrow > 0) {
     DeviceGuard guard(s->blocks[0]->device);
-    const int64_t off = s->world > 1 ? s->result_off : s->partial_off;
     SB_CUDA(cudaMemcpyAsync(out, exchange_window_base(s->windows[0]) + off, sizeof(double) * static_cast<size_t>(s->nrow),
                             cudaMemcpyDeviceToHost, s->blocks[0]->stream));
   }
@@ -458,8 +470,8 @@ int ensure_spmm_state(sb200_sharded* s) {
   return SB200_OK;
 }
 
-// block w's partial holds at least `bytes`; the current device is block w's
-int ensure_partial(sb200_sharded* s, int w, size_t bytes) {
+// block w's partial holds at least `bytes`; the current device is block w's.  `what` names the partial in the error.
+int ensure_partial(sb200_sharded* s, int w, size_t bytes, const char* what) {
   if (s->mm_partial_bytes[w] >= bytes) return SB200_OK;
   for (cudaEvent_t e : s->ev_reduced) SB_CUDA(cudaEventSynchronize(e));  // no reader still has the old one in flight
   if (s->mm_partial[w]) cudaFree(s->mm_partial[w]);
@@ -468,8 +480,7 @@ int ensure_partial(sb200_sharded* s, int w, size_t bytes) {
   if (cudaMalloc(reinterpret_cast<void**>(&s->mm_partial[w]), bytes) != cudaSuccess) {
     cudaGetLastError();
     s->mm_partial[w] = nullptr;
-    return fail(SB200_E_NOMEM, "sharded spmm: the row-major partial (8 nrow k bytes) does not fit on device " +
-                                   std::to_string(s->devices[w]));
+    return fail(SB200_E_NOMEM, std::string(what) + " does not fit on device " + std::to_string(s->devices[w]));
   }
   s->mm_partial_bytes[w] = bytes;
   return SB200_OK;
@@ -516,7 +527,7 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
     rc = pool_alloc(reinterpret_cast<void**>(&dB[w]), std::max<size_t>(16, sizeof(double) * static_cast<size_t>(b_n(w) * k)), m->stream);
     if (rc == SB200_OK)
       rc = pool_alloc(reinterpret_cast<void**>(&dY[w]), std::max<size_t>(16, sizeof(double) * static_cast<size_t>(y_n(w) * k)), m->stream);
-    if (rc == SB200_OK && !transposed) rc = ensure_partial(s, w, sizeof(double) * static_cast<size_t>(nrow * k));
+    if (rc == SB200_OK && !transposed) rc = ensure_partial(s, w, sizeof(double) * static_cast<size_t>(nrow * k), "sharded spmm: the row-major partial (8 nrow k bytes)");
   }
   tr.phase("scratch");
   // 1. operands up: block w's rows of B, a strided slice (A B) or all of it (A^T B)
@@ -597,6 +608,73 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
     if (t1[w]) cudaEventDestroy(t1[w]);
   }
   if (rc == SB200_E_NOMEM) cudaGetLastError();  // a refused allocation leaves the streams usable
+  return rc;
+}
+
+// ---- rowVars: the rank-ordered reduce of the blocks' sums of squares and counts ---------------------------------------
+// Rows [r0, r1): S and cnt are the blocks' partials (P.p[w][r] and P.p[w][nrow + r]) added in block order with __dadd_rn,
+// like xg_reduce_kernel, and out[r] = var_from_sums(S, cnt, mean[r], n).  The same bits on every device and every run.
+__global__ void __launch_bounds__(256) sharded_row_var_kernel(const __grid_constant__ PartialPtrs P, int world, int64_t nrow, int64_t r0,
+                                                              int64_t r1, const double* __restrict__ mean, double n,
+                                                              double* __restrict__ out) {
+  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
+  for (int64_t r = r0 + static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; r < r1; r += stride) {
+    double S = P.p[0][r], c = P.p[0][nrow + r];
+    for (int q = 1; q < world; ++q) {
+      S = __dadd_rn(S, P.p[q][r]);
+      c = __dadd_rn(c, P.p[q][nrow + r]);
+    }
+    out[r] = var_from_sums(S, c, mean[r], n);
+  }
+}
+
+// rowVars on every device: (1) the global row means as sb200_sharded_row_means computes them, in every window; (2) every
+// block's S and counts over its own columns into its peer-readable partial (16 nrow bytes, kept between calls); (3)
+// device q reduces rows [q nrow / W, (q+1) nrow / W) of all partials and copies them home.  Steps 2 and 3 are ordered
+// by CUDA events only, so blocks may share a device.
+int run_row_vars(sb200_sharded* s, double* out) {
+  const int W = s->world;
+  const int64_t nrow = s->nrow;
+  DeviceGuard restore(s->blocks[0]->device);
+  SB_TRY(ensure_spmm_state(s));
+  int64_t mean_off = 0;
+  int rc = rows_into_windows(s, SWEEP_ROWSUM, nullptr, static_cast<double>(s->ncol), &mean_off);
+  PartialPtrs P{};
+  for (int w = 0; w < W && rc == SB200_OK; ++w) {
+    sb200_matrix* m = s->blocks[w];
+    DeviceGuard g(m->device);
+    rc = ensure_partial(s, w, 2 * sizeof(double) * static_cast<size_t>(nrow), "sharded rowVars: the sums and counts (16 nrow bytes)");
+    if (rc != SB200_OK) break;
+    P.p[w] = s->mm_partial[w];
+    const double* mean = reinterpret_cast<const double*>(exchange_window_base(s->windows[w]) + mean_off);
+    rc = launch_row_var_sums(m, mean, s->mm_partial[w], s->mm_partial[w] + nrow);
+    if (rc == SB200_OK && cudaEventRecord(s->ev_partial[w], m->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaEventRecord");
+  }
+  for (int q = 0; q < W && rc == SB200_OK; ++q) {
+    sb200_matrix* m = s->blocks[q];
+    DeviceGuard g(m->device);
+    for (int w = 0; w < W && rc == SB200_OK; ++w)
+      if (cudaStreamWaitEvent(m->stream, s->ev_partial[w], 0) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaStreamWaitEvent");
+    const int64_t r0 = nrow * q / W, r1 = nrow * (q + 1) / W;
+    if (rc != SB200_OK || r1 == r0) continue;
+    const double* mean = reinterpret_cast<const double*>(exchange_window_base(s->windows[q]) + mean_off);
+    int64_t blocks = (r1 - r0 + 255) / 256;
+    if (blocks > static_cast<int64_t>(m->sm_count) * 8) blocks = static_cast<int64_t>(m->sm_count) * 8;
+    sharded_row_var_kernel<<<static_cast<unsigned>(blocks), 256, 0, m->stream>>>(P, W, nrow, r0, r1, mean, static_cast<double>(s->ncol),
+                                                                               m->d_stage_out);
+    count_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaEventRecord(s->ev_reduced[q], m->stream);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(out + r0, m->d_stage_out + r0, sizeof(double) * static_cast<size_t>(r1 - r0), cudaMemcpyDeviceToHost, m->stream);
+    if (e != cudaSuccess) rc = cuda_fail(e, "sharded rowVars: reduce", __FILE__, __LINE__);
+  }
+  for (int w = 0; w < W; ++w) {  // every device is waited for, whatever happened on another
+    DeviceGuard g(s->blocks[w]->device);
+    const cudaError_t e = cudaStreamSynchronize(s->blocks[w]->stream);
+    if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded rowVars", __FILE__, __LINE__);
+  }
+  if (rc == SB200_E_NOMEM) cudaGetLastError();
   return rc;
 }
 
@@ -767,6 +845,20 @@ int sb200_sharded_row_means(sb200_sharded* s, double* out) {
     return SB200_OK;
   }
   return run_rows(s, SWEEP_ROWSUM, nullptr, static_cast<double>(s->ncol), out);
+}
+int sb200_sharded_col_vars(sb200_sharded* s, double* out) {
+  SB_TRY(check_sharded(s));
+  return run_columns(s, SWEEP_COLVAR, nullptr, 0.0, out);
+}
+int sb200_sharded_row_vars(sb200_sharded* s, double* out) {
+  SB_TRY(check_sharded(s));
+  if (s->nrow == 0) return SB200_OK;
+  if (!out) return fail(SB200_E_INVALID, "output buffer is NULL");
+  if (s->ncol < 2) {  // no variance of fewer than two values (R: NA)
+    for (int32_t r = 0; r < s->nrow; ++r) out[r] = std::numeric_limits<double>::quiet_NaN();
+    return SB200_OK;
+  }
+  return run_row_vars(s, out);
 }
 int sb200_sharded_spmv(sb200_sharded* s, const double* v, double* y) {
   SB_TRY(check_sharded(s));

@@ -6,6 +6,7 @@
 //   A^T v (iterator idiom, gather shape of :133-135)                        -> SWEEP_SPMV_T
 //   A v   (iterator idiom, scatter shape of :140-142)                       -> SWEEP_SPMV
 //   rowSums / rowMeans     RcppSparse.h:138-144,151-156                     -> rowsum_stream_kernel
+//   colVars (second pass: sum of (x - mean)^2 per column, formula at the store) -> SWEEP_COLVAR (vars.cu)
 //
 // Work decomposition.  The sweep is a merge of two sorted lists: the column end offsets
 // A[c] = p[c+1] and the entry indices B[k] = k.  One merge "item" is either "consume entry
@@ -78,6 +79,7 @@ struct SweepParams {
   double* carry_val;   // [grid]
   unsigned int* ticket;
   int mask;  // SPMV_T only: v is an indicator — entries whose v[row] is 0 are SKIPPED (x * 0 would turn Inf into NaN)
+  double var_n;  // COLVAR only (v = the column means): the column length n of var_from_sums; 0 = store the raw sums
 };
 
 struct StageMeta {
@@ -115,12 +117,13 @@ __device__ __forceinline__ void consumer_sync() { asm volatile("bar.sync 1, %0;"
 
 template <int MODE, int STAGES>
 __global__ void __launch_bounds__(SWEEP_BLOCK) sweep_kernel(const SweepParams prm) {
-  constexpr int IPT = (MODE == SWEEP_COLSUM) ? SWEEP_IPT : GATHER_IPT;
+  constexpr bool VAR = (MODE == SWEEP_COLVAR);
+  constexpr int IPT = (MODE == SWEEP_COLSUM || VAR) ? SWEEP_IPT : GATHER_IPT;
   using G = SweepGeom<IPT>;
   constexpr int THREADS = SWEEP_THREADS;
   constexpr int TILE = G::TILE;
   constexpr bool WITH_I = (MODE == SWEEP_SPMV_T || MODE == SWEEP_SPMV);
-  constexpr bool REDUCES = (MODE == SWEEP_COLSUM || MODE == SWEEP_SPMV_T);
+  constexpr bool REDUCES = (MODE == SWEEP_COLSUM || MODE == SWEEP_SPMV_T || VAR);
   constexpr int WARPS = THREADS / 32;
   static_assert(WARPS <= 32, "warp fold uses one lane per warp");
 
@@ -213,6 +216,46 @@ __global__ void __launch_bounds__(SWEEP_BLOCK) sweep_kernel(const SweepParams pr
   double cta_carry = 0.0;  // partial sum of the column in progress, carried across this CTA's tiles
   int32_t last_c1 = 0, last_k1 = 0;
 
+  // COLVAR: every item adds (x - m)^2 with m = its column's mean, and a column's store applies var_from_sums.  The one
+  // exception is the column earlier CTAs carry into (it began before this CTA's first item): its store here is only
+  // this CTA's share, and the last CTA applies the formula when it folds the carries in.  Every other mode compiles
+  // these helpers down to the plain sum and store.
+  int32_t in_col = -1;
+  if constexpr (VAR) {
+    if (n_local > 0) {
+      const int32_t c = __ldg(prm.plan + t_begin);
+      if (c < prm.ncol && t_begin * TILE - c > __ldg(prm.p + c)) in_col = c;
+    }
+  }
+  auto mean_of = [&](int64_t c) -> double {
+    if constexpr (VAR)
+      return c < prm.ncol ? __ldg(prm.v + c) : 0.0;
+    else
+      return 0.0;
+  };
+  auto term = [&](double xv, double mu) -> double {
+    if constexpr (VAR) {
+      const double d = __dsub_rn(xv, mu);
+      return __dmul_rn(d, d);
+    } else {
+      return xv;
+    }
+  };
+  auto finish = [&](int32_t c, double s) -> double {
+    if constexpr (VAR) {
+      if (prm.var_n == 0.0) return s;
+      return var_from_sums(s, static_cast<double>(__ldg(prm.p + c + 1) - __ldg(prm.p + c)), __ldg(prm.v + c), prm.var_n);
+    } else {
+      return s;
+    }
+  };
+  auto store_col = [&](int32_t c, double s) {
+    if constexpr (VAR)
+      prm.out[c] = (c == in_col) ? s : finish(c, s);
+    else
+      prm.out[c] = s;
+  };
+
   for (int j = 0; j < n_local; ++j) {
     const int s = j % STAGES;
     const int buf = j & 1;
@@ -264,20 +307,21 @@ __global__ void __launch_bounds__(SWEEP_BLOCK) sweep_kernel(const SweepParams pr
           if (c < nseg) {
             const int beg = (c == 0) ? 0 : as[c - 1] - mt.k0;
             const int end = (c == mt.nc) ? mt.nk : as[c] - mt.k0;
+            const double mu = mean_of(mt.c0 + c);
             double a0 = 0.0, a1 = 0.0;
             int k = beg + gl;
             for (; k + L < end; k += 2 * L) {
-              a0 = __dadd_rn(a0, xs[k]);
-              a1 = __dadd_rn(a1, xs[k + L]);
+              a0 = __dadd_rn(a0, term(xs[k], mu));
+              a1 = __dadd_rn(a1, term(xs[k + L], mu));
             }
-            if (k < end) a0 = __dadd_rn(a0, xs[k]);
+            if (k < end) a0 = __dadd_rn(a0, term(xs[k], mu));
             sacc = __dadd_rn(a0, a1);
           }
 #pragma unroll
           for (int off = L / 2; off > 0; off >>= 1) sacc = __dadd_rn(sacc, __shfl_xor_sync(0xffffffffu, sacc, off));
           if (gl == 0 && c < nseg) {
             if (c < mt.nc)
-              prm.out[mt.c0 + c] = (c == 0) ? __dadd_rn(cta_carry, sacc) : sacc;  // earlier CTAs' shares: fix-up below
+              store_col(mt.c0 + c, (c == 0) ? __dadd_rn(cta_carry, sacc) : sacc);  // earlier CTAs' shares: fix-up below
             else
               seg_carry[buf] = sacc;
           }
@@ -333,33 +377,36 @@ __global__ void __launch_bounds__(SWEEP_BLOCK) sweep_kernel(const SweepParams pr
       }
     } else if (n_my == IPT && ki + IPT <= col_end) {
       // common case (columns much longer than IPT): all my items are entries of one column
+      const double mu = mean_of(mt.c0 + ci);
       double a0 = 0.0, a1 = 0.0;
 #pragma unroll
       for (int it = 0; it + 1 < IPT; it += 2) {
-        a0 = __dadd_rn(a0, xs[ki + it]);
-        a1 = __dadd_rn(a1, xs[ki + it + 1]);
+        a0 = __dadd_rn(a0, term(xs[ki + it], mu));
+        a1 = __dadd_rn(a1, term(xs[ki + it + 1], mu));
       }
-      if (IPT & 1) a0 = __dadd_rn(a0, xs[ki + IPT - 1]);
+      if (IPT & 1) a0 = __dadd_rn(a0, term(xs[ki + IPT - 1], mu));
       acc = __dadd_rn(a0, a1);
     } else {
       // a column ends among my items (short columns; the row-ordered copy of a wide matrix): straight-line
       // adds, the rare end handled in place — the rest of the warp waits for this path, so it is unrolled
+      double mu = mean_of(mt.c0 + ci);
 #pragma unroll
       for (int it = 0; it < IPT; ++it) {
         if (it < n_my) {
           if (ki < col_end) {
-            acc = __dadd_rn(acc, xs[ki]);
+            acc = __dadd_rn(acc, term(xs[ki], mu));
             ++ki;
           } else {
             if (first_ci < 0) {
               first_ci = ci;
               head = acc;
             } else {
-              prm.out[mt.c0 + ci] = acc;  // began and ended inside this thread
+              store_col(mt.c0 + ci, acc);  // began and ended inside this thread
             }
             acc = 0.0;
             ++ci;
             col_end = as[ci] - mt.k0;
+            mu = mean_of(mt.c0 + ci);
           }
         }
       }
@@ -430,7 +477,7 @@ __global__ void __launch_bounds__(SWEEP_BLOCK) sweep_kernel(const SweepParams pr
           carry_in = prev_fl ? prev_sc : __dadd_rn(pre, prev_sc);
         // partial sums carried in by EARLIER CTAs (a column spanning CTA boundaries) are added
         // afterwards, in CTA order, by the last CTA to finish
-        prm.out[mt.c0 + first_ci] = __dadd_rn(carry_in, head);
+        store_col(mt.c0 + first_ci, __dadd_rn(carry_in, head));
       }
       cta_carry = all;
     }
@@ -462,7 +509,7 @@ __global__ void __launch_bounds__(SWEEP_BLOCK) sweep_kernel(const SweepParams pr
         double tot = 0.0;
         for (int h = g; h < G_ && __ldcg(prm.carry_col + h) == col; ++h) tot = __dadd_rn(tot, __ldcg(prm.carry_val + h));
         // the CTA in which `col` ends stored only its own share (its cta_carry started from 0)
-        prm.out[col] = __dadd_rn(tot, __ldcg(prm.out + col));
+        prm.out[col] = finish(col, __dadd_rn(tot, __ldcg(prm.out + col)));
       }
       if (tid == 0) *prm.ticket = 0u;  // ready for the next launch
     }
@@ -549,7 +596,7 @@ static SweepConfig sweep_config(SweepMode mode) {
 }
 
 template <int MODE>
-using GeomOf = SweepGeom<(MODE == SWEEP_COLSUM) ? SWEEP_IPT : GATHER_IPT>;
+using GeomOf = SweepGeom<(MODE == SWEEP_COLSUM || MODE == SWEEP_COLVAR) ? SWEEP_IPT : GATHER_IPT>;
 
 template <int MODE, int STAGES>
 static int launch_sweep_t(sb200_matrix* m, const SweepParams& prm, int ctas_per_sm) {
@@ -611,19 +658,21 @@ int launch_vec_div(cudaStream_t s, double* d, int64_t n, double divisor) {
   return SB200_OK;
 }
 
-static int launch_tile_sweep(sb200_matrix* m, SweepMode mode, const double* d_v, double* d_out, int mask) {
+static int launch_tile_sweep(sb200_matrix* m, SweepMode mode, const double* d_v, double* d_out, int mask, double var_n = 0.0) {
   if (m->n_tiles == 0) return SB200_OK;  // ncol == 0 and nnz == 0: nothing to produce
+  const bool cols = (mode == SWEEP_COLSUM || mode == SWEEP_COLVAR);  // the column-sum geometry and plan
   SweepParams prm;
   prm.i = m->d_i;
   prm.p = m->d_p;
   prm.x = m->d_x;
-  prm.plan = (mode == SWEEP_COLSUM) ? m->d_plan : m->d_plan_g;
-  prm.n_tiles = (mode == SWEEP_COLSUM) ? m->n_tiles : m->n_tiles_g;
+  prm.plan = cols ? m->d_plan : m->d_plan_g;
+  prm.n_tiles = cols ? m->n_tiles : m->n_tiles_g;
   prm.ncol = m->ncol;
   prm.nnz = static_cast<int32_t>(m->nnz);
   prm.v = d_v;
   prm.out = d_out;
   prm.mask = mask;
+  prm.var_n = var_n;
   // workspace layout: [ticket u32 | pad to 16] [carry_col int32 x 1024] [carry_val f64 x 1024]
   unsigned char* ws = static_cast<unsigned char*>(m->d_ws);
   prm.ticket = reinterpret_cast<unsigned int*>(ws);
@@ -634,11 +683,14 @@ static int launch_tile_sweep(sb200_matrix* m, SweepMode mode, const double* d_v,
     case SWEEP_COLSUM: return launch_sweep_m<SWEEP_COLSUM>(m, prm, cfg);
     case SWEEP_SPMV_T: return launch_sweep_m<SWEEP_SPMV_T>(m, prm, cfg);
     case SWEEP_SPMV: return launch_sweep_m<SWEEP_SPMV>(m, prm, cfg);
+    case SWEEP_COLVAR: return launch_sweep_m<SWEEP_COLVAR>(m, prm, cfg);
     default: return fail(SB200_E_INVALID, "unknown sweep mode");
   }
 }
 
 int launch_sweep(sb200_matrix* m, SweepMode mode, const double* d_v, double divisor, double* d_out) {
+  if (mode == SWEEP_COLVAR) return launch_col_vars(m, d_out);  // two passes (vars.cu)
+  if (mode == SWEEP_ROWVAR) return launch_row_vars(m, d_out);
   if ((mode == SWEEP_ROWSUM || mode == SWEEP_SPMV) && m->nnz > 0 && m->nrow > 0) {
     // A mirror whose row-indexed sweeps keep being asked for gets a row-major copy of itself: from then on a
     // row sum is the same streaming segmented sweep as a column sum (8 B per entry, no atomics) and A v is the
@@ -715,5 +767,11 @@ int launch_sweep(sb200_matrix* m, SweepMode mode, const double* d_v, double divi
 // writes with InnerIteratorInRange / InnerIteratorNotInRange (reference RcppSparse.h:238-321), all columns at once.
 // Always the tile sweep on the CSC arrays: skipping an entry is not the same as multiplying it by 0.0.
 int launch_masked_col_sums(sb200_matrix* m, const double* d_mask, double* d_out) { return launch_tile_sweep(m, SWEEP_SPMV_T, d_mask, d_out, 1); }
+
+// Second pass of colVars: d_out[c] = var_from_sums(sum over column c's entries of (x - d_mean[c])^2, its entry count,
+// d_mean[c], n), or the sum itself when n = 0.  Same tiles, walk and carry fold as the column sums.
+int launch_col_var_sweep(sb200_matrix* m, const double* d_mean, double n, double* d_out) {
+  return launch_tile_sweep(m, SWEEP_COLVAR, d_mean, d_out, 0, n);
+}
 
 }  // namespace sb200

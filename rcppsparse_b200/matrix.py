@@ -194,6 +194,15 @@ class DeviceMatrix:
     def row_means(self, out=None):
         return self._host_vec(_lib.lib().sb200_row_means, self.nrow, out)
 
+    def col_vars(self, out=None):
+        """Sample variance of every column, implicit zeros included, over nrow - 1 (R's var(A[, c])); two passes around
+        the col_means result (sparse_b200.h sb200_col_vars).  NaN everywhere when nrow < 2."""
+        return self._host_vec(_lib.lib().sb200_col_vars, self.ncol, out)
+
+    def row_vars(self, out=None):
+        """Sample variance of every row over ncol - 1 (R's var(A[r, ])), around the row_means result."""
+        return self._host_vec(_lib.lib().sb200_row_vars, self.nrow, out)
+
     def crossprod(self):
         """Dense A^T A, (ncol, ncol), exactly symmetric (reference Matrix::crossprod(), RcppSparse.h:158-194)."""
         out = np.empty((self.ncol, self.ncol), np.float64)
@@ -271,6 +280,12 @@ class DeviceMatrix:
 
     def row_sums_dev(self, d_out, divisor: float = 0.0) -> None:
         check(_lib.lib().sb200_row_sums_dev(self._h, divisor, _ptr(d_out)))
+
+    def col_vars_dev(self, d_out) -> None:
+        check(_lib.lib().sb200_col_vars_dev(self._h, _ptr(d_out)))
+
+    def row_vars_dev(self, d_out) -> None:
+        check(_lib.lib().sb200_row_vars_dev(self._h, _ptr(d_out)))
 
     def spmv_dev(self, d_v, d_y) -> None:
         check(_lib.lib().sb200_spmv_dev(self._h, _ptr(d_v), _ptr(d_y)))
@@ -370,6 +385,14 @@ class ShardedHostMatrix:
 
     def row_means(self):
         return self._vec(_lib.lib().sb200_sharded_row_means, self.nrow)
+
+    def col_vars(self):
+        """Column variances on every GPU of the handle (sparse_b200.h sb200_sharded_col_vars)."""
+        return self._vec(_lib.lib().sb200_sharded_col_vars, self.ncol)
+
+    def row_vars(self):
+        """Row variances on every GPU of the handle: per-block sums of squares and counts, reduced in block order."""
+        return self._vec(_lib.lib().sb200_sharded_row_vars, self.nrow)
 
     def spmv(self, v):
         v = np.ascontiguousarray(v, np.float64)
@@ -592,6 +615,13 @@ class Matrix:
 
     def crossprod(self):
         return self._call(True, lambda m: m.crossprod())
+
+    # ---- sample variances of the columns / rows (sparseMatrixStats::colVars / rowVars): additions -------------------------
+    def colVars(self):
+        return self._call(True, lambda m: m.col_vars())
+
+    def rowVars(self):
+        return self._call(True, lambda m: m.row_vars())
 
     # ---- A v and A^T v: additions (the reference has only the iterator idiom, SURVEY.md D1) -----------------------------
     def spmv(self, v):
