@@ -705,42 +705,11 @@ __global__ void __launch_bounds__(BAND_THREADS) band_transpose_kernel(const Tran
   }
 }
 
-struct PhaseTrace {  // SB200_TRACE=1: per-phase device time on stderr
-  bool on;
-  cudaStream_t st;
-  cudaEvent_t ev[10];
-  const char* name[10];
-  int n = 0;
-  explicit PhaseTrace(cudaStream_t s) : on(getenv("SB200_TRACE") != nullptr), st(s) {}
-  void mark(const char* what) {
-    if (!on || n >= 10) return;
-    cudaEventCreate(&ev[n]);
-    cudaEventRecord(ev[n], st);
-    name[n++] = what;
-  }
-  void report(const char* title, const BandPlan* bp);
-};
-
 }  // namespace
 
 // ================================================================================================
 // the plan
 // ================================================================================================
-namespace {
-void PhaseTrace::report(const char* title, const BandPlan* bp) {
-  if (!on) return;
-  cudaStreamSynchronize(st);
-  fprintf(stderr, "[sb200 trace] %s nb=%d S=%d maxrows=%d:", title, bp ? bp->nb : 0, bp ? bp->S : 0, bp ? bp->max_rows : 0);
-  for (int k = 1; k < n; ++k) {
-    float ms = 0;
-    cudaEventElapsedTime(&ms, ev[k - 1], ev[k]);
-    fprintf(stderr, " %s %.3f ms;", name[k], ms);
-  }
-  fprintf(stderr, "\n");
-  for (int k = 0; k < n; ++k) cudaEventDestroy(ev[k]);
-}
-}  // namespace
-
 void free_band_plan(BandPlan* bp, cudaStream_t s) {
   if (!bp) return;
   pool_free(bp->d_rb, s);
@@ -867,7 +836,7 @@ int build_band_plan(sb200_matrix* m, int rows_cap, int want_bands, int S, BandPl
   tr.mark("band ptrs");
   SB_CUDA(cudaStreamSynchronize(st));
   bp->max_rows = h_maxrows;
-  tr.report("band plan", bp);
+  tr.report("band plan nb=%d S=%d maxrows=%d:", bp->nb, bp->S, bp->max_rows);
   if (h_maxrows > rows_cap) return fail(SB200_E_UNSUPPORTED, "band plan: a row band exceeds its shared-memory budget");
   guard.armed = false;
   *out = bp;

@@ -5,7 +5,6 @@
 #include <string.h>
 
 #include <atomic>
-#include <chrono>
 #include <thread>
 #include <new>
 #include <string>
@@ -233,15 +232,9 @@ int finish_matrix(sb200_matrix* m, unsigned flags) {
 // colSums on a matrix whose `i` is garbage (it never reads it, RcppSparse.h:133-135).
 int ensure_rows(sb200_matrix* m) {
   if (!m->lazy_i) return SB200_OK;
-  const int32_t* i = m->lazy_i;
-  const size_t bi = sizeof(int32_t) * static_cast<size_t>(m->nnz);
-  if (m->nnz > 0 && bi >= STAGED_COPY_MIN_BYTES && host_is_pageable(i)) {
-    SB_CUDA(cudaStreamSynchronize(m->stream));  // d_i was allocated in this stream's order; the workers use their own
-    SB_TRY(staged_h2d(m->device, m->d_i, i, bi));
-  } else if (m->nnz > 0) {
-    SB_CUDA(cudaMemcpyAsync(m->d_i, i, bi, cudaMemcpyHostToDevice, m->stream));
-    SB_CUDA(cudaStreamSynchronize(m->stream));  // the caller's array is not needed after this call
-  }
+  SB_TRY(host_copies(m->device, m->stream, cudaMemcpyHostToDevice,
+                     {{const_cast<int32_t*>(m->lazy_i), m->d_i, sizeof(int32_t) * static_cast<size_t>(m->nnz)}}));
+  SB_CUDA(cudaStreamSynchronize(m->stream));  // the caller's array is not needed after this call
   if (m->lazy_validate) SB_TRY(validate_rows(m));
   m->lazy_i = nullptr;
   return SB200_OK;
@@ -326,8 +319,8 @@ int sb200_matrix_create(const int32_t* i, const int32_t* p, const double* x, int
   std::string x_err_text;  // sb200_last_error() is per thread: the values-upload thread reports through this
   // Pageable arrays (what R owns) go through the worker threads of hostcopy.cu; pinned or registered ones are
   // handed to the copy engine directly.
-  const bool stage_i = nnz > 0 && !lazy && !pinned_i && bi >= STAGED_COPY_MIN_BYTES && host_is_pageable(i);
-  const bool stage_x = nnz > 0 && !pinned_x && bx >= STAGED_COPY_MIN_BYTES && host_is_pageable(x);
+  const bool stage_i = nnz > 0 && !lazy && !pinned_i && copy_is_staged(i, bi);
+  const bool stage_x = nnz > 0 && !pinned_x && copy_is_staged(x, bx);
   cudaStream_t xs = nullptr;
   cudaError_t e = cudaStreamCreateWithFlags(&xs, cudaStreamNonBlocking);
   int rc = SB200_OK, rc_x = SB200_OK;
@@ -343,16 +336,11 @@ int sb200_matrix_create(const int32_t* i, const int32_t* p, const double* x, int
     if (allocated) cudaEventDestroy(allocated);
   }
   if (e == cudaSuccess) e = cudaMemcpyAsync(m->d_p, p, bp, cudaMemcpyHostToDevice, m->stream);
-  if (e == cudaSuccess && nnz > 0 && !lazy) {
-    if (stage_i)
-      rc = staged_h2d(device, m->d_i, i, bi);
-    else
-      e = cudaMemcpyAsync(m->d_i, i, bi, cudaMemcpyHostToDevice, m->stream);
-  }
+  if (e == cudaSuccess && nnz > 0 && !lazy) rc = host_copies(device, m->stream, cudaMemcpyHostToDevice, {{const_cast<int32_t*>(i), m->d_i, bi}});
   if (e == cudaSuccess && rc == SB200_OK && nnz > 0) {
     if (stage_x) {
       x_thread = std::thread([&] {
-        rc_x = staged_h2d(device, m->d_x, x, bx);
+        rc_x = host_copies(device, xs, cudaMemcpyHostToDevice, {{const_cast<double*>(x), m->d_x, bx}});
         if (rc_x != SB200_OK) x_err_text = sb200_last_error();
       });
     } else {
@@ -446,12 +434,8 @@ int sb200_matrix_refresh_values(sb200_matrix* m, const double* x) {
   if (!x) return fail(SB200_E_INVALID, "x is NULL");
   drop_row_companion(m);  // its values are the old ones; the call count starts over
   drop_band_companion(m, m->stream);
-  const size_t bx = sizeof(double) * static_cast<size_t>(m->nnz);
-  if (bx >= STAGED_COPY_MIN_BYTES && host_is_pageable(x)) {
-    SB_CUDA(cudaStreamSynchronize(m->stream));  // nothing on the stream still reads the old values
-    return staged_h2d(m->device, m->d_x, x, bx);
-  }
-  SB_CUDA(cudaMemcpyAsync(m->d_x, x, bx, cudaMemcpyHostToDevice, m->stream));
+  SB_TRY(host_copies(m->device, m->stream, cudaMemcpyHostToDevice,
+                     {{const_cast<double*>(x), m->d_x, sizeof(double) * static_cast<size_t>(m->nnz)}}));
   SB_CUDA(cudaStreamSynchronize(m->stream));
   return SB200_OK;
 }
@@ -617,41 +601,30 @@ int sb200_spmv_t(sb200_matrix* m, const double* v, double* y) {
 int sb200_transpose(sb200_matrix* m, int32_t* p_out, int32_t* i_out, double* x_out) {
   ENTER(m);
   if (!p_out || (m->nnz > 0 && (!i_out || !x_out))) return fail(SB200_E_INVALID, "NULL output array");
-  const bool trace = getenv("SB200_TRACE") != nullptr;
-  auto t_prev = std::chrono::steady_clock::now();
-  auto phase = [&](const char* what) {
-    if (!trace) return;
-    const auto now = std::chrono::steady_clock::now();
-    fprintf(stderr, "[sb200 trace] transpose to host: %s %.2f ms\n", what, std::chrono::duration<double, std::milli>(now - t_prev).count());
-    t_prev = now;
-  };
+  WallTrace tr("transpose to host");
   sb200_matrix* t = nullptr;
   SB_TRY(alloc_matrix(m->device, m->ncol, m->nrow, m->nnz, &t));
   cudaStreamSynchronize(t->stream);  // t's arrays were allocated in its own stream's order, written in m's
-  phase("result allocated");
+  tr.phase("result allocated");
   int rc = transpose_device(m, t->d_p, t->d_i, t->d_x);
   cudaError_t e = cudaSuccess;
   if (rc == SB200_OK) {
     const size_t bi = sizeof(int32_t) * static_cast<size_t>(m->nnz), bx = sizeof(double) * static_cast<size_t>(m->nnz);
     e = cudaMemcpyAsync(p_out, t->d_p, sizeof(int32_t) * (static_cast<size_t>(m->nrow) + 1), cudaMemcpyDeviceToHost, m->stream);
-    // the result goes back into the caller's (R-allocated, pageable) vectors: through the pinned-chunk workers
-    const bool stage_i = m->nnz > 0 && bi >= STAGED_COPY_MIN_BYTES && host_is_pageable(i_out);
-    const bool stage_x = m->nnz > 0 && bx >= STAGED_COPY_MIN_BYTES && host_is_pageable(x_out);
-    if (e == cudaSuccess && m->nnz > 0 && !stage_i) e = cudaMemcpyAsync(i_out, t->d_i, bi, cudaMemcpyDeviceToHost, m->stream);
-    if (e == cudaSuccess && m->nnz > 0 && !stage_x) e = cudaMemcpyAsync(x_out, t->d_x, bx, cudaMemcpyDeviceToHost, m->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(m->stream);  // the transposed arrays are complete
-    phase("transposed on the device (plan + kernels, p' copied)");
-    if (e == cudaSuccess && stage_i) rc = staged_d2h(m->device, i_out, t->d_i, bi);
-    phase("i' to the host");
-    if (e == cudaSuccess && rc == SB200_OK && stage_x) rc = staged_d2h(m->device, x_out, t->d_x, bx);
-    phase("x' to the host");
+    // the result goes back into the caller's (R-allocated, pageable) vectors: large ones through the pinned-chunk workers,
+    // once the transposed arrays are complete
+    if (e == cudaSuccess)
+      rc = host_copies(m->device, m->stream, cudaMemcpyDeviceToHost,
+                       {{i_out, t->d_i, bi, 1, 0, 0, "i' to the host"}, {x_out, t->d_x, bx, 1, 0, 0, "x' to the host"}}, &tr,
+                       "transposed on the device (plan + kernels, p' copied)");
+    if (e == cudaSuccess && rc == SB200_OK) e = cudaStreamSynchronize(m->stream);
   }
   if (rc != SB200_OK || e != cudaSuccess) {
     cudaStreamSynchronize(m->stream);  // nothing on m's stream still touches t's arrays when they are freed
     cudaGetLastError();
   }
   free_matrix(t);
-  phase("result freed");
+  tr.phase("result freed");
   if (rc != SB200_OK) return rc;
   if (e != cudaSuccess) return cuda_fail(e, "download of the transposed matrix", __FILE__, __LINE__);
   return SB200_OK;
@@ -676,22 +649,10 @@ static int spmm_to_host(sb200_matrix* m, bool transposed, const double* B, int64
   double *d_B = nullptr, *d_Y = nullptr;
   int rc = pool_alloc(reinterpret_cast<void**>(&d_B), b_bytes > 0 ? b_bytes : 16, m->stream);
   if (rc == SB200_OK) rc = pool_alloc(reinterpret_cast<void**>(&d_Y), y_bytes > 0 ? y_bytes : 16, m->stream);
-  // R's matrices are pageable: large ones go through the pinned-chunk workers, which use their own streams
-  if (rc == SB200_OK && b_bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(B)) {
-    rc = cudaStreamSynchronize(m->stream) == cudaSuccess ? SB200_OK : fail(SB200_E_CUDA, "spmm: stream sync failed");
-    if (rc == SB200_OK) rc = staged_h2d(m->device, d_B, B, b_bytes);
-  } else if (rc == SB200_OK && b_bytes > 0) {
-    const cudaError_t e = cudaMemcpyAsync(d_B, B, b_bytes, cudaMemcpyHostToDevice, m->stream);
-    if (e != cudaSuccess) rc = cuda_fail(e, "spmm: operand upload", __FILE__, __LINE__);
-  }
+  // R's matrices are pageable: large ones go through the pinned-chunk workers
+  if (rc == SB200_OK) rc = host_copies(m->device, m->stream, cudaMemcpyHostToDevice, {{const_cast<double*>(B), d_B, b_bytes}});
   if (rc == SB200_OK) rc = launch_spmm(m, transposed, d_B, k, d_Y);
-  if (rc == SB200_OK && y_bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(Y)) {
-    rc = cudaStreamSynchronize(m->stream) == cudaSuccess ? SB200_OK : fail(SB200_E_CUDA, "spmm: stream sync failed");
-    if (rc == SB200_OK) rc = staged_d2h(m->device, Y, d_Y, y_bytes);
-  } else if (rc == SB200_OK && y_bytes > 0) {
-    const cudaError_t e = cudaMemcpyAsync(Y, d_Y, y_bytes, cudaMemcpyDeviceToHost, m->stream);
-    if (e != cudaSuccess) rc = cuda_fail(e, "spmm: result download", __FILE__, __LINE__);
-  }
+  if (rc == SB200_OK) rc = host_copies(m->device, m->stream, cudaMemcpyDeviceToHost, {{Y, d_Y, y_bytes}});
   const cudaError_t es = cudaStreamSynchronize(m->stream);
   if (rc == SB200_OK && es != cudaSuccess) rc = cuda_fail(es, "spmm: stream sync", __FILE__, __LINE__);
   if (rc == SB200_E_NOMEM) cudaGetLastError();

@@ -2,9 +2,14 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <stdarg.h>
 #include <stdint.h>
+#include <stdio.h>
+#include <stdlib.h>
 
 #include <atomic>
+#include <chrono>
+#include <initializer_list>
 #include <string>
 
 #include "../../include/sparse_b200.h"
@@ -129,6 +134,58 @@ struct DeviceGuard {
   }
 };
 
+// SB200_TRACE=1: host wall clock of the phases of an entry point on stderr, one line per phase
+struct WallTrace {
+  bool on = getenv("SB200_TRACE") != nullptr;
+  const char* title;
+  std::chrono::steady_clock::time_point t = std::chrono::steady_clock::now();
+  explicit WallTrace(const char* what) : title(what) {}
+  void phase(const char* what) {
+    if (!on) return;
+    const auto now = std::chrono::steady_clock::now();
+    fprintf(stderr, "[sb200 trace] %s: %s %.2f ms\n", title, what, std::chrono::duration<double, std::milli>(now - t).count());
+    t = now;
+  }
+};
+
+// SB200_TRACE=1: device time between marks on one stream, one line on stderr.  mark(name) records an event; report()
+// prints the caller's header and then " name ms;" for the gap that ends at every mark after the first.
+struct PhaseTrace {
+  static constexpr int MAX_MARKS = 8;
+  bool on = getenv("SB200_TRACE") != nullptr;
+  cudaStream_t st;
+  cudaEvent_t ev[MAX_MARKS];
+  const char* name[MAX_MARKS];
+  int n = 0;
+  explicit PhaseTrace(cudaStream_t s) : st(s) {}
+  ~PhaseTrace() {
+    for (int k = 0; k < n; ++k) cudaEventDestroy(ev[k]);
+  }
+  void mark(const char* what) {
+    if (!on || n >= MAX_MARKS) return;
+    cudaEventCreate(&ev[n]);
+    cudaEventRecord(ev[n], st);
+    name[n++] = what;
+  }
+  __attribute__((format(printf, 2, 3))) void report(const char* header, ...) {
+    if (!on) return;
+    cudaStreamSynchronize(st);
+    char buf[256];
+    va_list ap;
+    va_start(ap, header);
+    vsnprintf(buf, sizeof(buf), header, ap);
+    va_end(ap);
+    std::string line = std::string("[sb200 trace] ") + buf;
+    for (int k = 1; k < n; ++k) {
+      float ms = 0;
+      cudaEventElapsedTime(&ms, ev[k - 1], ev[k]);
+      snprintf(buf, sizeof(buf), " %s %.3f ms;", name[k], ms);
+      line += buf;
+    }
+    fprintf(stderr, "%s\n", line.c_str());  // one write: concurrent plans on other threads do not cut into the line
+  }
+};
+
 // sweep.cu
 // COLVAR / ROWVAR: colVars / rowVars through launch_sweep (vars.cu); COLVAR is also the kernel mode of their second pass
 enum SweepMode { SWEEP_COLSUM = 0, SWEEP_SPMV_T = 1, SWEEP_ROWSUM = 2, SWEEP_SPMV = 3, SWEEP_COLVAR = 4, SWEEP_ROWVAR = 5 };
@@ -181,14 +238,25 @@ bool split_transpose_fits(const sb200_matrix* m);
 int transpose_split_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, double* d_x_out);
 void free_split_plan(SplitPlan* sp, cudaStream_t s);
 int64_t split_plan_bytes(const SplitPlan* sp);
-// hostcopy.cu: pageable host memory through worker threads with pinned chunks (blocking)
-bool host_is_pageable(const void* p);
-int staged_h2d(int device, void* d_dst, const void* h_src, size_t bytes);
-int staged_d2h(int device, void* h_dst, const void* d_src, size_t bytes);
-// strided: `runs` runs of `width` bytes, dpitch / hpitch bytes apart on the device / the host
-int staged_h2d_2d(int device, void* d_dst, size_t dpitch, const void* h_src, size_t hpitch, size_t width, size_t runs);
-int staged_d2h_2d(int device, void* h_dst, size_t hpitch, const void* d_src, size_t dpitch, size_t width, size_t runs);
-constexpr size_t STAGED_COPY_MIN_BYTES = 32u << 20;  // below this the driver's own staging is as good
+// hostcopy.cu: copies between host and device memory.  One copy is `runs` runs of `width` bytes, hpitch / dpitch bytes
+// apart on the host / the device (runs = 1: a contiguous range).
+struct HostCopy {
+  void* host;
+  void* dev;
+  size_t width;
+  size_t runs = 1;
+  size_t hpitch = 0, dpitch = 0;
+  const char* phase = nullptr;  // SB200_TRACE: the WallTrace phase that ends when this copy has arrived
+};
+// Whether a copy of `bytes` from or to `host` goes through the pinned-chunk workers: large, and in pageable memory (what
+// R owns), which the driver would stage through one pinned buffer from one thread.
+bool copy_is_staged(const void* host, size_t bytes);
+// Copies in one direction between host memory and `device`, for work on stream `st`.  The copies the driver does well
+// are enqueued on the stream first; then, if any copy is staged, the stream is synchronised and the staged copies run
+// through the pinned-chunk workers.  Returns when the staged copies have arrived; the others are only enqueued.  With a
+// trace that is on, the stream is synchronised in any case and reported as `synced`, then every copy's `phase`.
+int host_copies(int device, cudaStream_t st, cudaMemcpyKind kind, std::initializer_list<HostCopy> copies, WallTrace* tr = nullptr,
+                const char* synced = nullptr);
 int launch_crossprod(const sb200_matrix* T, int32_t ncol_a, double* d_res, cudaStream_t st);  // crossprod.cu
 // crossprod.cu: slab (ncol x blk->ncol, column-major) = A^T A_blk in ascending row order, on blk's stream; rp / rc / rv are
 // the row-ordered copy of the WHOLE matrix (global column ids) on blk's device

@@ -9,6 +9,7 @@
 // Buffers, streams and events are created once per process and device.
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 #include <thread>
 #include <vector>
@@ -190,7 +191,7 @@ Span span(void* d, const void* h, size_t dpitch, size_t hpitch, size_t width, si
   return Span{static_cast<unsigned char*>(d), static_cast<unsigned char*>(const_cast<void*>(h)), dpitch, hpitch, width, runs};
 }
 
-}  // namespace
+constexpr size_t STAGED_COPY_MIN_BYTES = 32u << 20;  // below this the driver's own staging is as good
 
 // true for ordinary malloc'ed / R-allocated memory (neither cudaHostAlloc'ed nor cudaHostRegister'ed nor managed)
 bool host_is_pageable(const void* p) {
@@ -203,19 +204,35 @@ bool host_is_pageable(const void* p) {
   return attr.type == cudaMemoryTypeUnregistered;
 }
 
-// Blocking.  The device range must not be in use by work that has not completed (callers synchronise the stream
-// that allocated / produced it first); on return the data has arrived.
-int staged_h2d(int device, void* d_dst, const void* h_src, size_t bytes) { return staged(device, span(d_dst, h_src, 0, 0, bytes, 1), true); }
-int staged_d2h(int device, void* h_dst, const void* d_src, size_t bytes) {
-  return staged(device, span(const_cast<void*>(d_src), h_dst, 0, 0, bytes, 1), false);
-}
-// Strided forms: `runs` runs of `width` bytes, `dpitch` bytes apart on the device and `hpitch` apart on the host (a
-// column-major slice of a host matrix: runs = its columns).
-int staged_h2d_2d(int device, void* d_dst, size_t dpitch, const void* h_src, size_t hpitch, size_t width, size_t runs) {
-  return staged(device, span(d_dst, h_src, dpitch, hpitch, width, runs), true);
-}
-int staged_d2h_2d(int device, void* h_dst, size_t hpitch, const void* d_src, size_t dpitch, size_t width, size_t runs) {
-  return staged(device, span(const_cast<void*>(d_src), h_dst, dpitch, hpitch, width, runs), false);
+}  // namespace
+
+bool copy_is_staged(const void* host, size_t bytes) { return bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(host); }
+
+int host_copies(int device, cudaStream_t st, cudaMemcpyKind kind, std::initializer_list<HostCopy> copies, WallTrace* tr,
+                const char* synced) {
+  const bool up = kind == cudaMemcpyHostToDevice;
+  const bool traced = tr && tr->on;
+  std::vector<bool> stage;
+  for (const HostCopy& c : copies) {
+    const size_t bytes = c.width * c.runs;
+    stage.push_back(bytes > 0 && copy_is_staged(c.host, bytes));
+    if (bytes == 0 || stage.back()) continue;
+    if (c.runs == 1)
+      SB_CUDA(up ? cudaMemcpyAsync(c.dev, c.host, c.width, kind, st) : cudaMemcpyAsync(c.host, c.dev, c.width, kind, st));
+    else if (up)
+      SB_CUDA(cudaMemcpy2DAsync(c.dev, c.dpitch, c.host, c.hpitch, c.width, c.runs, kind, st));
+    else
+      SB_CUDA(cudaMemcpy2DAsync(c.host, c.hpitch, c.dev, c.dpitch, c.width, c.runs, kind, st));
+  }
+  // the workers use their own streams: whatever the stream still has to do with the device ranges comes first
+  if (traced || std::find(stage.begin(), stage.end(), true) != stage.end()) SB_CUDA(cudaStreamSynchronize(st));
+  if (traced && synced) tr->phase(synced);
+  size_t k = 0;
+  for (const HostCopy& c : copies) {
+    if (stage[k++]) SB_TRY(staged(device, span(c.dev, c.host, c.dpitch, c.hpitch, c.width, c.runs), up));
+    if (traced && c.phase) tr->phase(c.phase);
+  }
+  return SB200_OK;
 }
 
 }  // namespace sb200

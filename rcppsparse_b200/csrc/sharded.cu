@@ -34,7 +34,6 @@
 
 #include <algorithm>
 #include <limits>
-#include <chrono>
 #include <new>
 #include <string>
 #include <thread>
@@ -53,9 +52,10 @@ struct sb200_sharded {
   std::vector<sb200_matrix*> blocks;
   std::vector<sb200_exchange*> windows;
   int64_t partial_off, result_off;  // byte offsets of the row partial / the row result inside every window
-  // k-wide A B: per block a row-major nrow x k partial (cudaMalloc: peers read it), grown on demand, kept between calls
-  std::vector<double*> mm_partial;
-  std::vector<size_t> mm_partial_bytes;
+  // per block a partial its peers read (cudaMalloc: pool memory is not peer-readable), grown on demand, kept between
+  // calls: A B's row-major nrow x k partial, rowVars' sums and counts
+  std::vector<double*> peer_partial;
+  std::vector<size_t> peer_partial_bytes;
   std::vector<cudaEvent_t> ev_partial;  // per block: its partial is complete
   std::vector<cudaEvent_t> ev_reduced;  // per block: its reduce has read every partial
 };
@@ -70,16 +70,97 @@ int check_sharded(const sb200_sharded* s) {
   return SB200_OK;
 }
 
-struct WallTrace {  // SB200_TRACE=1: host wall clock of the phases of an entry point on stderr
-  bool on = getenv("SB200_TRACE") != nullptr;
-  const char* title;
-  std::chrono::steady_clock::time_point t = std::chrono::steady_clock::now();
-  explicit WallTrace(const char* what) : title(what) {}
-  void phase(const char* what) {
+// Waits for every block's stream, whatever happened on another; the first error
+cudaError_t sync_blocks(const sb200_sharded* s) {
+  cudaError_t first = cudaSuccess;
+  for (int w = 0; w < s->world; ++w) {
+    DeviceGuard g(s->blocks[w]->device);
+    const cudaError_t e = cudaStreamSynchronize(s->blocks[w]->stream);
+    if (first == cudaSuccess) first = e;
+  }
+  return first;
+}
+
+// fn(w) on one host thread per block, on the block's device; the first failure, with its message, is returned
+template <typename F>
+int on_every_block(const sb200_sharded* s, const char* what, F fn) {
+  std::vector<int> rcs(s->world, SB200_OK);
+  std::vector<std::string> errs(s->world);
+  std::vector<std::thread> workers;
+  for (int w = 0; w < s->world; ++w)
+    workers.emplace_back([&, w] {
+      if (cudaSetDevice(s->devices[w]) != cudaSuccess) {
+        rcs[w] = SB200_E_CUDA;
+        errs[w] = "cudaSetDevice failed";
+        return;
+      }
+      rcs[w] = fn(w);
+      if (rcs[w] != SB200_OK) errs[w] = sb200_last_error();
+    });
+  for (auto& t : workers) t.join();
+  for (int w = 0; w < s->world; ++w)
+    if (rcs[w] != SB200_OK)
+      return fail(rcs[w], std::string(what) + ", column block " + std::to_string(w) + " (device " + std::to_string(s->devices[w]) +
+                              "): " + errs[w]);
+  return SB200_OK;
+}
+
+// Contiguous ranges of [0, len) with about total / n entries each: out[0] = 0, out[n] = len, and out[k] the first index
+// whose offset off[index] reaches k * total / n.  off is a prefix array of len + 1 entries (p of a CSC matrix).
+template <typename B>
+void nnz_balanced_bounds(const int32_t* off, int64_t len, int64_t total, int n, B* out) {
+  out[0] = 0;
+  for (int k = 1; k < n; ++k) {
+    const int64_t target = (total * k) / n;
+    int64_t lo = out[k - 1], hi = len;
+    while (lo < hi) {
+      const int64_t mid = lo + ((hi - lo) >> 1);
+      if (off[mid] < target)
+        lo = mid + 1;
+      else
+        hi = mid;
+    }
+    out[k] = static_cast<B>(lo);
+  }
+  out[n] = static_cast<B>(len);
+}
+
+// SB200_TRACE=1: CUDA-event time of a call's device part on every block's stream, from start() to stop(); report()
+// prints its max and per-device times (tools/sharded_*_bench.py read "device part <ms> ms")
+struct DevicePartTimer {
+  const sb200_sharded* s;
+  bool on;
+  std::vector<cudaEvent_t> t0, t1;
+  DevicePartTimer(const sb200_sharded* sh, bool trace) : s(sh), on(trace), t0(sh->world, nullptr), t1(sh->world, nullptr) {}
+  ~DevicePartTimer() {
+    for (int w = 0; w < s->world; ++w) {
+      DeviceGuard g(s->blocks[w]->device);
+      if (t0[w]) cudaEventDestroy(t0[w]);
+      if (t1[w]) cudaEventDestroy(t1[w]);
+    }
+  }
+  int record(std::vector<cudaEvent_t>& ev) {
+    for (int w = 0; w < s->world && on; ++w) {
+      DeviceGuard g(s->blocks[w]->device);
+      if (!ev[w]) SB_CUDA(cudaEventCreate(&ev[w]));
+      SB_CUDA(cudaEventRecord(ev[w], s->blocks[w]->stream));
+    }
+    return SB200_OK;
+  }
+  int start() { return record(t0); }
+  int stop() { return record(t1); }
+  void report(const char* title) {  // every stream has passed stop()
     if (!on) return;
-    const auto now = std::chrono::steady_clock::now();
-    fprintf(stderr, "[sb200 trace] %s: %s %.2f ms\n", title, what, std::chrono::duration<double, std::milli>(now - t).count());
-    t = now;
+    std::string per;
+    float worst = 0.0f;
+    for (int w = 0; w < s->world; ++w) {
+      DeviceGuard g(s->blocks[w]->device);
+      float ms = 0.0f;
+      cudaEventElapsedTime(&ms, t0[w], t1[w]);
+      worst = std::max(worst, ms);
+      per += (w ? " " : "") + std::to_string(ms);
+    }
+    fprintf(stderr, "[sb200 trace] %s: device part %.4f ms (max over devices; per device: %s)\n", title, worst, per.c_str());
   }
 };
 
@@ -88,9 +169,9 @@ void destroy_sharded(sb200_sharded* s) {
   WallTrace tr("sharded destroy");
   for (cudaEvent_t e : s->ev_reduced)  // no reader still has a partial in flight (every call also ends synchronised)
     if (e) cudaEventSynchronize(e);
-  for (size_t k = 0; k < s->mm_partial.size(); ++k) {
+  for (size_t k = 0; k < s->peer_partial.size(); ++k) {
     DeviceGuard g(s->devices[k]);
-    if (s->mm_partial[k]) cudaFree(s->mm_partial[k]);
+    if (s->peer_partial[k]) cudaFree(s->peer_partial[k]);
   }
   for (size_t k = 0; k < s->ev_partial.size(); ++k) {
     DeviceGuard g(s->devices[k]);
@@ -124,11 +205,8 @@ int run_columns(sb200_sharded* s, SweepMode mode, const double* v_host, double d
       SB_CUDA(cudaMemcpyAsync(out + s->bounds[k], m->d_stage_out, sizeof(double) * static_cast<size_t>(m->ncol), cudaMemcpyDeviceToHost,
                               m->stream));
   }
-  for (int k = 0; k < s->world; ++k) {  // every device is waited for, whatever happened on another
-    DeviceGuard guard(s->blocks[k]->device);
-    const cudaError_t e = cudaStreamSynchronize(s->blocks[k]->stream);
-    if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded column sweep", __FILE__, __LINE__);
-  }
+  const cudaError_t e = sync_blocks(s);
+  if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded column sweep", __FILE__, __LINE__);
   return rc;
 }
 
@@ -171,11 +249,8 @@ int run_rows(sb200_sharded* s, SweepMode mode, const double* v_host, double divi
     SB_CUDA(cudaMemcpyAsync(out, exchange_window_base(s->windows[0]) + off, sizeof(double) * static_cast<size_t>(s->nrow),
                             cudaMemcpyDeviceToHost, s->blocks[0]->stream));
   }
-  for (int k = 0; k < s->world; ++k) {
-    DeviceGuard guard(s->blocks[k]->device);
-    const cudaError_t e = cudaStreamSynchronize(s->blocks[k]->stream);
-    if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded row sweep", __FILE__, __LINE__);
-  }
+  const cudaError_t e = sync_blocks(s);
+  if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded row sweep", __FILE__, __LINE__);
   return rc;
 }
 
@@ -244,10 +319,10 @@ struct RowExchange {
   std::vector<int64_t*> dstk;  // device k: its slice of dst
   RowExchange(sb200_sharded* sh, std::vector<const sb200_matrix*> t) : s(sh), T(std::move(t)), dstk(sh->world, nullptr) {}
   ~RowExchange() {  // released on every way out, once nothing reads it any more
-    for (int k = s->world - 1; k >= 0; --k) {
+    sync_blocks(s);
+    for (int k = s->world - 1; k > 0; --k) {
       DeviceGuard g(s->blocks[k]->device);
-      cudaStreamSynchronize(s->blocks[k]->stream);
-      if (k > 0) pool_free(dstk[k], s->blocks[k]->stream);
+      pool_free(dstk[k], s->blocks[k]->stream);
     }
     cudaStream_t st0 = s->blocks[0]->stream;
     DeviceGuard g(s->blocks[0]->device);
@@ -417,49 +492,10 @@ int launch_sum_transpose(cudaStream_t st, int sm_count, const PartialPtrs& P, in
   return SB200_OK;
 }
 
-// Strided copy between a column-major host matrix and a device buffer: `runs` columns of `width` bytes, hpitch / dpitch
-// bytes apart.  Blocking: returns when the data has arrived.  Large pageable ones go through the pinned-chunk workers,
-// the rest is one cudaMemcpy2DAsync on the block's stream.
-int copy_columns(const sb200_matrix* m, bool up, double* host, size_t hpitch, double* dev, size_t dpitch, size_t width, int64_t runs) {
-  if (width == 0 || runs == 0) return SB200_OK;
-  SB_CUDA(cudaStreamSynchronize(m->stream));  // the device buffer was allocated in the stream's order
-  if (width * static_cast<size_t>(runs) >= STAGED_COPY_MIN_BYTES && host_is_pageable(host))
-    return up ? staged_h2d_2d(m->device, dev, dpitch, host, hpitch, width, static_cast<size_t>(runs))
-              : staged_d2h_2d(m->device, host, hpitch, dev, dpitch, width, static_cast<size_t>(runs));
-  if (up)
-    SB_CUDA(cudaMemcpy2DAsync(dev, dpitch, host, hpitch, width, static_cast<size_t>(runs), cudaMemcpyHostToDevice, m->stream));
-  else
-    SB_CUDA(cudaMemcpy2DAsync(host, hpitch, dev, dpitch, width, static_cast<size_t>(runs), cudaMemcpyDeviceToHost, m->stream));
-  SB_CUDA(cudaStreamSynchronize(m->stream));
-  return SB200_OK;
-}
-
-// fn(w) on one host thread per block; the first failure, with its message, is returned
-template <typename F>
-int on_every_block(sb200_sharded* s, const char* what, F fn) {
-  std::vector<int> rcs(s->world, SB200_OK);
-  std::vector<std::string> errs(s->world);
-  std::vector<std::thread> workers;
-  for (int w = 0; w < s->world; ++w)
-    workers.emplace_back([&, w] {
-      if (cudaSetDevice(s->blocks[w]->device) != cudaSuccess) {
-        rcs[w] = SB200_E_CUDA;
-        errs[w] = "cudaSetDevice failed";
-        return;
-      }
-      rcs[w] = fn(w);
-      if (rcs[w] != SB200_OK) errs[w] = sb200_last_error();
-    });
-  for (auto& t : workers) t.join();
-  for (int w = 0; w < s->world; ++w)
-    if (rcs[w] != SB200_OK) return fail(rcs[w], std::string(what) + ", column block " + std::to_string(w) + ": " + errs[w]);
-  return SB200_OK;
-}
-
-int ensure_spmm_state(sb200_sharded* s) {
+int ensure_peer_partials(sb200_sharded* s) {
   if (!s->ev_partial.empty()) return SB200_OK;
-  s->mm_partial.assign(s->world, nullptr);
-  s->mm_partial_bytes.assign(s->world, 0);
+  s->peer_partial.assign(s->world, nullptr);
+  s->peer_partial_bytes.assign(s->world, 0);
   s->ev_partial.assign(s->world, nullptr);
   s->ev_reduced.assign(s->world, nullptr);
   for (int w = 0; w < s->world; ++w) {
@@ -472,17 +508,17 @@ int ensure_spmm_state(sb200_sharded* s) {
 
 // block w's partial holds at least `bytes`; the current device is block w's.  `what` names the partial in the error.
 int ensure_partial(sb200_sharded* s, int w, size_t bytes, const char* what) {
-  if (s->mm_partial_bytes[w] >= bytes) return SB200_OK;
+  if (s->peer_partial_bytes[w] >= bytes) return SB200_OK;
   for (cudaEvent_t e : s->ev_reduced) SB_CUDA(cudaEventSynchronize(e));  // no reader still has the old one in flight
-  if (s->mm_partial[w]) cudaFree(s->mm_partial[w]);
-  s->mm_partial[w] = nullptr;
-  s->mm_partial_bytes[w] = 0;
-  if (cudaMalloc(reinterpret_cast<void**>(&s->mm_partial[w]), bytes) != cudaSuccess) {
+  if (s->peer_partial[w]) cudaFree(s->peer_partial[w]);
+  s->peer_partial[w] = nullptr;
+  s->peer_partial_bytes[w] = 0;
+  if (cudaMalloc(reinterpret_cast<void**>(&s->peer_partial[w]), bytes) != cudaSuccess) {
     cudaGetLastError();
-    s->mm_partial[w] = nullptr;
+    s->peer_partial[w] = nullptr;
     return fail(SB200_E_NOMEM, std::string(what) + " does not fit on device " + std::to_string(s->devices[w]));
   }
-  s->mm_partial_bytes[w] = bytes;
+  s->peer_partial_bytes[w] = bytes;
   return SB200_OK;
 }
 
@@ -505,7 +541,7 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
     return fail(SB200_E_NOMEM, "spmm: the dense operand or result does not fit in device memory");
   WallTrace tr(transposed ? "sharded spmm_t" : "sharded spmm");
   DeviceGuard restore(s->blocks[0]->device);
-  SB_TRY(ensure_spmm_state(s));
+  SB_TRY(ensure_peer_partials(s));
   // rows of the operand block w reads and of the result piece it brings home
   auto b_lo = [&](int w) { return transposed ? int64_t{0} : s->bounds[w]; };
   auto b_n = [&](int w) { return transposed ? nrow : s->bounds[w + 1] - s->bounds[w]; };
@@ -518,7 +554,7 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
     DeviceGuard g(m->device);
     const double partial = transposed ? 0.0 : 8.0 * static_cast<double>(k) * static_cast<double>(nrow);
     const double need = 8.0 * static_cast<double>(k) * static_cast<double>(b_n(w) + y_n(w)) +
-                        std::max(0.0, partial - static_cast<double>(s->mm_partial_bytes[w]));
+                        std::max(0.0, partial - static_cast<double>(s->peer_partial_bytes[w]));
     if (need > static_cast<double>(device_free_bytes())) {
       rc = fail(SB200_E_NOMEM, "sharded spmm: the operand, result and partial of block " + std::to_string(w) +
                                    " do not fit on device " + std::to_string(m->device));
@@ -530,22 +566,23 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
     if (rc == SB200_OK && !transposed) rc = ensure_partial(s, w, sizeof(double) * static_cast<size_t>(nrow * k), "sharded spmm: the row-major partial (8 nrow k bytes)");
   }
   tr.phase("scratch");
+  // block w's piece of B or Y: n rows of each of the k columns of the host matrix (`rows` rows), blocking
+  auto copy_piece = [&](int w, cudaMemcpyKind kind, double* host, int64_t rows, double* dev, int64_t n) {
+    sb200_matrix* m = s->blocks[w];
+    const size_t width = sizeof(double) * static_cast<size_t>(n);
+    SB_TRY(host_copies(m->device, m->stream, kind, {{host, dev, width, static_cast<size_t>(k), sizeof(double) * static_cast<size_t>(rows), width}}));
+    SB_CUDA(cudaStreamSynchronize(m->stream));
+    return SB200_OK;
+  };
   // 1. operands up: block w's rows of B, a strided slice (A B) or all of it (A^T B)
   if (rc == SB200_OK)
     rc = on_every_block(s, "sharded spmm: operand upload", [&](int w) {
-      return copy_columns(s->blocks[w], true, const_cast<double*>(B) + b_lo(w), sizeof(double) * static_cast<size_t>(b_rows), dB[w],
-                          sizeof(double) * static_cast<size_t>(b_n(w)), sizeof(double) * static_cast<size_t>(b_n(w)), k);
+      return copy_piece(w, cudaMemcpyHostToDevice, const_cast<double*>(B) + b_lo(w), b_rows, dB[w], b_n(w));
     });
   tr.phase("operands up");
-  // 2. the device part, from every operand resident to every result piece complete (SB200_TRACE: CUDA-event time per device)
-  std::vector<cudaEvent_t> t0(W, nullptr), t1(W, nullptr);
-  const bool timed = tr.on;
-  for (int w = 0; w < W && timed && rc == SB200_OK; ++w) {
-    DeviceGuard g(s->blocks[w]->device);
-    if (cudaEventCreate(&t0[w]) != cudaSuccess || cudaEventCreate(&t1[w]) != cudaSuccess ||
-        cudaEventRecord(t0[w], s->blocks[w]->stream) != cudaSuccess)
-      rc = fail(SB200_E_CUDA, "sharded spmm: timing events");
-  }
+  // 2. the device part, from every operand resident to every result piece complete
+  DevicePartTimer dp(s, tr.on);
+  if (rc == SB200_OK) rc = dp.start();
   if (rc == SB200_OK && transposed) {
     for (int w = 0; w < W && rc == SB200_OK; ++w) {
       DeviceGuard g(s->blocks[w]->device);
@@ -556,8 +593,8 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
     for (int w = 0; w < W && rc == SB200_OK; ++w) {
       sb200_matrix* m = s->blocks[w];
       DeviceGuard g(m->device);
-      P.p[w] = s->mm_partial[w];
-      rc = launch_spmm_rm(m, false, dB[w], k, s->mm_partial[w]);
+      P.p[w] = s->peer_partial[w];
+      rc = launch_spmm_rm(m, false, dB[w], k, s->peer_partial[w]);
       if (rc == SB200_OK && cudaEventRecord(s->ev_partial[w], m->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaEventRecord");
     }
     for (int q = 0; q < W && rc == SB200_OK; ++q) {
@@ -569,44 +606,23 @@ int run_block_product(sb200_sharded* s, bool transposed, const double* B, int64_
       if (rc == SB200_OK && cudaEventRecord(s->ev_reduced[q], m->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaEventRecord");
     }
   }
-  for (int w = 0; w < W && timed && rc == SB200_OK; ++w) {
-    DeviceGuard g(s->blocks[w]->device);
-    if (cudaEventRecord(t1[w], s->blocks[w]->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "sharded spmm: timing events");
-  }
+  if (rc == SB200_OK) rc = dp.stop();
   tr.phase("launched");
   // 3. results home: block w's piece of Y, `y_n(w)` rows of every column
   if (rc == SB200_OK)
-    rc = on_every_block(s, "sharded spmm: result download", [&](int w) {
-      return copy_columns(s->blocks[w], false, Y + y_lo(w), sizeof(double) * static_cast<size_t>(y_rows), dY[w],
-                          sizeof(double) * static_cast<size_t>(y_n(w)), sizeof(double) * static_cast<size_t>(y_n(w)), k);
-    });
+    rc = on_every_block(s, "sharded spmm: result download",
+                        [&](int w) { return copy_piece(w, cudaMemcpyDeviceToHost, Y + y_lo(w), y_rows, dY[w], y_n(w)); });
   tr.phase("results home");
   // 4. every stream is waited for (no partial is rewritten or freed while a reader may still run), scratch released
+  const cudaError_t e = sync_blocks(s);
+  if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded spmm", __FILE__, __LINE__);
   for (int w = 0; w < W; ++w) {
     sb200_matrix* m = s->blocks[w];
     DeviceGuard g(m->device);
-    const cudaError_t e = cudaStreamSynchronize(m->stream);
-    if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded spmm", __FILE__, __LINE__);
     pool_free(dB[w], m->stream);
     pool_free(dY[w], m->stream);
   }
-  if (timed && rc == SB200_OK) {
-    std::string per;
-    float worst = 0.0f;
-    for (int w = 0; w < W; ++w) {
-      DeviceGuard g(s->blocks[w]->device);
-      float ms = 0.0f;
-      cudaEventElapsedTime(&ms, t0[w], t1[w]);
-      worst = std::max(worst, ms);
-      per += (w ? " " : "") + std::to_string(ms);
-    }
-    fprintf(stderr, "[sb200 trace] %s: device part %.4f ms (max over devices; per device: %s)\n", tr.title, worst, per.c_str());
-  }
-  for (int w = 0; w < W; ++w) {
-    DeviceGuard g(s->blocks[w]->device);
-    if (t0[w]) cudaEventDestroy(t0[w]);
-    if (t1[w]) cudaEventDestroy(t1[w]);
-  }
+  if (rc == SB200_OK) dp.report(tr.title);
   if (rc == SB200_E_NOMEM) cudaGetLastError();  // a refused allocation leaves the streams usable
   return rc;
 }
@@ -636,7 +652,7 @@ int run_row_vars(sb200_sharded* s, double* out) {
   const int W = s->world;
   const int64_t nrow = s->nrow;
   DeviceGuard restore(s->blocks[0]->device);
-  SB_TRY(ensure_spmm_state(s));
+  SB_TRY(ensure_peer_partials(s));
   int64_t mean_off = 0;
   int rc = rows_into_windows(s, SWEEP_ROWSUM, nullptr, static_cast<double>(s->ncol), &mean_off);
   PartialPtrs P{};
@@ -645,9 +661,9 @@ int run_row_vars(sb200_sharded* s, double* out) {
     DeviceGuard g(m->device);
     rc = ensure_partial(s, w, 2 * sizeof(double) * static_cast<size_t>(nrow), "sharded rowVars: the sums and counts (16 nrow bytes)");
     if (rc != SB200_OK) break;
-    P.p[w] = s->mm_partial[w];
+    P.p[w] = s->peer_partial[w];
     const double* mean = reinterpret_cast<const double*>(exchange_window_base(s->windows[w]) + mean_off);
-    rc = launch_row_var_sums(m, mean, s->mm_partial[w], s->mm_partial[w] + nrow);
+    rc = launch_row_var_sums(m, mean, s->peer_partial[w], s->peer_partial[w] + nrow);
     if (rc == SB200_OK && cudaEventRecord(s->ev_partial[w], m->stream) != cudaSuccess) rc = fail(SB200_E_CUDA, "cudaEventRecord");
   }
   for (int q = 0; q < W && rc == SB200_OK; ++q) {
@@ -669,11 +685,8 @@ int run_row_vars(sb200_sharded* s, double* out) {
       e = cudaMemcpyAsync(out + r0, m->d_stage_out + r0, sizeof(double) * static_cast<size_t>(r1 - r0), cudaMemcpyDeviceToHost, m->stream);
     if (e != cudaSuccess) rc = cuda_fail(e, "sharded rowVars: reduce", __FILE__, __LINE__);
   }
-  for (int w = 0; w < W; ++w) {  // every device is waited for, whatever happened on another
-    DeviceGuard g(s->blocks[w]->device);
-    const cudaError_t e = cudaStreamSynchronize(s->blocks[w]->stream);
-    if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded rowVars", __FILE__, __LINE__);
-  }
+  const cudaError_t e = sync_blocks(s);
+  if (e != cudaSuccess && rc == SB200_OK) rc = cuda_fail(e, "sharded rowVars", __FILE__, __LINE__);
   if (rc == SB200_E_NOMEM) cudaGetLastError();
   return rc;
 }
@@ -714,60 +727,27 @@ int sb200_sharded_create(const int32_t* i, const int32_t* p, const double* x, in
       return fail(SB200_E_NODEVICE, "requested CUDA device " + std::to_string(devices ? devices[k] : k) + " not present");
     }
   }
-  // nnz-balanced contiguous column blocks: first column whose start offset reaches k * nnz / n (SURVEY.md 8e)
-  s->bounds.assign(n_gpus + 1, 0);
-  for (int k = 1; k < n_gpus; ++k) {
-    const int64_t target = (nnz * k) / n_gpus;
-    int64_t lo = s->bounds[k - 1], hi = ncol;
-    while (lo < hi) {
-      const int64_t mid = lo + ((hi - lo) >> 1);
-      if (p[mid] < target)
-        lo = mid + 1;
-      else
-        hi = mid;
-    }
-    s->bounds[k] = lo;
-  }
-  s->bounds[n_gpus] = ncol;
+  // nnz-balanced contiguous column blocks (SURVEY.md 8e)
+  s->bounds.resize(n_gpus + 1);
+  nnz_balanced_bounds(p, ncol, nnz, n_gpus, s->bounds.data());
   s->blocks.assign(n_gpus, nullptr);
   s->windows.assign(n_gpus, nullptr);
   // upload the blocks concurrently: one worker per device
   WallTrace tr("sharded create");
-  std::vector<int> rcs(n_gpus, SB200_OK);
-  std::vector<std::string> errs(n_gpus);
-  std::vector<std::thread> workers;
-  for (int k = 0; k < n_gpus; ++k) {
-    workers.emplace_back([&, k] {
-      const int64_t c0 = s->bounds[k], c1 = s->bounds[k + 1];
-      const int64_t k0 = p[c0], k1 = p[c1];
-      std::vector<int32_t> pk(static_cast<size_t>(c1 - c0) + 1);
-      bool ok = true;
-      for (int64_t c = c0; c <= c1; ++c) {
-        pk[c - c0] = static_cast<int32_t>(p[c] - k0);
-        if (c > c0 && p[c] < p[c - 1]) ok = false;
-      }
-      if (!ok) {
-        rcs[k] = SB200_E_STRUCTURE;
-        errs[k] = "p is not monotone";
-        return;
-      }
-      rcs[k] = sb200_matrix_create(i + k0, pk.data(), x + k0, nrow, static_cast<int32_t>(c1 - c0), k1 - k0, s->devices[k], flags & ~SB200_LAZY_ROWS,
-                                   &s->blocks[k]);
-      if (rcs[k] != SB200_OK) errs[k] = sb200_last_error();
-    });
-  }
-  for (auto& w : workers) w.join();
-  tr.phase("blocks uploaded");
-  for (int k = 0; k < n_gpus; ++k)
-    if (rcs[k] != SB200_OK) {
-      const int rc = rcs[k];
-      const std::string msg = "column block " + std::to_string(k) + " (device " + std::to_string(s->devices[k]) + "): " + errs[k];
-      destroy_sharded(s);
-      return fail(rc, msg);
+  int rc = on_every_block(s, "sharded create", [&](int k) {
+    const int64_t c0 = s->bounds[k], c1 = s->bounds[k + 1];
+    const int64_t k0 = p[c0], k1 = p[c1];
+    std::vector<int32_t> pk(static_cast<size_t>(c1 - c0) + 1);
+    for (int64_t c = c0; c <= c1; ++c) {
+      pk[c - c0] = static_cast<int32_t>(p[c] - k0);
+      if (c > c0 && p[c] < p[c - 1]) return fail(SB200_E_STRUCTURE, "p is not monotone");
     }
+    return sb200_matrix_create(i + k0, pk.data(), x + k0, nrow, static_cast<int32_t>(c1 - c0), k1 - k0, s->devices[k], flags & ~SB200_LAZY_ROWS,
+                               &s->blocks[k]);
+  });
+  tr.phase("blocks uploaded");
   // windows: [row partial | row result], 256-byte aligned, behind the exchange header
   const int64_t vec = ((static_cast<int64_t>(nrow > 0 ? nrow : 1) * 8 + 255) / 256) * 256;
-  int rc = SB200_OK;
   int prev = 0;
   cudaGetDevice(&prev);
   for (int k = 0; k < n_gpus && rc == SB200_OK; ++k) {
@@ -892,36 +872,17 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
     return SB200_OK;
   }
   DeviceGuard restore(s->blocks[0]->device);
-  const bool trace = getenv("SB200_TRACE") != nullptr;
-  auto t_prev = std::chrono::steady_clock::now();
-  auto lap = [&](const char* what) {
-    if (!trace) return;
-    const auto now = std::chrono::steady_clock::now();
-    fprintf(stderr, "[sb200 trace] sharded transpose: %s %.2f ms\n", what, std::chrono::duration<double, std::milli>(now - t_prev).count());
-    t_prev = now;
-  };
-  // 1. local transposes, concurrently (the entry point blocks)
+  WallTrace tr("sharded transpose");
   std::vector<sb200_matrix*> T(W, nullptr);
-  std::vector<int> rcs(W, SB200_OK);
-  std::vector<std::string> errs(W);
-  {
-    std::vector<std::thread> workers;
-    for (int k = 0; k < W; ++k)
-      workers.emplace_back([&, k] {
-        rcs[k] = sb200_transpose_dev(s->blocks[k], &T[k]);
-        if (rcs[k] != SB200_OK) errs[k] = sb200_last_error();
-      });
-    for (auto& w : workers) w.join();
-  }
   struct Scratch {  // the local transposes and the owners' arrays are released on every way out
     std::vector<sb200_matrix*>& T;
     sb200_sharded* s;
     std::vector<int32_t*> oc;  // the owners' arrays: plain cudaMalloc, visible to the peers (pool memory is not)
     std::vector<double*> ov;
     ~Scratch() {
+      sync_blocks(s);
       for (int k = 0; k < s->world; ++k) {
         DeviceGuard g(s->blocks[k]->device);
-        cudaStreamSynchronize(s->blocks[k]->stream);
         if (k < static_cast<int>(oc.size()) && oc[k]) cudaFree(oc[k]);
         if (k < static_cast<int>(ov.size()) && ov[k]) cudaFree(ov[k]);
         if (T[k]) sb200_matrix_destroy(T[k]);
@@ -929,82 +890,49 @@ int sb200_sharded_transpose(sb200_sharded* s, int32_t* p_out, int32_t* i_out, do
       cudaGetLastError();
     }
   } sc{T, s};
-  lap("local transposes");
-  for (int k = 0; k < W; ++k)
-    if (rcs[k] != SB200_OK) return fail(rcs[k], "sharded transpose, column block " + std::to_string(k) + ": " + errs[k]);
+  // 1. local transposes, concurrently (the entry point blocks)
+  int rc = on_every_block(s, "sharded transpose", [&](int k) { return sb200_transpose_dev(s->blocks[k], &T[k]); });
+  tr.phase("local transposes");
+  SB_TRY(rc);
   // 2. row counts over the blocks -> p_out
   RowExchange rx(s, std::vector<const sb200_matrix*>(T.begin(), T.end()));
   SB_TRY(rx.count(p_out));
-  lap("row counts, scan, p_out");
+  tr.phase("row counts, scan, p_out");
   // 3. rows dealt to the devices: nnz-balanced contiguous ranges
   RowBounds rb;
-  rb.rb[0] = 0;
-  for (int q = 1; q < W; ++q) {
-    const int64_t target = (s->nnz * q) / W;
-    int32_t lo = rb.rb[q - 1], hi = nrow;
-    while (lo < hi) {
-      const int32_t mid = lo + ((hi - lo) >> 1);
-      if (p_out[mid] < target)
-        lo = mid + 1;
-      else
-        hi = mid;
-    }
-    rb.rb[q] = lo;
-  }
-  for (int q = W; q <= PUSH_MAX_RANKS; ++q) rb.rb[q] = nrow;
+  nnz_balanced_bounds(p_out, nrow, s->nnz, W, rb.rb);
+  for (int q = W + 1; q <= PUSH_MAX_RANKS; ++q) rb.rb[q] = nrow;
   SB_TRY(rx.offsets(rb));
-  {
-    // 4. the owners' arrays
-    sc.oc.assign(W, nullptr);
-    sc.ov.assign(W, nullptr);
-    for (int q = 0; q < W; ++q) {
-      DeviceGuard gq(s->blocks[q]->device);
-      const size_t n = static_cast<size_t>(p_out[rb.rb[q + 1]] - p_out[rb.rb[q]]);
-      SB_CUDA(cudaMalloc(reinterpret_cast<void**>(&sc.oc[q]), padded_bytes(sizeof(int32_t) * (n + 1))));
-      SB_CUDA(cudaMalloc(reinterpret_cast<void**>(&sc.ov[q]), padded_bytes(sizeof(double) * (n + 1))));
-    }
-    // 5. every device pushes its pieces
-    PtrDest pd;
-    for (int q = 0; q < PUSH_MAX_RANKS; ++q) {
-      pd.c[q] = q < W ? sc.oc[q] : nullptr;
-      pd.v[q] = q < W ? sc.ov[q] : nullptr;
-    }
-    SB_TRY(rx.push(rb, pd));
-    for (int k = 0; k < W; ++k) {
-      DeviceGuard gk(s->blocks[k]->device);
-      SB_CUDA(cudaStreamSynchronize(s->blocks[k]->stream));
-    }
-    lap("push");
-    // 6. every owner brings its range home over its own link
-    std::vector<int> drc(W, SB200_OK);
-    std::vector<std::thread> workers;
-    for (int q = 0; q < W; ++q)
-      workers.emplace_back([&, q] {
-        const int64_t o = p_out[rb.rb[q]];
-        const size_t n = static_cast<size_t>(p_out[rb.rb[q + 1]] - o);
-        if (n == 0) return;
-        const int dev = s->blocks[q]->device;
-        if (cudaSetDevice(dev) != cudaSuccess) {
-          drc[q] = SB200_E_CUDA;
-          return;
-        }
-        const size_t bi = sizeof(int32_t) * n, bx = sizeof(double) * n;
-        if (bi >= STAGED_COPY_MIN_BYTES && host_is_pageable(i_out + o))
-          drc[q] = staged_d2h(dev, i_out + o, sc.oc[q], bi);
-        else if (cudaMemcpy(i_out + o, sc.oc[q], bi, cudaMemcpyDeviceToHost) != cudaSuccess)
-          drc[q] = SB200_E_CUDA;
-        if (drc[q] != SB200_OK) return;
-        if (bx >= STAGED_COPY_MIN_BYTES && host_is_pageable(x_out + o))
-          drc[q] = staged_d2h(dev, x_out + o, sc.ov[q], bx);
-        else if (cudaMemcpy(x_out + o, sc.ov[q], bx, cudaMemcpyDeviceToHost) != cudaSuccess)
-          drc[q] = SB200_E_CUDA;
-      });
-    for (auto& w : workers) w.join();
-    lap("copies to the host");
-    for (int q = 0; q < W; ++q)
-      if (drc[q] != SB200_OK) return fail(drc[q], "sharded transpose: copying rows of device " + std::to_string(q) + " to the host failed");
+  // 4. the owners' arrays
+  sc.oc.assign(W, nullptr);
+  sc.ov.assign(W, nullptr);
+  for (int q = 0; q < W; ++q) {
+    DeviceGuard gq(s->blocks[q]->device);
+    const size_t n = static_cast<size_t>(p_out[rb.rb[q + 1]] - p_out[rb.rb[q]]);
+    SB_CUDA(cudaMalloc(reinterpret_cast<void**>(&sc.oc[q]), padded_bytes(sizeof(int32_t) * (n + 1))));
+    SB_CUDA(cudaMalloc(reinterpret_cast<void**>(&sc.ov[q]), padded_bytes(sizeof(double) * (n + 1))));
   }
-  return SB200_OK;
+  // 5. every device pushes its pieces
+  PtrDest pd;
+  for (int q = 0; q < PUSH_MAX_RANKS; ++q) {
+    pd.c[q] = q < W ? sc.oc[q] : nullptr;
+    pd.v[q] = q < W ? sc.ov[q] : nullptr;
+  }
+  SB_TRY(rx.push(rb, pd));
+  SB_CUDA(sync_blocks(s));
+  tr.phase("push");
+  // 6. every owner brings its range home over its own link
+  rc = on_every_block(s, "sharded transpose: copy to the host", [&](int q) {
+    sb200_matrix* m = s->blocks[q];
+    const int64_t o = p_out[rb.rb[q]];
+    const size_t n = static_cast<size_t>(p_out[rb.rb[q + 1]] - o);
+    SB_TRY(host_copies(m->device, m->stream, cudaMemcpyDeviceToHost,
+                       {{i_out + o, sc.oc[q], sizeof(int32_t) * n}, {x_out + o, sc.ov[q], sizeof(double) * n}}));
+    SB_CUDA(cudaStreamSynchronize(m->stream));
+    return SB200_OK;
+  });
+  tr.phase("copies to the host");
+  return rc;
 }
 
 // Matrix::crossprod() (RcppSparse.h:158-194): block w computes the full-height slab A^T A_w, result columns
@@ -1051,10 +979,10 @@ int sb200_sharded_crossprod(sb200_sharded* s, double* out) {
     std::vector<int32_t*> rp, rc;    // every block's copy of the whole matrix's rows
     std::vector<double*> rv, slab;
     ~Scratch() {
+      sync_blocks(s);
       for (int w = 0; w < s->world; ++w) {
         sb200_matrix* m = s->blocks[w];
         DeviceGuard g(m->device);
-        cudaStreamSynchronize(m->stream);
         if (rc[w]) cudaFree(rc[w]);
         if (rv[w]) cudaFree(rv[w]);
         pool_free(rp[w], m->stream);
@@ -1109,26 +1037,9 @@ int sb200_sharded_crossprod(sb200_sharded* s, double* out) {
   }
   if (rc != SB200_OK) return rc;
   tr.phase("scratch");
-  // 4. the device part: the gather, then the ordered sweep (SB200_TRACE: CUDA-event time per device)
-  std::vector<cudaEvent_t> t0(W, nullptr), t1(W, nullptr);
-  struct Events {
-    sb200_sharded* s;
-    std::vector<cudaEvent_t>& a;
-    std::vector<cudaEvent_t>& b;
-    ~Events() {
-      for (int w = 0; w < s->world; ++w) {
-        DeviceGuard g(s->blocks[w]->device);
-        if (a[w]) cudaEventDestroy(a[w]);
-        if (b[w]) cudaEventDestroy(b[w]);
-      }
-    }
-  } ev{s, t0, t1};
-  for (int w = 0; w < W && tr.on; ++w) {
-    DeviceGuard g(s->blocks[w]->device);
-    SB_CUDA(cudaEventCreate(&t0[w]));
-    SB_CUDA(cudaEventCreate(&t1[w]));
-    SB_CUDA(cudaEventRecord(t0[w], s->blocks[w]->stream));
-  }
+  // 4. the device part: the gather, then the ordered sweep
+  DevicePartTimer dp(s, tr.on);
+  SB_TRY(dp.start());
   for (int w = 0; w < W; ++w) {
     if (ncol_w(w) == 0) continue;
     sb200_matrix* m0 = s->blocks[0];
@@ -1140,42 +1051,24 @@ int sb200_sharded_crossprod(sb200_sharded* s, double* out) {
     pd.v[0] = sc.rv[w];
     SB_TRY(rx.push(all, pd));
   }
-  for (int w = 0; w < W; ++w) {  // every piece has landed in every copy
-    DeviceGuard g(s->blocks[w]->device);
-    SB_CUDA(cudaStreamSynchronize(s->blocks[w]->stream));
-  }
+  SB_CUDA(sync_blocks(s));  // every piece has landed in every copy
   tr.phase("rows gathered");
   for (int w = 0; w < W; ++w) {
     DeviceGuard g(s->blocks[w]->device);
     SB_TRY(launch_crossprod_slab(s->blocks[w], sc.rp[w], sc.rc[w], sc.rv[w], ncol, sc.slab[w]));
-    if (tr.on) SB_CUDA(cudaEventRecord(t1[w], s->blocks[w]->stream));
   }
+  SB_TRY(dp.stop());
   tr.phase("launched");
   // 5. every slab home over its block's own link
   SB_TRY(on_every_block(s, "sharded crossprod: result download", [&](int w) {
     sb200_matrix* m = s->blocks[w];
     const size_t bytes = sizeof(double) * static_cast<size_t>(ncol) * static_cast<size_t>(ncol_w(w));
-    if (bytes == 0) return SB200_OK;
-    double* host = out + s->bounds[w] * ncol;
-    SB_CUDA(cudaStreamSynchronize(m->stream));
-    if (bytes >= STAGED_COPY_MIN_BYTES && host_is_pageable(host)) return staged_d2h(m->device, host, sc.slab[w], bytes);
-    SB_CUDA(cudaMemcpyAsync(host, sc.slab[w], bytes, cudaMemcpyDeviceToHost, m->stream));
+    SB_TRY(host_copies(m->device, m->stream, cudaMemcpyDeviceToHost, {{out + s->bounds[w] * ncol, sc.slab[w], bytes}}));
     SB_CUDA(cudaStreamSynchronize(m->stream));
     return SB200_OK;
   }));
   tr.phase("results home");
-  if (tr.on) {
-    std::string per;
-    float worst = 0.0f;
-    for (int w = 0; w < W; ++w) {
-      DeviceGuard g(s->blocks[w]->device);
-      float ms = 0.0f;
-      cudaEventElapsedTime(&ms, t0[w], t1[w]);
-      worst = std::max(worst, ms);
-      per += (w ? " " : "") + std::to_string(ms);
-    }
-    fprintf(stderr, "[sb200 trace] %s: device part %.4f ms (max over devices; per device: %s)\n", tr.title, worst, per.c_str());
-  }
+  dp.report(tr.title);
   return SB200_OK;
 }
 

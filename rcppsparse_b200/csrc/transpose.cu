@@ -592,32 +592,6 @@ int launch_place(sb200_matrix* m, const BandPlan* bp, int32_t* d_i_out, double* 
   return SB200_OK;
 }
 
-struct PhaseTimer {  // SB200_TRACE=1: device time of the plan and of the placement on stderr
-  bool on;
-  cudaStream_t st;
-  cudaEvent_t ev[4];
-  int n = 0;
-  explicit PhaseTimer(cudaStream_t s) : on(getenv("SB200_TRACE") != nullptr), st(s) {}
-  void mark() {
-    if (!on || n >= 4) return;
-    cudaEventCreate(&ev[n]);
-    cudaEventRecord(ev[n++], st);
-  }
-  void report(const char* what, const BandPlan* bp, int kind) {
-    if (!on) return;
-    cudaStreamSynchronize(st);
-    fprintf(stderr, "[sb200 trace] transpose (%s, %s) nb=%d S=%d maxrows=%d:", what, kind == 2 ? "chunk-sort placement" : "banded two-pass",
-            bp->nb, bp->S, bp->max_rows);
-    for (int k = 1; k < n; ++k) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, ev[k - 1], ev[k]);
-      fprintf(stderr, " phase%d %.3f ms;", k, ms);
-    }
-    fprintf(stderr, "\n");
-    for (int k = 0; k < n; ++k) cudaEventDestroy(ev[k]);
-  }
-};
-
 }  // namespace
 
 // kind: 1 = banded two-pass kernel of bands.cu (2432-row bands), 2 = chunk-sort placement (384-row bands),
@@ -651,8 +625,8 @@ int transpose_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, double
     SB_CUDA(cudaGetLastError());
     return SB200_OK;
   }
-  PhaseTimer tr(st);
-  tr.mark();
+  PhaseTrace tr(st);
+  tr.mark("start");
   int kind = transpose_kind(m);
   if (kind == 3) {
     const int rc3 = transpose_split_device(m, d_p_out, d_i_out, d_x_out);
@@ -687,7 +661,7 @@ int transpose_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, double
     m->plan_transpose = bp;
   }
   const BandPlan* bp = m->plan_transpose;
-  tr.mark();
+  tr.mark("phase1");
   SB_CUDA(cudaMemcpyAsync(d_p_out, bp->d_rowptr, sizeof(int32_t) * (static_cast<size_t>(nrow) + 1), cudaMemcpyDeviceToDevice, st));
   int rc;
   if (kind == 2) {
@@ -715,8 +689,9 @@ int transpose_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, double
   } else {
     rc = launch_transpose_banded(m, bp, d_i_out, d_x_out);
   }
-  tr.mark();
-  tr.report(cached ? "cached plan" : "plan built", bp, kind);
+  tr.mark("phase2");
+  tr.report("transpose (%s, %s) nb=%d S=%d maxrows=%d:", cached ? "cached plan" : "plan built",
+            kind == 2 ? "chunk-sort placement" : "banded two-pass", bp->nb, bp->S, bp->max_rows);
   return rc;
 }
 

@@ -36,7 +36,6 @@
 
 #include <algorithm>
 #include <new>
-#include <chrono>
 #include <vector>
 
 #include "common.cuh"
@@ -599,33 +598,6 @@ cudaError_t launch_split_cfg(const SplitArgs& a, int sm_count, int64_t units, cu
   return launch_split<PASS, SP_THREADS, SP_TE / SP_THREADS>(a, sm_count, units, st);
 }
 
-struct Trace {  // SB200_TRACE=1: device time of the plan and of the two passes on stderr
-  bool on;
-  cudaStream_t st;
-  cudaEvent_t ev[4];
-  int n = 0;
-  explicit Trace(cudaStream_t s) : on(getenv("SB200_TRACE") != nullptr), st(s) {}
-  void mark() {
-    if (!on || n >= 4) return;
-    cudaEventCreate(&ev[n]);
-    cudaEventRecord(ev[n++], st);
-  }
-  void report(const SplitPlan* sp, bool cached) {
-    if (!on) return;
-    cudaStreamSynchronize(st);
-    fprintf(stderr, "[sb200 trace] transpose (%s, two stream splits) rows/band=%d bands=%d tiles=%lld plan=%.1f MB:", cached ? "cached plan" : "plan built",
-            1 << sp->sh, sp->nb, static_cast<long long>(sp->ntiles), sp->bytes / 1048576.0);
-    static const char* names[] = {"plan", "pass1", "pass2"};
-    for (int k = 1; k < n; ++k) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, ev[k - 1], ev[k]);
-      fprintf(stderr, " %s %.3f ms;", names[k - 1], ms);
-    }
-    fprintf(stderr, "\n");
-    for (int k = 0; k < n; ++k) cudaEventDestroy(ev[k]);
-  }
-};
-
 int segment_chunks() {
   if (const char* e = getenv("SB200_SPLIT_SEG")) {
     const int v = atoi(e);
@@ -715,14 +687,7 @@ static int build_split_plan(sb200_matrix* m, SplitPlan** out) {
       }
     }
   } guard{&sp, st, drop};
-  const bool trace = getenv("SB200_TRACE") != nullptr;
-  auto t_prev = std::chrono::steady_clock::now();
-  auto phase = [&](const char* what) {  // host wall clock: a stall inside a driver call shows here, not in the device's event times
-    if (!trace) return;
-    const auto now = std::chrono::steady_clock::now();
-    fprintf(stderr, "[sb200 trace] split plan: %s %.2f ms\n", what, std::chrono::duration<double, std::milli>(now - t_prev).count());
-    t_prev = now;
-  };
+  WallTrace wt("split plan");  // host wall clock: a stall inside a driver call shows here, not in the device's event times
   const size_t ws_bytes = scan_workspace_bytes(cells > m->nrow ? cells : m->nrow);
   SB_TRY(pool_alloc(reinterpret_cast<void**>(&d_hc), sizeof(uint32_t) * static_cast<size_t>(cells), st));
   SB_TRY(pool_alloc(reinterpret_cast<void**>(&d_rowcnt), sizeof(uint32_t) * static_cast<size_t>(m->nrow), st));
@@ -735,7 +700,7 @@ static int build_split_plan(sb200_matrix* m, SplitPlan** out) {
   SB_TRY(pool_alloc(reinterpret_cast<void**>(&sp->d_counters), sizeof(unsigned int) * 2, st));
   sp->bytes = sizeof(int32_t) * (static_cast<size_t>(m->nrow) + 1 + static_cast<size_t>(cells) + nb + 1 + static_cast<size_t>(nt) + 1) + 8;
 
-  phase("tables allocated");
+  wt.phase("tables allocated");
   SB_CUDA(cudaMemsetAsync(d_rowcnt, 0, sizeof(uint32_t) * static_cast<size_t>(m->nrow), st));
   int64_t grid = nt < static_cast<int64_t>(m->sm_count) * 4 ? nt : static_cast<int64_t>(m->sm_count) * 4;
   split_hist_kernel<<<static_cast<unsigned>(grid), SP_THREADS, sizeof(uint32_t) * nb, st>>>(m->d_i, m->nnz, sp->sh, nb, sp->te, nt, d_hc, d_rowcnt);
@@ -754,10 +719,10 @@ static int build_split_plan(sb200_matrix* m, SplitPlan** out) {
   SB_CUDA(cudaGetLastError());
   // pass-2 units: every band's stream in segments of SP_SEG_CHUNKS chunks
   std::vector<int32_t> bs(static_cast<size_t>(nb) + 1), seg, segfirst(static_cast<size_t>(nb) + 1);
-  phase("kernels enqueued");
+  wt.phase("kernels enqueued");
   SB_CUDA(cudaMemcpyAsync(bs.data(), sp->d_bstart, sizeof(int32_t) * (nb + 1), cudaMemcpyDeviceToHost, st));
   SB_CUDA(cudaStreamSynchronize(st));
-  phase("band starts on the host");
+  wt.phase("band starts on the host");
   const int seg_chunks = segment_chunks();
   sp->seg_chunks = seg_chunks;
   const int64_t seglen = static_cast<int64_t>(seg_chunks) * sp->te;
@@ -778,7 +743,7 @@ static int build_split_plan(sb200_matrix* m, SplitPlan** out) {
   SB_CUDA(cudaMemcpyAsync(sp->d_seg, seg.data(), sizeof(int32_t) * seg.size(), cudaMemcpyHostToDevice, st));
   SB_CUDA(cudaMemcpyAsync(sp->d_segfirst, segfirst.data(), sizeof(int32_t) * (nb + 1), cudaMemcpyHostToDevice, st));
   SB_CUDA(cudaStreamSynchronize(st));
-  phase("segments uploaded");
+  wt.phase("segments uploaded");
   guard.armed = false;
   *out = sp;
   return SB200_OK;
@@ -786,8 +751,8 @@ static int build_split_plan(sb200_matrix* m, SplitPlan** out) {
 
 int transpose_split_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, double* d_x_out) {
   cudaStream_t st = m->stream;
-  Trace tr(st);
-  tr.mark();
+  PhaseTrace tr(st);
+  tr.mark("start");
   if (m->plan_split && (m->plan_split->sh != band_shift(m) || m->plan_split->seg_chunks != segment_chunks() ||
                         m->plan_split->te != split_cfg().threads * split_cfg().ept)) {
     free_split_plan(m->plan_split, st);
@@ -796,7 +761,7 @@ int transpose_split_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, 
   const bool cached = m->plan_split != nullptr;
   if (!cached) SB_TRY(build_split_plan(m, &m->plan_split));
   const SplitPlan* sp = m->plan_split;
-  tr.mark();
+  tr.mark("plan");
   SB_CUDA(cudaMemcpyAsync(d_p_out, sp->d_rowptr, sizeof(int32_t) * (static_cast<size_t>(m->nrow) + 1), cudaMemcpyDeviceToDevice, st));
   Rec* rec = nullptr;  // per-call scratch: the pool hands the same block back call after call (measured: no jitter from it)
   const size_t n = static_cast<size_t>(m->nnz);
@@ -826,7 +791,7 @@ int transpose_split_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, 
       a.counter = sp->d_counters;
       e = launch_split_cfg<1>(a, m->sm_count, sp->ntiles, st);
     }
-    tr.mark();
+    tr.mark("pass1");
     if (e == cudaSuccess && !m->plan_split->segcur_ready && sp->nseg > 0) {
       // first call: the cursors every segment starts from, counted from the record stream that now exists
       const int R = 1 << sp->sh;
@@ -844,11 +809,12 @@ int transpose_split_device(sb200_matrix* m, int32_t* d_p_out, int32_t* d_i_out, 
       a.counter = sp->d_counters + 1;
       e = launch_split_cfg<2>(a, m->sm_count, sp->nseg, st);
     }
-    tr.mark();
+    tr.mark("pass2");
     if (e != cudaSuccess) rc = cuda_fail(e, "transpose: stream split launch", __FILE__, __LINE__);
   }
   pool_free(rec, st);
-  tr.report(sp, cached);
+  tr.report("transpose (%s, two stream splits) rows/band=%d bands=%d tiles=%lld plan=%.1f MB:", cached ? "cached plan" : "plan built",
+            1 << sp->sh, sp->nb, static_cast<long long>(sp->ntiles), sp->bytes / 1048576.0);
   return rc;
 }
 
